@@ -576,10 +576,30 @@ def lerf_train_leg(rank: int, world: int, dev, hash_model, tf_peak: float, rays:
                       f"{rays} rays/GPU/step, 64 + 128 samples, random unit 512-d targets; random-init O(1) language weights"}
 
 
+def dump_outputs(out_dir: str, model, step_out: dict, rank: int, max_rows: int = 8192) -> None:
+    """Writes what the last timed training step computed as <out_dir>/<name>.npy, float32: the loss, the fine pass's rgb [R,3] and depths z [R,S+N]
+    of rank 0's rays (a fixed, seeded sample of max_rows rays when R is larger) and the parameters after the step's Adam update (hash table +
+    NeRFSmall weights, 8.9 M values at the benchmark's shape; under 64 MB in all).  Collective under the fused data-parallel optimiser."""
+    import numpy as np
+    import torch
+    params = model.state_dict()["params"]          # gathers the owners' shards first under the fused optimiser
+    if rank != 0:
+        return
+    rgb, z = step_out["rgb"], step_out["z"]
+    if rgb.shape[0] > max_rows:
+        rows = torch.randperm(rgb.shape[0], generator=torch.Generator().manual_seed(0))[:max_rows].sort().values.to(rgb.device)
+        rgb, z = rgb[rows], z[rows]
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, t in (("loss", model.loss), ("rgb", rgb), ("z", z), ("params", params)):
+        np.save(d / f"{name}.npy", t.detach().float().cpu().numpy())
+
+
 def main() -> None:
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=200,
+                    help="timed steps of the headline (its resident and e2e regions); the secondary legs keep their own step counts")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--rays", type=int, default=RAYS_PER_GPU, help="rays per GPU per step (weak scaling, the headline)")
@@ -590,7 +610,14 @@ def main() -> None:
     ap.add_argument("--quick", action="store_true", help="headline + roofline only: skip the render / LeRF / classic / C++-loop legs")
     ap.add_argument("--dp", default="fused", choices=["fused", "nccl"],
                     help="N>1 optimiser step: one peer-memory kernel (reduce-scatter + Adam + shadow all-gather) or NCCL all-reduce + dense Adam")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the headline's timed steps, write what its last step computed (loss, fine-pass rgb and z of rank 0's rays, the "
+                         "updated parameters) as DIR/<name>.npy, so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of this repository's path: it does not apply to --impl reference")
     # stdout carries exactly ONE JSON line: everything native libraries print on file descriptor 1 while the job runs (NCCL's version
     # banner, for one) is sent to stderr; the line itself goes to the saved descriptor at the end
     sys.stdout.flush()
@@ -652,7 +679,7 @@ def main() -> None:
             scale = parallel.allreduce_gradients(model.grads, world)
             model.optimizer_step(grad_scale=scale)
 
-    def train_leg(rays_per_gpu: int, steps: int, n_warm: int, seed0: int, with_e2e: bool):
+    def train_leg(rays_per_gpu: int, steps: int, n_warm: int, seed0: int, with_e2e: bool, dump_dir: str | None = None):
         """Timed regions of one configuration.  What a step consumes is the list of pixels sampled for it (NeRFDataset::get_batch draws them,
         src/NeRFDataset.cpp:154-155): rays (GetRayBatch, :109-144) and targets (the image gather, :156) are formed on the device inside the step's
         first kernel from the resident training view (HashNeRF.set_camera).  value: `steps` replays of the captured step with the pixel lists
@@ -668,6 +695,7 @@ def main() -> None:
         host_pix = [synthetic_pixels(rays_per_gpu, 800, 800, seed=seed0 + 3000 + 1000 * rank + i).pin_memory() for i in range(pool)]
         dev_pix = [p.to(dev) for p in host_pix]
         use_graph = not args.no_graph
+        last_out = {}
         if use_graph:
             model.capture_train_step(rays_per_gpu, world, lambda g: parallel.allreduce_gradients(g, world), pixels=True)
             step = lambda pix: model.train_step_graph(pix)   # noqa: E731 - copies the pixel list (device or pinned host) into its static input
@@ -677,7 +705,9 @@ def main() -> None:
 
             def step(pix):
                 stage_pix.copy_(pix, non_blocking=True)
-                model.forward_backward(stage_pix)
+                fb_out = model.forward_backward(stage_pix)
+                if dump_dir is not None:
+                    last_out.update(fb_out)
                 if model.peer is not None:
                     model.optimizer_step_sharded()
                 else:
@@ -696,6 +726,8 @@ def main() -> None:
         sync_all()
         out = {"ms_total": parallel.max_over_ranks(e0.elapsed_time(e1), world, dev), "loss": float(model.loss), "launches_per_step": launches_per_step,
                "dev_batches": dev_batches, "use_graph": use_graph}
+        if dump_dir is not None:
+            dump_outputs(dump_dir, model, model.graph_outputs if use_graph else last_out, rank)
         if with_e2e:
             for i in range(3):
                 step(host_pix[i % pool])
@@ -715,7 +747,7 @@ def main() -> None:
     # ---- headline: weak scaling, R rays per GPU (BASELINE C2 at N=1; C3's per-GPU share at N=8)
     sampler = ClockSampler(local_rank)
     sampler.start()
-    head = train_leg(R, args.steps, warmup, 0, with_e2e=True)
+    head = train_leg(R, args.steps, warmup, 0, with_e2e=True, dump_dir=args.dump_outputs)
     clocks = sampler.stop()
     ms_total, ms_e2e, use_graph, launches_per_step = head["ms_total"], head["ms_e2e"], head["use_graph"], head["launches_per_step"]
     dev_batches = head["dev_batches"]

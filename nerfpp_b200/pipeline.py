@@ -223,6 +223,11 @@ class FlatAdamModel:
         self._sched_step = self.step
         return self.loss
 
+    @property
+    def graph_outputs(self) -> dict:
+        """What the captured step's forward_backward returns (its static output buffers): after a replay, that step's results."""
+        return self._g_out
+
     def train_step(self, *inputs):
         self.forward_backward(*inputs)
         self.optimizer_step()

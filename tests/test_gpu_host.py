@@ -58,8 +58,23 @@ def _need(ref_cuda):
         pytest.skip("oracle/_ref/nerfpp_ref_cuda.so not loadable")
 
 
-def test_seeded_construction_and_names_match_reference(host, ref_cuda):
-    _need(ref_cuda)
+def _fixture_pipe(host, seed, log2_t):
+    """A drop-in HashNeRF pipeline built the way tests/golden/make_golden_cuda.py built the reference's for its fixtures: same seeds, same arguments."""
+    host.manual_seed(seed)
+    torch.manual_seed(seed)
+    return host.make_cuhash(torch.tensor(BBOX).cuda(), 16, 2, log2_t, 16, 512, 4, 2, 64, 15, 3, 64)
+
+
+def test_seeded_construction_and_names_match_reference(host, ref_cuda, golden):
+    # the reference's seeded draws stored in tests/golden/cuhash.npz (seed 42, 2^10 table): primes, biases, level sizes / offsets bit for bit
+    g = golden("cuhash.npz")
+    p = _fixture_pipe(host, 42, 10)
+    bufs = dict(zip(p.embed_buffer_names(), p.embed_buffers()))
+    for k in ("primes", "biases", "feat_local_idx", "feat_local_size"):
+        assert np.array_equal(bufs["embedder_" + k].cpu().numpy(), g[k]), k
+    assert p.embed_param_names() == ["embedder_embeddings"] and tuple(p.embed_params()[0].shape) == g["table_f16"].shape
+    if ref_cuda is None:
+        return
     ours, ref = _pair(host, ref_cuda)
     assert ours.embed_buffer_names() == ref.embed_buffer_names()            # checkpoint compatibility (SURVEY §5)
     assert ours.model_param_names() == ref.model_param_names()
@@ -72,8 +87,27 @@ def test_seeded_construction_and_names_match_reference(host, ref_cuda):
     assert ours.output_dims() == 32
 
 
-def test_embedders_forward_backward_match_reference(host, ref_cuda):
-    _need(ref_cuda)
+def test_embedders_forward_backward_match_reference(host, ref_cuda, golden):
+    # the reference's CuHashEmbedder forward / backward and CuSHEncoder outputs stored in tests/golden/cuhash.npz and cush.npz
+    g = golden("cuhash.npz")
+    p = _fixture_pipe(host, 42, 10)
+    with torch.no_grad():
+        p.embed_params()[0].copy_(torch.from_numpy(g["table_f16"]).float().cuda())
+    e, k = p.embed(torch.from_numpy(g["points"]).cuda())
+    assert np.array_equal(k.cpu().numpy(), g["keep"])
+    ge = torch.from_numpy(g["enc"]).cuda()
+    assert (e - ge).abs().max().item() <= 2 ** -9 and (e == ge).float().mean().item() > 0.95
+    e.backward(torch.from_numpy(g["grad_enc"]).cuda())
+    gt = p.embed_params()[0].grad.cpu().numpy()
+    assert gt.shape == g["grad_table"].shape
+    assert np.abs(gt - g["grad_table"]).max() <= 2e-2 * np.abs(g["grad_table"]).max()      # reference: x128 fp16 atomics
+    c = golden("cush.npz")
+    d = torch.from_numpy(c["dirs"]).cuda()
+    for deg in range(1, 9):
+        b = torch.from_numpy(c[f"sh{deg}"]).cuda()
+        assert torch.allclose(host.cu_sh_encoder(d, deg), b, rtol=2e-5, atol=2e-6 * b.abs().max().item()), deg
+    if ref_cuda is None:
+        return
     ours, ref = _pair(host, ref_cuda)
     with torch.no_grad():
         t = torch.rand_like(ref.embed_params()[0]) * 2 - 1
@@ -110,8 +144,25 @@ def test_embedders_forward_backward_match_reference(host, ref_cuda):
     assert torch.allclose(host.embedder(x, 10), ref_cuda.embedder(x, 10), rtol=1e-5, atol=2e-5)
 
 
-def test_model_and_render_stages_match_reference(host, ref_cuda):
-    _need(ref_cuda)
+def test_model_and_render_stages_match_reference(host, ref_cuda, golden):
+    # Render() of the reference's NeRFRenderer<CuHashEmbedder,CuSHEncoder,NeRFSmall> stored in tests/golden/cuhash_render.npz (single chunk, ThinRay, no
+    # noise): the same seeded primes, and the maps on the fixture's table and weights
+    g = golden("cuhash_render.npz")
+    p = _fixture_pipe(host, 7, 12)
+    bufs = dict(zip(p.embed_buffer_names(), p.embed_buffers()))
+    assert np.array_equal(bufs["embedder_primes"].cpu().numpy(), g["primes"])
+    with torch.no_grad():
+        p.embed_params()[0].copy_(torch.from_numpy(g["table_f16"]).float().cuda())
+        for i, w in enumerate(p.model_params()):
+            w.copy_(torch.from_numpy(g[f"w{i}"]).cuda())
+    r = p.render(torch.from_numpy(g["o"]).cuda(), torch.from_numpy(g["d"]).cuda(), 64, 128, 4096, False, True)
+    assert tuple(r["weights"].shape) == g["weights"].shape == (48, 192)                  # sample count exact
+    for k in ("rgb", "acc", "depth"):
+        scale = max(1.0, float(np.abs(g[k]).max()))
+        err = np.abs(r[k].detach().cpu().numpy() - g[k]) / scale
+        assert np.median(err) < 2e-3 and err.max() < 3e-2, (k, float(np.median(err)), float(err.max()))
+    if ref_cuda is None:
+        return
     ours, ref = _pair(host, ref_cuda, seed=7)
     with torch.no_grad():                                                   # O(1) signal instead of the 1e-4 / 0.1-gain init
         t = (torch.rand_like(ref.embed_params()[0]) * 2 - 1).half().float()
@@ -262,8 +313,26 @@ def test_shipped_configuration_runs(host):
     assert tv.ndim == 0 and bool(torch.isfinite(tv))
 
 
-def test_classic_pipeline_matches_reference(host, ref_cuda):
-    _need(ref_cuda)
+def test_classic_pipeline_matches_reference(host, ref_cuda, golden):
+    # Render() of the reference's NeRFRenderer<Embedder,Embedder,NeRF> stored in tests/golden/render_rays_classic.npz (width 32, the fixture's
+    # weights; black and white background)
+    g = golden("render_rays_classic.npz")
+    host.manual_seed(5)
+    torch.manual_seed(5)
+    c = host.make_classic(torch.tensor(BBOX).cuda(), 10, 4, 8, 32, True)
+    c.init_model()
+    with torch.no_grad():
+        for name, t in zip(c.model_param_names(), c.model_params()):
+            t.copy_(torch.from_numpy(g[name.replace(".", "__")]).cuda())
+    o, d = torch.from_numpy(g["o"]).cuda(), torch.from_numpy(g["d"]).cuda()
+    for white, rgb_key in ((False, "rgb"), (True, "rgb_white")):
+        r = c.render(o, d, 64, 128, 4096, white, True)
+        assert torch.allclose(r["rgb"].cpu(), torch.from_numpy(g[rgb_key]), rtol=1e-2, atol=1e-2), white
+        if not white:
+            for k in ("acc", "depth"):
+                assert torch.allclose(r[k].cpu(), torch.from_numpy(g[k]), rtol=1e-2, atol=1e-2), k
+    if ref_cuda is None:
+        return
     pipes = []
     for mod, extra in ((host, ()), (ref_cuda, (True,))):
         mod.manual_seed(5)
@@ -287,27 +356,29 @@ def test_classic_pipeline_matches_reference(host, ref_cuda):
 def test_classic_inference_runs_on_the_fused_tcgen05_forward(host, ref_cuda):
     """Under NoGradGuard (render_image) the drop-in NeRF::forward is ONE nrf_mlp_nerf_fwd launch; the reference renders the same
     image through 11 cuBLAS SGEMMs.  fp16 operands vs fp32: maps agree to 1e-2; and the drop-in's own autograd path (torch::linear)
-    agrees with its fused path."""
-    _need(ref_cuda)
+    agrees with its fused path.  The comparison with the reference runs where oracle/_ref/nerfpp_ref_cuda.so is loadable."""
     from nerfpp_b200 import cabi
     pipes = []
     for mod, extra in ((host, ()), (ref_cuda, (True,))):
+        if mod is None:
+            continue
         mod.manual_seed(9)
         torch.manual_seed(9)
         p = mod.make_classic(torch.tensor(BBOX).cuda(), 10, 4, 8, 256, True, *extra)
         p.init_model()
         pipes.append(p)
-    ours, ref = pipes
-    _positive_density(ours, ref)
+    ours = pipes[0]
+    _positive_density(*pipes)
     K = torch.tensor([[30.0, 0, 12.0], [0, 30.0, 10.0], [0, 0, 1]])
     c2w = torch.eye(4)
     c2w[2, 3] = 4.0
     n0 = cabi.launch_count()
     a = ours.render_image(20, 24, K.cuda(), c2w.cuda(), 64, 128, 4096, False, True)
     assert cabi.launch_count() > n0
-    b = ref.render_image(20, 24, K.cuda(), c2w.cuda(), 64, 128, 4096, False, True)
-    for k in ("rgb", "acc", "depth"):
-        assert torch.allclose(a[k], b[k], rtol=1e-2, atol=1e-2), k
+    if ref_cuda is not None:
+        b = pipes[1].render_image(20, 24, K.cuda(), c2w.cuda(), 64, 128, 4096, False, True)
+        for k in ("rgb", "acc", "depth"):
+            assert torch.allclose(a[k], b[k], rtol=1e-2, atol=1e-2), k
     # staged inference evaluates the importance samples only (one network for both passes): the coarse samples' rows come from the coarse pass.
     # Same rows through the same row-independent kernel => the same maps bit for bit, with a third fewer network evaluations
     ours.reuse_coarse_rows(False)

@@ -185,8 +185,7 @@ int nrf_mlp_small_fwd(const nrf_mlp_small_shape* shape, const void* packed, nrf_
  * perm[ray, j] of enc_merged [R, n_merged, 32] (keep_merged [R, n_merged], nullable, likewise; views: ray_sh [R,16]) and writes
  * raw_merged [R, n_merged, 4] at the same row.  perm [R, n_merged] int16 = nrf_sample_pdf_merge_perm's output; the coarse
  * samples' rows of raw_merged are the coarse pass's own rows, moved there by nrf_sample_pdf_merge_rows — the same bits a full
- * nrf_mlp_small_fwd over the merged rows produces (rows are independent), at n_importance / n_merged of its work.
- * NRF_ERR_UNSUPPORTED when the tcgen05 forward is switched off (NRF_MLP_FWD=mma): callers then evaluate all merged rows. */
+ * nrf_mlp_small_fwd over the merged rows produces (rows are independent), at n_importance / n_merged of its work. */
 int nrf_mlp_small_fwd_importance(const nrf_mlp_small_shape* shape, const void* packed, nrf_mlp_input in_kind, const void* enc_merged,
                                  const float* ray_sh, const uint8_t* keep_merged, const int16_t* perm, int64_t n_rays,
                                  int32_t n_importance, int32_t n_merged, float* raw_merged, nrf_stream stream);

@@ -1,7 +1,7 @@
-// Packed-weight blob of the fused NeRFSmall kernels (nrf_mlp_small_pack): layout constants shared by the mma.sync kernels
-// (mlp_small.cu) and the tcgen05 kernel (mlp_small_tc.cu).
+// Packed-weight blob of the fused NeRFSmall kernels (nrf_mlp_small_pack): layout constants shared by the mma.sync backward
+// (mlp_small.cu) and the tcgen05 forward (mlp_small_tc.cu).
 //
-//   words [0, kFwdWords)            forward B fragments for mma.sync m16n8k16, fp16, [layer][ks][nt][lane][2]
+//   words [0, kFwdWords)            forward B fragments for mma.sync m16n8k16 (the backward's recompute), fp16, [layer][ks][nt][lane][2]
 //   words [kFwdWords, kBlobWords)   backward (transposed) B fragments, bf16
 //   words [kViewBase, kPackedWords) fp32 view block of colour layer 0 for the per-ray view term (NRF_MLP_IN_ENC16_RAYBIAS)
 //   words [kUmmaBase, kTotalWords)  forward weights as UMMA shared-memory operands (tcgen05.mma B, K-major, no swizzle), fp16:

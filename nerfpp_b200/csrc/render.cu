@@ -100,11 +100,7 @@ static int render_impl(const nrf_render_config* cfg, const nrf_hash_grid* grid, 
 	// One network for both passes (src/NeRFRenderer.h:422,447): the merged fine pass re-uses the coarse pass's raw rows for the coarse
 	// samples and gathers / evaluates the importance samples only — the same bits as evaluating all S + N rows (tests/test_gpu_render.py).
 	// NRF_RENDER_REUSE=0 evaluates every merged row (the A/B baseline).
-	static const bool reuse = [] {
-		const char* e = getenv("NRF_RENDER_REUSE");
-		const char* f = getenv("NRF_MLP_FWD");             // the importance-only forward exists on the tcgen05 kernel only
-		return !(e && e[0] == '0') && !(f && f[0] == 'm');
-	}();
+	static const bool reuse = [] { const char* e = getenv("NRF_RENDER_REUSE"); return !(e && e[0] == '0'); }();
 	// The rays of a chunk are adjacent pixels of a frame (GetRays order): the encode kernel walks the same sample of kRayGroup neighbouring rays
 	// together (nrf_hash_encode_rays_fwd_grouped).  NRF_RENDER_RAY_GROUP=1 restores the per-ray order (the A/B baseline).
 	static const int group = [] { const char* e = getenv("NRF_RENDER_RAY_GROUP"); const int g = e ? atoi(e) : 32; return g >= 1 && g <= 1024 ? g : 32; }();

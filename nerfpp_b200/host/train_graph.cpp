@@ -113,10 +113,8 @@ void HashNeRFTrainGraph::Enqueue(bool with_optimizer)
 		perm.data_ptr<int16_t>(), raw_c.data_ptr<float>(), raw.data_ptr<float>(), st), "nrf_sample_pdf_merge_rows");
 	nrfhost::Check(nrf_hash_encode_rays_fwd(&grid, table16, ray_batch.data_ptr<float>(), 11, z_f.data_ptr<float>(), R, sf, 1, keep.data_ptr<uint8_t>(), enc.data_ptr(),
 		NRF_ENC_F16, perm.data_ptr<int16_t>(), enc_c.data_ptr(), keep_c.data_ptr<uint8_t>(), S, st), "nrf_hash_encode_rays_fwd");
-	if (nrf_mlp_small_fwd_importance(&shape, Packed.data_ptr(), NRF_MLP_IN_ENC16_RAYDIRS, enc.data_ptr(), ray_sh.data_ptr<float>(), keep.data_ptr<uint8_t>(), perm.data_ptr<int16_t>(), R, N, sf,
-		raw.data_ptr<float>(), st) != NRF_OK)      // NRF_MLP_FWD=mma: every merged row
-		nrfhost::Check(nrf_mlp_small_fwd(&shape, Packed.data_ptr(), NRF_MLP_IN_ENC16_RAYDIRS, enc.data_ptr(), ray_sh.data_ptr<float>(), sf, keep.data_ptr<uint8_t>(), nf,
-			raw.data_ptr<float>(), st), "nrf_mlp_small_fwd");
+	nrfhost::Check(nrf_mlp_small_fwd_importance(&shape, Packed.data_ptr(), NRF_MLP_IN_ENC16_RAYDIRS, enc.data_ptr(), ray_sh.data_ptr<float>(), keep.data_ptr<uint8_t>(),
+		perm.data_ptr<int16_t>(), R, N, sf, raw.data_ptr<float>(), st), "nrf_mlp_small_fwd_importance");
 	// RawToOutputs of the fine pass + huber_loss + their backward (src/NeRFRenderer.h:447-448, src/NeRFExecutor.h:883-890, 923): one launch
 	Rgb = F32({R, 3}, dev);
 	Tensor d_raw = F32({R, sf, 4}, dev);

@@ -275,7 +275,7 @@ class HashNeRF(FlatAdamModel):
         # Copy the coarse samples' encoding rows into the fine pass instead of gathering them again: the merged z list contains the
         # coarse samples bit for bit, so the rows are bit-identical (tests/test_gpu_hash.py::test_row_reuse...); ~10 % of the fine-pass encode.
         self.reuse_coarse_rows = True
-        self.reuse_coarse_raw = os.environ.get("NRF_MLP_FWD", "")[:1] != "m"   # the importance-only forward exists on the tcgen05 kernel only
+        self.reuse_coarse_raw = True
         self._u_cache = {}
         self._render_ws = None
         self._cam = None

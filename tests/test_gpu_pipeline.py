@@ -243,8 +243,7 @@ def test_coarse_reuse_leaves_the_render_unchanged():
     o[:7] = torch.tensor([3.0, 2.5, -4.0], device=o.device)          # outside the box, looking away: near = far - 1e-6
     d[:7] = torch.tensor([0.3, 0.8, -0.52], device=o.device)
     outs = []
-    modes = ((False, False), (True, False), (True, True)) if m.reuse_coarse_raw else ((False, False), (True, False))   # NRF_MLP_FWD=mma: no raw reuse
-    for rows, raw in modes:
+    for rows, raw in ((False, False), (True, False), (True, True)):
         m.reuse_coarse_rows, m.reuse_coarse_raw = rows, raw
         outs.append(m.render_rays(o, d, keep_for_backward=True))
     a = outs[0]

@@ -1,7 +1,5 @@
 """The A/B variants that ship in libnerfpp_b200.so behind environment switches (read once per process) stay correct: each is run in a fresh
 process through the parity tests of the default path.
-  NRF_MLP_FWD=mma       the mma.sync forward of NeRFSmall (baseline of the tcgen05 kernel, csrc/mlp_small.cu)
-  NRF_MLP_BWD_DW=mma    weight gradients of NeRFSmall on mma.sync + ldmatrix.trans instead of tcgen05 (csrc/mlp_small.cu)
   NRF_NERF_CLUSTER=2    classic-NeRF forward with 2-CTA clusters sharing one multicast weight stream (csrc/mlp_nerf_tc.cu)
   NRF_LERF_EPI_WARPS=8  eight epilogue warps in the LeRF SIGMA / HIDDEN programs (csrc/lerf_tc.cu)
   NRF_ADAM_L2HINT=0     Adam without the L2 eviction-priority hints (csrc/optim.cu)
@@ -9,8 +7,7 @@ process through the parity tests of the default path.
                         the test compares it with the composed path, which reuses — bit for bit
   NRF_HASH_SPLIT=0      hash forward with one thread per point instead of four lanes per point (csrc/hash_encode.cu)
   NRF_PDL=1             programmatic dependent launch along the step's kernel chain (csrc/common.cuh launch_kernel / pdl_prologue)
-  NRF_SAMPLER_BLOCK=0   warp-per-ray sampler also for training-sized batches (csrc/sampler.cu)
-  NRF_MLP_BWD_WARPS=8   NeRFSmall backward with 8 warps / 128-row tiles instead of 12 / 192 (csrc/mlp_small.cu)"""
+  NRF_SAMPLER_BLOCK=0   warp-per-ray sampler also for training-sized batches (csrc/sampler.cu)"""
 import os
 import subprocess
 import sys
@@ -21,17 +18,13 @@ pytestmark = pytest.mark.gpu
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 VARIANTS = [
-    ({"NRF_MLP_FWD": "mma"}, ["test_gpu_mlp.py"], "fixture or fused_input"),
-    ({"NRF_MLP_BWD_DW": "mma"}, ["test_gpu_mlp.py"], "fixture or fused_input"),
     ({"NRF_NERF_CLUSTER": "2"}, ["test_gpu_mlp_nerf.py"], "forward_matches_oracle or repeatable"),
     ({"NRF_LERF_EPI_WARPS": "8"}, ["test_gpu_lerf.py"], "fixture or oracle"),
     ({"NRF_ADAM_L2HINT": "0"}, ["test_gpu_render.py"], "adam"),
     ({"NRF_RENDER_REUSE": "0"}, ["test_gpu_pipeline.py"], "fused_render_entry"),
-    ({"NRF_MLP_FWD": "mma"}, ["test_gpu_pipeline.py"], "fused_render_entry or coarse_reuse"),
     ({"NRF_HASH_SPLIT": "0"}, ["test_gpu_hash.py"], "fixture or reuse or rays"),
     ({"NRF_PDL": "1"}, ["test_gpu_pipeline.py"], "graph or gradients or trains or reuse or render"),
     ({"NRF_SAMPLER_BLOCK": "0"}, ["test_gpu_render.py"], "sample_pdf or merge or sampler"),
-    ({"NRF_MLP_BWD_WARPS": "8"}, ["test_gpu_mlp.py"], "fixture or fused_input or per_ray"),
 ]
 
 

@@ -133,6 +133,34 @@ int nrf_hash_encode_rays_bwd_levels(const nrf_hash_grid* grid, const float* ray_
                                     int64_t n_rays, int32_t n_samples, int clamp_points, const void* grad_enc, nrf_grad_layout layout,
                                     float* grad_table, int32_t level_begin, int32_t level_end, nrf_stream stream);
 
+/* The ray entries above with the per-sample perturbations of the reference's shipped training configuration (src/main.cpp:187
+ * thin_ray = false; src/NeRFExecutor.h:411-412 RawNoiseStd / StochasticPreconditioningAlpha) applied inside the kernels, in the order of
+ * src/NeRFRenderer.h:419-445:
+ *     p = o + d z                                                     (:419 / :432)
+ *     sp_noise != NULL:   p = ReflectBoundary(p + sp_noise * alpha)   (:435-443, :285-304; the caller passes it for the fine pass only)
+ *     cone_angle != NULL: p += (t r cos(theta) + b r sin(theta)) * cone_angle * z, then clamped into the grid's box if clamp_to_box
+ *                                                                     (TangentScatter, :307-362)
+ * then the encode's own clamp / keep mask as above.  This replaces nrf_sample_points -> nrf_precondition_points -> nrf_tangent_scatter ->
+ * nrf_hash_encode_fwd / _bwd on the [R,S,3] array, with the same arithmetic (bit-identical points); no point array exists in either
+ * direction: the backward re-derives the forward's points from the same variates.  The variates are the caller's torch draws, so the
+ * Philox stream stays the reference's.  No row reuse (a jittered sample is re-jittered with fresh draws in the fine pass). */
+typedef struct nrf_point_jitter {
+	const float* cone_angle;   /* NULL = thin rays; one scalar (cone_stride 0) or one per ray at cone_angle[ray * cone_stride]         */
+	int32_t cone_stride;
+	const float* rand_r;       /* [R,S] uniforms: the two torch::rand draws of src/NeRFRenderer.h:342-343 (needed with a cone)          */
+	const float* rand_theta;
+	int32_t clamp_to_box;      /* TangentScatter's clamp into the grid's box (bounding box given, :356-360)                            */
+	const float* sp_noise;     /* [R,S,3] standard normal (randn_like(pts), :437); NULL = no stochastic preconditioning                 */
+	const float* sp_alpha;     /* DEVICE scalar: the step's StochasticPreconditioningAlpha (needed with sp_noise)                      */
+} nrf_point_jitter;
+
+int nrf_hash_encode_rays_jitter_fwd(const nrf_hash_grid* grid, const void* table_f16, const float* ray_batch, int32_t ray_stride,
+                                    const float* z, int64_t n_rays, int32_t n_samples, int clamp_points, uint8_t* keep, void* enc_out,
+                                    nrf_enc_layout layout, const nrf_point_jitter* jitter, nrf_stream stream);
+int nrf_hash_encode_rays_jitter_bwd(const nrf_hash_grid* grid, const float* ray_batch, int32_t ray_stride, const float* z,
+                                    int64_t n_rays, int32_t n_samples, int clamp_points, const void* grad_enc, nrf_grad_layout layout,
+                                    float* grad_table, const nrf_point_jitter* jitter, nrf_stream stream);
+
 /* ------------------------------------------------------------------------------------------------------------
  * Direction / position encoders
  * ---------------------------------------------------------------------------------------------------------- */

@@ -71,6 +71,12 @@ class RenderConfig(Structure):
                 ("near_plane", c_float), ("bbox", c_float * 6)]
 
 
+class PointJitter(Structure):
+    """struct nrf_point_jitter"""
+    _fields_ = [("cone_angle", c_void_p), ("cone_stride", c_int32), ("rand_r", c_void_p), ("rand_theta", c_void_p), ("clamp_to_box", c_int32),
+                ("sp_noise", c_void_p), ("sp_alpha", c_void_p)]
+
+
 NRF_MAX_PEERS = 8
 
 
@@ -96,6 +102,10 @@ SIGNATURES = {
                                                    c_int32, _P]),
     "nrf_hash_encode_rays_bwd": (c_int32, [POINTER(HashGrid), _P, c_int32, _P, c_int64, c_int32, c_int32, _P, c_int32, _P, _P]),
     "nrf_hash_encode_rays_bwd_levels": (c_int32, [POINTER(HashGrid), _P, c_int32, _P, c_int64, c_int32, c_int32, _P, c_int32, _P, c_int32, c_int32, _P]),
+    "nrf_hash_encode_rays_jitter_fwd": (c_int32, [POINTER(HashGrid), _P, _P, c_int32, _P, c_int64, c_int32, c_int32, _P, _P, c_int32,
+                                                  POINTER(PointJitter), _P]),
+    "nrf_hash_encode_rays_jitter_bwd": (c_int32, [POINTER(HashGrid), _P, c_int32, _P, c_int64, c_int32, c_int32, _P, c_int32, _P,
+                                                  POINTER(PointJitter), _P]),
     "nrf_sample_pdf_merge_perm": (c_int32, [_P, _P, _P, c_int32, c_int64, c_int32, c_int32, _P, _P, _P, _P]),
     "nrf_sample_pdf_merge_rows": (c_int32, [_P, _P, _P, c_int32, c_int64, c_int32, c_int32, _P, _P, _P, _P, _P, _P]),
     "nrf_sh_encode_fwd": (c_int32, [_P, c_int32, c_int64, c_int32, _P, _P]),

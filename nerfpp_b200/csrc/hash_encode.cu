@@ -17,6 +17,7 @@
 //   * level metadata (scale, primes, offsets) is staged once per CTA in shared memory;
 //   * the backward accumulates in fp32 with vector RED (red.global.add.v2.f32), no x128 loss scale.
 #include "common.cuh"
+#include "jitter.cuh"
 #include <stdlib.h>
 #include <string.h>
 
@@ -103,6 +104,50 @@ __device__ __forceinline__ void load_point(const PointSrc& ps, int64_t i, float&
 		x = __fadd_rn(__ldg(rb + 0), __fmul_rn(__ldg(rb + 3), zi));
 		y = __fadd_rn(__ldg(rb + 1), __fmul_rn(__ldg(rb + 4), zi));
 		z = __fadd_rn(__ldg(rb + 2), __fmul_rn(__ldg(rb + 5), zi));
+	}
+}
+
+// The same rays with the per-sample perturbations of the reference's shipped training configuration (nrf_point_jitter), applied in the
+// order of src/NeRFRenderer.h:419-445: p = o + d z; [sp_noise] ReflectBoundary(p + noise * alpha) (:435-443); [cone] += TangentScatter
+// offset (:307-362), clamped into the box if asked (:356-360).  jitter.cuh holds the arithmetic, shared with nrf_tangent_scatter /
+// nrf_precondition_points, so the points are those the composed path materialises, bit for bit.  No row reuse, no ray grouping.
+struct JitterSrc {
+	const float* ray_batch;
+	const float* z;
+	int ray_stride, S;
+	const float* cone;
+	int cone_stride;
+	const float* rand_r;
+	const float* rand_theta;
+	int clamp_box;
+	const float* sp_noise;
+	const float* sp_alpha;
+	Box box;
+	static constexpr int group = 1, R = 0, S_work = 0;
+};
+
+__device__ __forceinline__ void load_point(const JitterSrc& ps, int64_t i, float& x, float& y, float& z)
+{
+	const uint32_t ray = static_cast<uint32_t>(i) / static_cast<uint32_t>(ps.S);   // N < 2^31 checked by the host
+	const float* rb = ps.ray_batch + static_cast<int64_t>(ray) * ps.ray_stride;
+	const float zi = ps.z[i];
+	const float dx = __ldg(rb + 3), dy = __ldg(rb + 4), dz = __ldg(rb + 5);
+	x = __fadd_rn(__ldg(rb + 0), __fmul_rn(dx, zi));
+	y = __fadd_rn(__ldg(rb + 1), __fmul_rn(dy, zi));
+	z = __fadd_rn(__ldg(rb + 2), __fmul_rn(dz, zi));
+	if (ps.sp_noise) {
+		const float alpha = __ldg(ps.sp_alpha);
+		const float* nz = ps.sp_noise + i * 3;
+		x = precondition_coord(x, __ldg(nz + 0), alpha, ps.box.lo[0], ps.box.hi[0]);
+		y = precondition_coord(y, __ldg(nz + 1), alpha, ps.box.lo[1], ps.box.hi[1]);
+		z = precondition_coord(z, __ldg(nz + 2), alpha, ps.box.lo[2], ps.box.hi[2]);
+	}
+	if (ps.cone) {
+		float off[3];
+		tangent_direction(dx, dy, dz, __ldg(ps.rand_r + i), __ldg(ps.rand_theta + i), off);
+		const float radius = __fmul_rn(__ldg(ps.cone + (ps.cone_stride ? static_cast<int64_t>(ray) * ps.cone_stride : 0)), zi);
+		apply_tangent_offset(off, radius, x, y, z);
+		if (ps.clamp_box) clamp_to_box(ps.box, x, y, z);
 	}
 }
 
@@ -210,9 +255,9 @@ __device__ __forceinline__ void unpack(const typename FeatVec<F>::type& v, float
 // neighbouring lanes share a point and each handles ONE chunk of CH levels, so a warp writes 32 / SPLIT complete rows as one contiguous
 // block and an item is 1 / SPLIT of the dependent-latency chain.  Every thread handles `iters` items at a stride of the whole grid: the
 // launch passes iters = 1 (one item per thread; see launch_plan for the persistent-grid experiment that was not kept).
-template <int F, bool OUT_F32, int SPLIT>
-__global__ void __launch_bounds__(128) hash_fwd_kernel(HashArgs a, const __half* __restrict__ table,
-	PointSrc ps, Reuse ru, int64_t n_items, int64_t stride, int iters, int clamp_points, uint8_t* __restrict__ keep, void* __restrict__ out)
+template <int F, bool OUT_F32, int SPLIT, class PS>
+__device__ __forceinline__ void hash_fwd_body(const HashArgs& a, const __half* __restrict__ table,
+	const PS& ps, const Reuse& ru, int64_t n_items, int64_t stride, int iters, int clamp_points, uint8_t* __restrict__ keep, void* __restrict__ out)
 {
 	constexpr int CH = 8 / F;
 	using V = typename FeatVec<F>::type;
@@ -331,6 +376,21 @@ __global__ void __launch_bounds__(128) hash_fwd_kernel(HashArgs a, const __half*
 	}
 }
 
+template <int F, bool OUT_F32, int SPLIT>
+__global__ void __launch_bounds__(128) hash_fwd_kernel(HashArgs a, const __half* __restrict__ table,
+	PointSrc ps, Reuse ru, int64_t n_items, int64_t stride, int iters, int clamp_points, uint8_t* __restrict__ keep, void* __restrict__ out)
+{
+	hash_fwd_body<F, OUT_F32, SPLIT>(a, table, ps, ru, n_items, stride, iters, clamp_points, keep, out);
+}
+
+// a separate instantiation, so that the parity kernels above keep their code; `ru` (same launch signature) is not read: no row reuse
+template <int F, bool OUT_F32, int SPLIT>
+__global__ void __launch_bounds__(128) hash_fwd_jitter_kernel(HashArgs a, const __half* __restrict__ table,
+	JitterSrc ps, Reuse ru, int64_t n_items, int64_t stride, int iters, int clamp_points, uint8_t* __restrict__ keep, void* __restrict__ out)
+{
+	hash_fwd_body<F, OUT_F32, SPLIT>(a, table, ps, Reuse{nullptr, nullptr, nullptr, 0}, n_items, stride, iters, clamp_points, keep, out);
+}
+
 __device__ __forceinline__ void red_add_v2(float* addr, float a, float b)
 {
 	asm volatile("red.global.add.v2.f32 [%0], {%1, %2};" ::"l"(addr), "f"(a), "f"(b) : "memory");
@@ -352,8 +412,8 @@ __device__ __forceinline__ void red_add_v4(float* addr, float a, float b, float 
 // Any point order is handled correctly (a run is defined by adjacency, not by key equality); ray-major order is what
 // makes it pay.  The reference issues N*L*8 half2 atomics regardless (SURVEY §8a-a3).
 // Thread t handles points t, t + stride, ... (`iters` of them, warp-uniform; the launch passes iters = 1).
-template <int F, bool GRAD_BF16>
-__global__ void __launch_bounds__(128) hash_bwd_kernel(HashArgs a, PointSrc ps, int64_t n_points, int64_t stride, int iters,
+template <int F, bool GRAD_BF16, class PS>
+__device__ __forceinline__ void hash_bwd_body(HashArgs a, PS ps, int64_t n_points, int64_t stride, int iters,
 	int clamp_points, const void* __restrict__ grad_enc, float* __restrict__ grad_table, int level_begin, int level_end)
 {
 	constexpr int CH = 8 / F;   // levels per 8-value gradient chunk (16 B of bf16 / 32 B of fp32)
@@ -478,6 +538,26 @@ __global__ void __launch_bounds__(128) hash_bwd_kernel(HashArgs a, PointSrc ps, 
 	}
 	}   // items of this thread
 }
+
+template <int F, bool GRAD_BF16>
+__global__ void __launch_bounds__(128) hash_bwd_kernel(HashArgs a, PointSrc ps, int64_t n_points, int64_t stride, int iters,
+	int clamp_points, const void* __restrict__ grad_enc, float* __restrict__ grad_table, int level_begin, int level_end)
+{
+	hash_bwd_body<F, GRAD_BF16>(a, ps, n_points, stride, iters, clamp_points, grad_enc, grad_table, level_begin, level_end);
+}
+
+template <int F, bool GRAD_BF16>
+__global__ void __launch_bounds__(128) hash_bwd_jitter_kernel(HashArgs a, JitterSrc ps, int64_t n_points, int64_t stride, int iters,
+	int clamp_points, const void* __restrict__ grad_enc, float* __restrict__ grad_table, int level_begin, int level_end)
+{
+	hash_bwd_body<F, GRAD_BF16>(a, ps, n_points, stride, iters, clamp_points, grad_enc, grad_table, level_begin, level_end);
+}
+
+// kernel of a point source, for the launch code shared by both
+template <int F, bool O, int SP> auto fwd_kernel(const PointSrc&) { return hash_fwd_kernel<F, O, SP>; }
+template <int F, bool O, int SP> auto fwd_kernel(const JitterSrc&) { return hash_fwd_jitter_kernel<F, O, SP>; }
+template <int F, bool G> auto bwd_kernel(const PointSrc&) { return hash_bwd_kernel<F, G>; }
+template <int F, bool G> auto bwd_kernel(const JitterSrc&) { return hash_bwd_jitter_kernel<F, G>; }
 
 // Inspection entry (tests): the scalar addresses and trilinear weights the encode kernels use, from the SAME clamp_point / locate code.
 __global__ void __launch_bounds__(128) hash_cells_kernel(HashArgs a, const float* __restrict__ points, int64_t n_points, int clamp_points,
@@ -606,7 +686,10 @@ int nrf_table_to_half(const float* table_f32, void* table_f16, int64_t n_scalars
 	return NRF_OK;
 }
 
-static int launch_hash_fwd(const nrf_hash_grid* grid, const void* table_f16, const PointSrc& ps, const Reuse& ru, int64_t n_points,
+}  // extern "C"
+
+template <class PS>
+static int launch_hash_fwd(const nrf_hash_grid* grid, const void* table_f16, const PS& ps, const Reuse& ru, int64_t n_points,
 	int clamp_points, uint8_t* keep, void* enc_out, nrf_enc_layout layout, nrf_stream stream)
 {
 	HashArgs a;
@@ -625,8 +708,8 @@ static int launch_hash_fwd(const nrf_hash_grid* grid, const void* table_f16, con
 	do {                                                                                                                          \
 		const int64_t items = (ps.group > 1 ? (static_cast<int64_t>(ps.R) + ps.group - 1) / ps.group * ps.group * ps.S_work : n_points) * (SP); \
 		const LaunchPlan lp = launch_plan(items, 128);                                                                           \
-		if (occ_pad_bytes() > 48 * 1024) cudaFuncSetAttribute(hash_fwd_kernel<FF, O32, SP>, cudaFuncAttributeMaxDynamicSharedMemorySize, occ_pad_bytes()); \
-		launch_kernel(hash_fwd_kernel<FF, O32, SP>, lp.grid, 128, occ_pad_bytes(), s, a, t, ps, ru, items, lp.stride, lp.iters, clamp_points, keep, enc_out); \
+		if (occ_pad_bytes() > 48 * 1024) cudaFuncSetAttribute(fwd_kernel<FF, O32, SP>(ps), cudaFuncAttributeMaxDynamicSharedMemorySize, occ_pad_bytes()); \
+		launch_kernel(fwd_kernel<FF, O32, SP>(ps), lp.grid, 128, occ_pad_bytes(), s, a, t, ps, ru, items, lp.stride, lp.iters, clamp_points, keep, enc_out); \
 	} while (0)
 #define NRF_LAUNCH_FWD(FF, SP)                                                     \
 	do {                                                                           \
@@ -648,7 +731,8 @@ static int launch_hash_fwd(const nrf_hash_grid* grid, const void* table_f16, con
 	return NRF_OK;
 }
 
-static int launch_hash_bwd(const nrf_hash_grid* grid, const PointSrc& ps, int64_t n_points, int clamp_points, const void* grad_enc,
+template <class PS>
+static int launch_hash_bwd(const nrf_hash_grid* grid, const PS& ps, int64_t n_points, int clamp_points, const void* grad_enc,
 	nrf_grad_layout layout, float* grad_table, nrf_stream stream, int level_begin = 0, int level_end = -1)
 {
 	HashArgs a;
@@ -664,8 +748,8 @@ static int launch_hash_bwd(const nrf_hash_grid* grid, const PointSrc& ps, int64_
 #define NRF_LAUNCH_BWD2(FF, BF)                                                                                                   \
 	do {                                                                                                                          \
 		const LaunchPlan lp = launch_plan(n_points, 128);                                                                        \
-		if (occ_pad_bytes() > 48 * 1024) cudaFuncSetAttribute(hash_bwd_kernel<FF, BF>, cudaFuncAttributeMaxDynamicSharedMemorySize, occ_pad_bytes()); \
-		launch_kernel(hash_bwd_kernel<FF, BF>, lp.grid, 128, occ_pad_bytes(), s, a, ps, n_points, lp.stride, lp.iters, clamp_points, grad_enc, grad_table, \
+		if (occ_pad_bytes() > 48 * 1024) cudaFuncSetAttribute(bwd_kernel<FF, BF>(ps), cudaFuncAttributeMaxDynamicSharedMemorySize, occ_pad_bytes()); \
+		launch_kernel(bwd_kernel<FF, BF>(ps), lp.grid, 128, occ_pad_bytes(), s, a, ps, n_points, lp.stride, lp.iters, clamp_points, grad_enc, grad_table, \
 			level_begin, level_end);                                                                                                  \
 	} while (0)
 #define NRF_LAUNCH_BWD(FF)                                             \
@@ -682,6 +766,8 @@ static int launch_hash_bwd(const nrf_hash_grid* grid, const PointSrc& ps, int64_
 	NRF_CHECK_LAUNCH("hash_bwd_kernel");
 	return NRF_OK;
 }
+
+extern "C" {
 
 int nrf_hash_encode_fwd(const nrf_hash_grid* grid, const void* table_f16, const float* points, int64_t n_points,
 	int clamp_points, uint8_t* keep, void* enc_out, nrf_enc_layout layout, nrf_stream stream)
@@ -753,6 +839,43 @@ int nrf_hash_encode_rays_bwd_levels(const nrf_hash_grid* grid, const float* ray_
 	NRF_REQUIRE(n_points < (int64_t(1) << 31), "n_rays * n_samples must be < 2^31 per call");
 	const PointSrc ps{nullptr, ray_batch, z, ray_stride, n_samples};
 	return launch_hash_bwd(grid, ps, n_points, clamp_points, grad_enc, layout, grad_table, stream, level_begin, level_end);
+}
+
+
+// argument checks and the point source of the two jitter entries
+static int jitter_src(const nrf_hash_grid* grid, const float* ray_batch, int32_t ray_stride, const float* z, int64_t n_rays, int32_t n_samples,
+	const nrf_point_jitter* j, JitterSrc& ps)
+{
+	NRF_REQUIRE(grid != nullptr && j != nullptr, "null grid / jitter");
+	NRF_REQUIRE(n_rays >= 0 && n_samples >= 1 && ray_stride >= 6, "bad sizes");
+	NRF_REQUIRE(n_rays * n_samples < (int64_t(1) << 31), "n_rays * n_samples must be < 2^31 per call");
+	NRF_REQUIRE(!j->cone_angle || (j->rand_r && j->rand_theta && j->cone_stride >= 0), "a cone needs rand_r, rand_theta and cone_stride >= 0");
+	NRF_REQUIRE(!j->sp_noise || j->sp_alpha, "sp_noise needs the device scalar sp_alpha");
+	NRF_REQUIRE(n_rays == 0 || (ray_batch && z), "null ray_batch / z");
+	ps = JitterSrc{ray_batch, z, ray_stride, n_samples, j->cone_angle, j->cone_stride, j->rand_r, j->rand_theta, j->clamp_to_box, j->sp_noise, j->sp_alpha, {}};
+	for (int k = 0; k < 3; k++) { ps.box.lo[k] = grid->box_min[k]; ps.box.hi[k] = grid->box_max[k]; }
+	return NRF_OK;
+}
+
+int nrf_hash_encode_rays_jitter_fwd(const nrf_hash_grid* grid, const void* table_f16, const float* ray_batch, int32_t ray_stride, const float* z,
+	int64_t n_rays, int32_t n_samples, int clamp_points, uint8_t* keep, void* enc_out, nrf_enc_layout layout, const nrf_point_jitter* jitter,
+	nrf_stream stream)
+{
+	JitterSrc ps;
+	if (int rc = jitter_src(grid, ray_batch, ray_stride, z, n_rays, n_samples, jitter, ps)) return rc;
+	if (n_rays == 0) { HashArgs a; return fill_args(grid, a); }
+	const Reuse ru{nullptr, nullptr, nullptr, 0};
+	return launch_hash_fwd(grid, table_f16, ps, ru, n_rays * n_samples, clamp_points, keep, enc_out, layout, stream);
+}
+
+int nrf_hash_encode_rays_jitter_bwd(const nrf_hash_grid* grid, const float* ray_batch, int32_t ray_stride, const float* z, int64_t n_rays,
+	int32_t n_samples, int clamp_points, const void* grad_enc, nrf_grad_layout layout, float* grad_table, const nrf_point_jitter* jitter,
+	nrf_stream stream)
+{
+	JitterSrc ps;
+	if (int rc = jitter_src(grid, ray_batch, ray_stride, z, n_rays, n_samples, jitter, ps)) return rc;
+	if (n_rays == 0) { HashArgs a; return fill_args(grid, a); }
+	return launch_hash_bwd(grid, ps, n_rays * n_samples, clamp_points, grad_enc, layout, grad_table, stream);
 }
 
 }

@@ -5,6 +5,7 @@
 // Arithmetic keeps ATen's un-fused order (__fmul_rn / __fadd_rn, no FMA contraction) so that z values, and through
 // them the sample points and hash cells, are the same floats the reference produces.
 #include "common.cuh"
+#include "jitter.cuh"
 #include "sh_basis.cuh"
 
 namespace nrf {
@@ -56,10 +57,6 @@ __global__ void __launch_bounds__(256) ray_batch_kernel(Cam c, const int32_t* __
 		for (int k = 0; k < img_c; k++) target[i * img_c + k] = __ldg(src + k);
 	}
 }
-
-struct Box {
-	float lo[3], hi[3];
-};
 
 // IntersectWithAABB (src/RayUtils.h:87-126) and viewdirs = rays_d / norm(rays_d) (src/NeRFRenderer.h:559) for one ray
 __device__ __forceinline__ void prepare_ray(const float (&o)[3], const float (&d)[3], const Box& box, float near_plane, float& tnear, float& tfar,
@@ -224,13 +221,7 @@ __global__ void __launch_bounds__(256) sample_points_kernel(const float* __restr
 
 // TangentScatter (src/NeRFRenderer.h:307-362): in-cone jitter of the sample points.  The two uniform variates per sample are
 // INPUTS (the host draws them with the same two torch::rand calls as the reference, :342-343, so the Philox stream stays
-// in lock-step with it); this kernel fuses the ~40 ATen launches that build the tangent frame and apply the offset.
-__device__ __forceinline__ void safe_normalize3(float& x, float& y, float& z)
-{
-	const float n = fmaxf(sqrtf(__fadd_rn(__fadd_rn(__fmul_rn(x, x), __fmul_rn(y, y)), __fmul_rn(z, z))), 1e-8f);
-	x = __fdiv_rn(x, n); y = __fdiv_rn(y, n); z = __fdiv_rn(z, n);
-}
-
+// in lock-step with it); this kernel fuses the ~40 ATen launches that build the tangent frame and apply the offset (jitter.cuh).
 __global__ void __launch_bounds__(256) tangent_scatter_kernel(float* __restrict__ pts, const float* __restrict__ z,
 	const float* __restrict__ cone_angle, int cone_stride, const float* __restrict__ rays_d, int d_stride,
 	const float* __restrict__ rand_r, const float* __restrict__ rand_theta, Box box, int clamp_box, int64_t R, int S)
@@ -238,54 +229,24 @@ __global__ void __launch_bounds__(256) tangent_scatter_kernel(float* __restrict_
 	const int64_t e = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
 	if (e >= R * S) return;
 	const int64_t ray = e / S;
-	float dx = rays_d[ray * d_stride], dy = rays_d[ray * d_stride + 1], dz = rays_d[ray * d_stride + 2];
-	safe_normalize3(dx, dy, dz);
-	// helper axis: the coordinate axis along which |d| is strictly smallest, z otherwise (:321-331)
-	const float ax = fabsf(dx), ay = fabsf(dy), az = fabsf(dz);
-	float ux = 0.f, uy = 0.f, uz = 0.f;
-	if (ax < ay && ax < az) ux = 1.f;
-	else if (ay < ax && ay < az) uy = 1.f;
-	else uz = 1.f;
-	// tangent = normalize(d x up), bitangent = normalize(d x tangent) (:333-336)
-	float tx = __fsub_rn(__fmul_rn(dy, uz), __fmul_rn(dz, uy));
-	float ty = __fsub_rn(__fmul_rn(dz, ux), __fmul_rn(dx, uz));
-	float tz = __fsub_rn(__fmul_rn(dx, uy), __fmul_rn(dy, ux));
-	safe_normalize3(tx, ty, tz);
-	float bx = __fsub_rn(__fmul_rn(dy, tz), __fmul_rn(dz, ty));
-	float by = __fsub_rn(__fmul_rn(dz, tx), __fmul_rn(dx, tz));
-	float bz = __fsub_rn(__fmul_rn(dx, ty), __fmul_rn(dy, tx));
-	safe_normalize3(bx, by, bz);
-	// uniform over the disc: r = sqrt(clamp(u1)), theta = fmod(u2 * 2 pi, 2 pi) (:342-345)
-	const float r = sqrtf(fminf(fmaxf(rand_r[e], 1e-8f), 1.0f - 1e-8f));
-	const float two_pi = 6.283185307179586f;
-	const float theta = fmodf(__fmul_rn(__fmul_rn(rand_theta[e], 2.0f), 3.14159265358979323846f), two_pi);
-	const float ox = __fmul_rn(r, cosf(theta)), oy = __fmul_rn(r, sinf(theta));
+	float off[3];
+	tangent_direction(rays_d[ray * d_stride], rays_d[ray * d_stride + 1], rays_d[ray * d_stride + 2], rand_r[e], rand_theta[e], off);
 	const float radius = __fmul_rn(cone_angle[cone_stride ? ray * cone_stride : 0], z[e]);   // cone_radii = cone_angle * z (:313)
 	float* p = pts + e * 3;
-	float px = __fadd_rn(p[0], __fmul_rn(__fadd_rn(__fmul_rn(tx, ox), __fmul_rn(bx, oy)), radius));
-	float py = __fadd_rn(p[1], __fmul_rn(__fadd_rn(__fmul_rn(ty, ox), __fmul_rn(by, oy)), radius));
-	float pz = __fadd_rn(p[2], __fmul_rn(__fadd_rn(__fmul_rn(tz, ox), __fmul_rn(bz, oy)), radius));
-	if (clamp_box) {
-		px = fminf(fmaxf(px, box.lo[0]), box.hi[0]);
-		py = fminf(fmaxf(py, box.lo[1]), box.hi[1]);
-		pz = fminf(fmaxf(pz, box.lo[2]), box.hi[2]);
-	}
+	float px = p[0], py = p[1], pz = p[2];
+	apply_tangent_offset(off, radius, px, py, pz);
+	if (clamp_box) clamp_to_box(box, px, py, pz);
 	p[0] = px; p[1] = py; p[2] = pz;
 }
 
-// Stochastic preconditioning of the fine-pass sample positions (src/NeRFRenderer.h:435-443): pts += noise * alpha, then ReflectBoundary
-// (:285-304): normalise to the box, fold with period 2 (fmod; q -> 2 - q above 1), map back.  noise [R,S,3] standard normal (the reference's
-// torch::randn_like draw, supplied by the host so that the Philox stream is the caller's).
+// Stochastic preconditioning of the fine-pass sample positions (src/NeRFRenderer.h:435-443) + ReflectBoundary (:285-304), jitter.cuh.  noise
+// [R,S,3] standard normal (the reference's torch::randn_like draw, supplied by the host so that the Philox stream is the caller's).
 __global__ void __launch_bounds__(256) precondition_kernel(float* __restrict__ pts, const float* __restrict__ noise, float alpha, Box box, int64_t n3)
 {
 	const int64_t e = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
 	if (e >= n3) return;
 	const int k = static_cast<int>(e % 3);
-	const float lo = box.lo[k], ext = __fsub_rn(box.hi[k], box.lo[k]);
-	const float p = __fadd_rn(pts[e], __fmul_rn(noise[e], alpha));
-	float q = fmodf(__fdiv_rn(__fsub_rn(p, lo), ext), 2.0f);
-	q = q > 1.0f ? __fsub_rn(2.0f, q) : q;
-	pts[e] = __fadd_rn(__fmul_rn(q, ext), lo);
+	pts[e] = precondition_coord(pts[e], noise[e], alpha, box.lo[k], box.hi[k]);
 }
 
 }  // namespace nrf

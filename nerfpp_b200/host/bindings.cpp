@@ -149,6 +149,57 @@ struct Pipeline {
 		}
 		return {secs, losses};
 	}
+	/// NeRFExecutor::Train's loop in the reference's shipped configuration (src/main.cpp:187 thin_ray = false; the per-step RawNoiseStd and
+	/// StochasticPreconditioningAlpha of FillRenderParams(i), src/NeRFExecutor.h:411-412, given as schedules): the graph of train_graph.h, or the
+	/// autograd loop over Render when use_train_graph(False)
+	std::pair<std::vector<double>, std::vector<float>> TrainStepsShipped(Tensor rays_o, Tensor rays_d, Tensor target, Tensor cone, int n_steps,
+		int n_samples, int n_importance, int chunk, float lr, int lrate_decay, std::vector<float> noise_std, std::vector<float> sp_alpha)
+	{
+		TORCH_CHECK(int(noise_std.size()) >= n_steps && int(sp_alpha.size()) >= n_steps, "train_steps_shipped: one noise / alpha value per step");
+		if constexpr (std::is_same_v<N, NeRFSmall>) {
+			if (train_graph) {
+				if (!graph)
+					graph = std::make_unique<HashNeRFTrainGraph>(embed, embeddirs, model, bbox, n_samples, n_importance, lr, lrate_decay, rays_o.size(0), false, chunk);
+				TORCH_CHECK(!graph->ThinRay(), "train_steps_shipped: this pipe's training graph was built for thin rays (train_steps)");
+				std::vector<double> secs; std::vector<float> losses;
+				for (int i = 0; i < n_steps; i++) {
+					auto t0 = std::chrono::steady_clock::now();
+					const float lv = graph->Step(rays_o, rays_d, target, cone, noise_std[i], sp_alpha[i]).template item<float>();
+					secs.push_back(std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count());
+					losses.push_back(lv);
+				}
+				return {secs, losses};
+			}
+		}
+		if (!opt) {
+			std::vector<Tensor> gv;
+			for (auto& p : embed->parameters()) gv.push_back(p);
+			for (auto& p : model->parameters()) gv.push_back(p);
+			const auto options = torch::optim::AdamOptions(lr).eps(1e-15).betas(std::make_tuple(0.9, 0.99));
+			if (fused_adam) opt = std::make_unique<FusedAdam>(gv, options);
+			else opt = std::make_unique<torch::optim::Adam>(gv, options);
+			global_step = 0;
+		}
+		std::vector<double> secs; std::vector<float> losses;
+		for (int i = 0; i < n_steps; i++) {
+			auto t0 = std::chrono::steady_clock::now();
+			auto p = Params(n_samples, n_importance, chunk, false, true, bbox, false, noise_std[i], sp_alpha[i]);
+			opt->zero_grad();
+			auto r = renderer->Render(0, 0, Tensor(), p, {rays_o, rays_d, cone}, Tensor(), Tensor());
+			auto loss = torch::nn::functional::huber_loss(r.Outputs.RGBMap, target.detach());
+			loss.backward();
+			opt->step();
+			const float new_lr = lr * powf(0.1f, float(global_step) / (lrate_decay * 1000));
+			for (auto& g : opt->param_groups()) g.options().set_lr(new_lr);
+			global_step++;
+			const float lv = loss.template item<float>();
+			secs.push_back(std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count());
+			losses.push_back(lv);
+		}
+		return {secs, losses};
+	}
+	/// kernels of the training graph's last step (0 before the first graph step)
+	int GraphKernels() { return graph ? graph->KernelsPerStep() : 0; }
 };
 
 // The language branch of NeRFExecutor (src/NeRFExecutor.h:458-470, 504-523, 531-535, 640-650, 957-983): second CuHashEmbedder + LeRF + LeRFRenderer
@@ -236,6 +287,8 @@ static void Bind(py::module_& m, const char* name)
 		.def("use_fused_inference", [](P& p, bool on) { p.renderer->UseFusedInference = on; })
 		.def("reuse_coarse_rows", [](P& p, bool on) { p.renderer->ReuseCoarseRows = on; })
 		.def("train_steps", &P::TrainSteps, py::call_guard<py::gil_scoped_release>())
+		.def("train_steps_shipped", &P::TrainStepsShipped, py::call_guard<py::gil_scoped_release>())
+		.def("graph_kernels", &P::GraphKernels)
 		// NeRFExecutor::SaveCheckpoint / the restore branch of Initialize (src/NeRFExecutor.h:1054-1068, 546-553): same file names
 		.def("save_checkpoint", [](P& p, const std::string& dir) {
 			torch::save(p.embed, dir + "/embedder_checkpoint.pt");

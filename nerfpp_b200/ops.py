@@ -139,15 +139,46 @@ def hash_encode_bwd(grid: HashGridSpec, points: torch.Tensor, grad_enc: torch.Te
     return grad_table
 
 
+@dataclass
+class PointJitter:
+    """Per-sample perturbations of the shipped training configuration, applied inside the ray encode kernels (struct nrf_point_jitter).
+    cone_angle: [1] (one scalar) or [R] device tensor, None = thin rays; rand_r / rand_theta [R,S] uniforms (TangentScatter's two torch.rand
+    draws); clamp_to_box: TangentScatter's clamp into the grid's box; sp_noise [R,S,3] standard normal and sp_alpha a [1] device tensor:
+    stochastic preconditioning (None = off)."""
+    cone_angle: torch.Tensor | None = None
+    rand_r: torch.Tensor | None = None
+    rand_theta: torch.Tensor | None = None
+    clamp_to_box: bool = True
+    sp_noise: torch.Tensor | None = None
+    sp_alpha: torch.Tensor | None = None
+
+    def c_struct(self) -> cabi.PointJitter:
+        j = cabi.PointJitter()
+        j.cone_angle = ptr(self.cone_angle, f32)
+        j.cone_stride = 0 if self.cone_angle is None or self.cone_angle.numel() == 1 else 1
+        j.rand_r, j.rand_theta = ptr(self.rand_r, f32), ptr(self.rand_theta, f32)
+        j.clamp_to_box = int(self.clamp_to_box)
+        j.sp_noise, j.sp_alpha = ptr(self.sp_noise, f32), ptr(self.sp_alpha, f32)
+        return j
+
+
 def hash_encode_rays_fwd(grid: HashGridSpec, table_f16: torch.Tensor, ray_batch: torch.Tensor, z: torch.Tensor, clamp: bool = True,
-                         out_f16: bool = True, reuse=None, ray_group: int = 1):
+                         out_f16: bool = True, reuse=None, ray_group: int = 1, jitter: PointJitter | None = None):
     """Fused point generation + encode.  reuse = (perm [R,S] int16, enc_prev [R*S_prev, D] | None, keep_prev [R*S_prev] | None, S_prev).
-    ray_group > 1: the kernel walks the same sample of ray_group neighbouring rays together (rays of a rendered frame); same results."""
+    ray_group > 1: the kernel walks the same sample of ray_group neighbouring rays together (rays of a rendered frame); same results.
+    jitter: the points are perturbed in-kernel (nrf_hash_encode_rays_jitter_fwd); not combinable with reuse / ray_group."""
     r, s = z.shape
     d = grid.n_levels * grid.n_features
     out = torch.empty((r * s, d), dtype=f16 if out_f16 else f32, device=z.device)
     keep = torch.empty(r * s, dtype=u8, device=z.device) if clamp else None
     g = grid.c_struct()
+    if jitter is not None:
+        if reuse is not None or ray_group != 1:
+            raise cabi.NrfError("jittered points take neither row reuse nor ray grouping")
+        j = jitter.c_struct()
+        _run("hash_encode_fwd", lambda: lib().nrf_hash_encode_rays_jitter_fwd(C.byref(g), ptr(table_f16, f16), ptr(ray_batch, f32), ray_batch.shape[1],
+                                        ptr(z, f32), r, s, int(clamp), ptr(keep), ptr(out), cabi.ENC_F16 if out_f16 else cabi.ENC_F32, C.byref(j), stream()))
+        return out, keep
     src, enc_prev, keep_prev, s_prev = reuse if reuse is not None else (None, None, None, 0)
     _run("hash_encode_fwd", lambda: lib().nrf_hash_encode_rays_fwd_grouped(C.byref(g), ptr(table_f16, f16), ptr(ray_batch, f32), ray_batch.shape[1], ptr(z, f32),
                                     r, s, int(clamp), ptr(keep), ptr(out), cabi.ENC_F16 if out_f16 else cabi.ENC_F32, ptr(src, torch.int16) if src is not None else None,
@@ -156,11 +187,19 @@ def hash_encode_rays_fwd(grid: HashGridSpec, table_f16: torch.Tensor, ray_batch:
 
 
 def hash_encode_rays_bwd(grid: HashGridSpec, ray_batch: torch.Tensor, z: torch.Tensor, grad_enc: torch.Tensor, grad_table: torch.Tensor,
-                         clamp: bool = True, levels: tuple[int, int] | None = None) -> torch.Tensor:
-    """levels = (begin, end): scatter those levels only (two calls over [0, k) and [k, L) add up to the full gradient)."""
+                         clamp: bool = True, levels: tuple[int, int] | None = None, jitter: PointJitter | None = None) -> torch.Tensor:
+    """levels = (begin, end): scatter those levels only (two calls over [0, k) and [k, L) add up to the full gradient).
+    jitter: the forward's perturbed points, re-derived from the same variates (nrf_hash_encode_rays_jitter_bwd; all levels)."""
     r, s = z.shape
     layout = {f32: cabi.GRAD_F32, bf16: cabi.GRAD_BF16}[grad_enc.dtype]
     g = grid.c_struct()
+    if jitter is not None:
+        if levels is not None:
+            raise cabi.NrfError("the jittered scatter covers all levels")
+        j = jitter.c_struct()
+        _run("hash_encode_bwd", lambda: lib().nrf_hash_encode_rays_jitter_bwd(C.byref(g), ptr(ray_batch, f32), ray_batch.shape[1], ptr(z, f32), r, s,
+                                        int(clamp), ptr(grad_enc), layout, ptr(grad_table, f32), C.byref(j), stream()))
+        return grad_table
     lb, le = levels if levels is not None else (0, -1)
     _run("hash_encode_bwd", lambda: lib().nrf_hash_encode_rays_bwd_levels(C.byref(g), ptr(ray_batch, f32), ray_batch.shape[1], ptr(z, f32), r, s, int(clamp),
                                     ptr(grad_enc), layout, ptr(grad_table, f32), lb, le, stream()))

@@ -42,40 +42,6 @@ struct __align__(128) ChainSmem {
 	uint32_t tmem_base;
 };
 
-__device__ __forceinline__ void tmem_st8(uint32_t taddr, const uint32_t (&r)[8])
-{
-	asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};"
-		::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]) : "memory");
-}
-__device__ __forceinline__ void tmem_ld_wait_for16b(uint32_t (&r)[16])
-{
-	asm volatile("tcgen05.wait::ld.sync.aligned;"
-		: "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3]), "+r"(r[4]), "+r"(r[5]), "+r"(r[6]), "+r"(r[7]), "+r"(r[8]), "+r"(r[9]), "+r"(r[10]),
-		  "+r"(r[11]), "+r"(r[12]), "+r"(r[13]), "+r"(r[14]), "+r"(r[15])
-		:: "memory");
-}
-__device__ __forceinline__ void publish_chain(uint64_t* bar, int lane)
-{
-	tmem_st_wait();
-	fence_before();
-	__syncwarp();
-	if (lane == 0) mbar_arrive(bar);
-}
-__device__ __forceinline__ void store_chunks4(uint8_t* __restrict__ region_row, int first_chunk, const uint32_t (&a16)[16])
-{
-#pragma unroll
-	for (int i = 0; i < 4; i++)
-		*reinterpret_cast<uint4*>(region_row + (first_chunk + i) * 1024) = make_uint4(a16[4 * i], a16[4 * i + 1], a16[4 * i + 2], a16[4 * i + 3]);
-}
-
-// KSTEPS K = 16 steps of one accumulator block with an MN-major B operand: A advances 8 TMEM columns, the B descriptor 256 bytes (16 output rows) per step
-template <int KSTEPS>
-__device__ __forceinline__ void issue_mn(uint32_t d, uint32_t a0, uint64_t b0, uint32_t idesc, uint32_t acc_first)
-{
-#pragma unroll
-	for (int j = 0; j < KSTEPS; j++) umma_ts(d, a0 + 8 * j, b0 + static_cast<uint64_t>(16 * j), idesc, j ? 1u : acc_first);
-}
-
 __global__ void __launch_bounds__(kChainThreads, 1) lerf_bwd_chain_kernel(const uint8_t* __restrict__ blob, const uint8_t* __restrict__ saved,
 	const uint8_t* __restrict__ keep, const float* __restrict__ d_raw4, const float2* __restrict__ coef, const float* __restrict__ u, int32_t n_samples,
 	int64_t n, uint8_t* __restrict__ grads, uint4* __restrict__ d_enc)
@@ -132,14 +98,14 @@ __global__ void __launch_bounds__(kChainThreads, 1) lerf_bwd_chain_kernel(const 
 			// ---- step 0: t = h2 G (fp16 operands, K-major B, as in the forward): 4 stages x 4 K steps, N = 256
 			mbar_wait(&sm.a_ready, pa); pa ^= 1u; fence_after();
 			{
-				const uint32_t idesc = idesc16(128, kHid, false, 0, 0), lbo = kHid * 16;
+				const uint32_t id = idesc(128, kHid, false, 0, 0), lbo = kHid * 16;
 				uint32_t a_col = tmem + kCH2;
 				for (int s = 0; s < 4; s++) {
 					const uint32_t slot = next_stage();
 					const uint32_t saddr = smem_u32(sm.ring[slot]);
 					if (leader) {
 #pragma unroll
-						for (int j = 0; j < 4; j++) umma_ts(tmem + kCD, a_col + 8 * j, smem_desc(saddr + j * 2 * lbo, lbo, 128), idesc, (s | j) ? 1u : 0u);
+						for (int j = 0; j < 4; j++) umma_ts(tmem + kCD, a_col + 8 * j, smem_desc(saddr + j * 2 * lbo, lbo, 128), id, (s | j) ? 1u : 0u);
 						umma_commit(&sm.empty[slot]);
 					}
 					__syncwarp();
@@ -154,7 +120,7 @@ __global__ void __launch_bounds__(kChainThreads, 1) lerf_bwd_chain_kernel(const 
 				const uint32_t slot = next_stage();
 				const uint64_t b0 = smem_desc(smem_u32(sm.ring[slot]), 128, kHid * 16);
 				if (leader) {
-					issue_mn<16>(tmem + kCD + 64 * s, tmem + kCA, b0, idesc16(128, s == 2 ? 32 : 64, true, 0, 1), 0u);
+					issue_k<16>(tmem + kCD + 64 * s, tmem + kCA, b0, idesc(128, s == 2 ? 32 : 64, true, 0, 1), 0u);
 					umma_commit(&sm.empty[slot]);
 				}
 				__syncwarp();
@@ -167,7 +133,7 @@ __global__ void __launch_bounds__(kChainThreads, 1) lerf_bwd_chain_kernel(const 
 				const uint32_t slot = next_stage();
 				const uint64_t b0 = smem_desc(smem_u32(sm.ring[slot]), 128, kSigN * 16);
 				if (leader) {
-					issue_mn<3>(tmem + kCD2, tmem + kCS, b0, idesc16(128, kHid, true, 0, 1), 0u);
+					issue_k<3>(tmem + kCD2, tmem + kCS, b0, idesc(128, kHid, true, 0, 1), 0u);
 					umma_commit(&sm.empty[slot]);
 					umma_commit(&sm.d_ready);
 				}
@@ -179,7 +145,7 @@ __global__ void __launch_bounds__(kChainThreads, 1) lerf_bwd_chain_kernel(const 
 				const uint32_t slot = next_stage();
 				const uint64_t b0 = smem_desc(smem_u32(sm.ring[slot]), 128, kHid * 16);
 				if (leader) {
-					issue_mn<16>(tmem + kCD + 64 * s, tmem + kCA, b0, idesc16(128, 64, true, 0, 1), 1u);
+					issue_k<16>(tmem + kCD + 64 * s, tmem + kCA, b0, idesc(128, 64, true, 0, 1), 1u);
 					umma_commit(&sm.empty[slot]);
 				}
 				__syncwarp();
@@ -217,7 +183,7 @@ __global__ void __launch_bounds__(kChainThreads, 1) lerf_bwd_chain_kernel(const 
 					tmem_st16(t_lane + kCH2 + 16 * c, a16);
 				}
 			}
-			publish_chain(&sm.a_ready, lane);
+			publish(&sm.a_ready, lane);
 
 			// ---- step 0: d a2 = (c u - beta t) * [h2 > 0]  (-> A operand + record), beta h2 (-> record)
 			mbar_wait(&sm.d_ready, pd); pd ^= 1u; fence_after();
@@ -238,7 +204,7 @@ __global__ void __launch_bounds__(kChainThreads, 1) lerf_bwd_chain_kernel(const 
 				for (int cc = 0; cc < 4; cc++) {
 					const int c = 4 * half + cc, b = cc & 1;
 					tmem_ld_wait_for(acc[b]);
-					tmem_ld_wait_for16b(hh[b]);
+					tmem_ld_wait_for(hh[b]);
 					if (cc + 1 < 4) fetch(c + 1, b ^ 1);         // the next chunk's TMEM / L1 reads fly under this chunk's arithmetic and stores
 					uint32_t a16[16], b16[16];
 #pragma unroll
@@ -252,11 +218,11 @@ __global__ void __launch_bounds__(kChainThreads, 1) lerf_bwd_chain_kernel(const 
 						b16[i] = pack_bf16(cb.y * h_lo, cb.y * h_hi);
 					}
 					tmem_st16(t_lane + kCA + 16 * c, a16);
-					store_chunks4(da2_row, 4 * c, a16);
-					store_chunks4(bh2_row, 4 * c, b16);
+					store_chunks(da2_row, 4 * c, a16);
+					store_chunks(bh2_row, 4 * c, b16);
 				}
 			}
-			publish_chain(&sm.a_ready, lane);
+			publish(&sm.a_ready, lane);
 
 			// ---- step 1: d g (accumulator columns 128..159) -> d s = [d g 32 | d sigma | 0..] (48 columns: A operand of step 2 + record)
 			mbar_wait(&sm.d_ready, pd); pd ^= 1u; fence_after();
@@ -274,11 +240,11 @@ __global__ void __launch_bounds__(kChainThreads, 1) lerf_bwd_chain_kernel(const 
 				tmem_st16(t_lane + kCS, a16);
 				tmem_st8(t_lane + kCS + 16, tail);
 				uint8_t* const ds_row = rec_g + kGradS + chunk_offset(kSigN, row, 0);
-				store_chunks4(ds_row, 0, a16);
+				store_chunks(ds_row, 0, a16);
 				*reinterpret_cast<uint4*>(ds_row + 4 * 1024) = make_uint4(tail[0], 0u, 0u, 0u);
 				*reinterpret_cast<uint4*>(ds_row + 5 * 1024) = make_uint4(0u, 0u, 0u, 0u);
 			}
-			publish_chain(&sm.a_ready, lane);
+			publish(&sm.a_ready, lane);
 
 			// ---- step 2: d a1 = d h1 * [h1 > 0] + record.  The bf16 pairs of chunk c go to columns 256 + 16 c: inside the accumulator columns of chunk
 			// c / 2, which belong to the OTHER half for c >= 4 — so both halves first read all their chunks, meet, and only then overwrite.
@@ -301,7 +267,7 @@ __global__ void __launch_bounds__(kChainThreads, 1) lerf_bwd_chain_kernel(const 
 						w &= ((bits[cc] >> i) & 0x00010001u) * 0xFFFFu;
 						packed[cc][i] = w;
 					}
-					store_chunks4(da1_row, 4 * c, packed[cc]);
+					store_chunks(da1_row, 4 * c, packed[cc]);
 				}
 				fence_before();
 				asm volatile("bar.sync 1, 256;" ::: "memory");       // all 8 epilogue warps: every tcgen05.ld of the d h1 accumulator has completed
@@ -309,7 +275,7 @@ __global__ void __launch_bounds__(kChainThreads, 1) lerf_bwd_chain_kernel(const 
 #pragma unroll
 				for (int cc = 0; cc < 4; cc++) tmem_st16(t_lane + kCA + 16 * (4 * half + cc), packed[cc]);
 			}
-			publish_chain(&sm.a_ready, lane);
+			publish(&sm.a_ready, lane);
 
 			// ---- step 3: d x (accumulator columns 0..127) -> bf16 [N, 128] row-major, the layout nrf_hash_encode_bwd reads
 			mbar_wait(&sm.d_ready, pd); pd ^= 1u; fence_after();

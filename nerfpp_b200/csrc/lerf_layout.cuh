@@ -14,7 +14,6 @@
 // their 16-bit format (a mixed descriptor faults on B200), so the weight-gradient products dW = dY^T X read BF16 copies of the activations.
 #pragma once
 #include "tcgen05.cuh"
-#include "mlp_small_layout.cuh"   // pack_f16 / pack_bf16 (+ relu variants)
 
 namespace nrf {
 namespace lerf_tc {
@@ -98,14 +97,8 @@ static_assert(make_mode(kSigma).n_stages == 3 && make_mode(kHidden).n_stages == 
 // h2 tile records of the HIDDEN program (inference): [32 column chunks][128 rows][8 fp16] = 64 KB per 128-row tile; a warp store covers 512 contiguous bytes
 constexpr int kHiddenTile = 128 * kHid * 2;
 
-// ---- training records, one per 128-row tile, made of regions of C columns stored as [row half (2)][C/8 column chunks][64 rows][8 elements]:
-// a 64-row half of a region is contiguous and is at the same time the MN-major A operand (M = columns, K = rows) and the MN-major B operand
-// (N = columns, K = rows) of a weight-gradient product dW = dY^T X (SBO 1024, LBO 128) — the classic-NeRF record layout (mlp_nerf_layout.cuh).
-__host__ __device__ constexpr int region_bytes(int cols) { return 128 * cols * 2; }
-__host__ __device__ constexpr uint32_t chunk_offset(int cols, int r, int chunk)
-{
-	return static_cast<uint32_t>((r >> 6) * (cols * 128) + chunk * 1024 + (r & 63) * 16);
-}
+// ---- training records, one per 128-row tile, made of regions of C columns in the record layout of tcgen05.cuh (region_bytes / chunk_offset):
+// a 64-row half of a region is the MN-major A or B operand of a weight-gradient product dW = dY^T X.
 // saved by the training forward: bf16 copies of [geo 32 | x 128] (the input of le_net[0]), h1 and h2 (B / A operands of the weight-gradient
 // products), h2 once more in fp16 (what the forward itself multiplied: the A operand of the chain's G h2 product and the source of the per-ray
 // sums, whose rounding the density gradient — a cancellation-prone residual of the compositing backward — amplifies), and the ReLU mask of h1
@@ -124,12 +117,6 @@ constexpr int kGradA1 = kGradS + region_bytes(kSigN);
 constexpr int kGradBH2 = kGradA1 + region_bytes(kHid);
 constexpr int kGradTile = kGradBH2 + region_bytes(kHid);         // 208 896 B per 128 rows
 
-// instruction descriptor, kind::f16, D fp32; A/B both fp16 (bf16 = false) or both bf16; majors: 0 = K, 1 = MN
-__host__ __device__ constexpr uint32_t idesc16(int M, int N, bool bf16, int a_mn, int b_mn)
-{
-	return (1u << 4) | (bf16 ? (1u << 7) | (1u << 10) : 0u) | (uint32_t(a_mn) << 15) | (uint32_t(b_mn) << 16) | (uint32_t(N >> 3) << 17) |
-	       (uint32_t(M >> 4) << 24);
-}
 __device__ __forceinline__ float2 half2_bits_to_float2(uint32_t w) { return __half22float2(*reinterpret_cast<const __half2*>(&w)); }
 __device__ __forceinline__ uint32_t half2_bits_to_bf16x2(uint32_t w)
 {

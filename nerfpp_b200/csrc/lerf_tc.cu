@@ -103,8 +103,7 @@ __global__ void __launch_bounds__(256) lerf_pack_kernel(Weights p, uint32_t* __r
 		while (l + 1 < 4 && wt * 4 >= layer_offset(l + 1)) l++;
 		int q = wt - layer_offset(l) / 4, st = 0, k_off = 0;
 		while (q >= stage_bytes(l, st) / 4) { q -= stage_bytes(l, st) / 4; k_off += stage_k(l, st); st++; }
-		const int N = layer_info(l).N;
-		const int kc = q / (4 * N), n = (q >> 2) % N, k = k_off + 8 * kc + 2 * (q & 3);
+		const auto [n, k] = stage_word(q, layer_info(l).N, k_off);
 		// W_e0 travels with its input columns as [x 128 | geo 32] in the training copy (lerf_bwd_tc.cu: the two products that meet in d x then
 		// write the same accumulator blocks); pairs (k, k + 1) never straddle the boundary
 		const int ks = l == 2 ? (k < kIn ? k + kGeo : k - kIn) : k;
@@ -115,9 +114,7 @@ __global__ void __launch_bounds__(256) lerf_pack_kernel(Weights p, uint32_t* __r
 	while (l + 1 < kLayers && w * 4 >= layer_offset(l + 1)) l++;
 	int q = w - layer_offset(l) / 4, s = 0, k_off = 0;
 	while (q >= stage_bytes(l, s) / 4) { q -= stage_bytes(l, s) / 4; k_off += stage_k(l, s); s++; }
-	// UMMA K-major core-matrix layout: word q of a stage holds (n, k) and (n, k+1); byte = (k/8)*(N*16) + n*16 + (k%8)*2
-	const int N = layer_info(l).N;
-	const int kc = q / (4 * N), n = (q >> 2) % N, k = k_off + 8 * kc + 2 * (q & 3);
+	const auto [n, k] = stage_word(q, layer_info(l).N, k_off);
 	blob[w] = pack_f16(wp(p, gram, l, n, k, g_inv), wp(p, gram, l, n, k + 1, g_inv));
 }
 
@@ -129,27 +126,6 @@ struct __align__(128) Smem {
 	uint64_t a_ready, d_ready;
 	uint32_t tmem_base;
 };
-
-// tcgen05.wait::ld tied to the destination registers of a narrower load (see tmem_ld_wait_for in tcgen05.cuh)
-__device__ __forceinline__ void tmem_ld_wait_for4(uint32_t (&r)[4])
-{
-	asm volatile("tcgen05.wait::ld.sync.aligned;" : "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3]) :: "memory");
-}
-__device__ __forceinline__ void tmem_ld_wait_for16(uint32_t (&r)[16])
-{
-	asm volatile("tcgen05.wait::ld.sync.aligned;"
-		: "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3]), "+r"(r[4]), "+r"(r[5]), "+r"(r[6]), "+r"(r[7]), "+r"(r[8]), "+r"(r[9]), "+r"(r[10]),
-		  "+r"(r[11]), "+r"(r[12]), "+r"(r[13]), "+r"(r[14]), "+r"(r[15])
-		:: "memory");
-}
-
-__device__ __forceinline__ void publish(uint64_t* bar, int lane)
-{
-	tmem_st_wait();
-	fence_before();
-	__syncwarp();
-	if (lane == 0) mbar_arrive(bar);
-}
 
 // Epilogue helpers.  HV = warps per TMEM lane quarter (1: four epilogue warps, one thread per row does all 256 accumulator columns;
 // 2: eight warps, warps w and w + 4 share a quarter and each takes 128 columns).  c0 = first 32-column chunk of this warp, CH = 8 / HV chunks.
@@ -261,7 +237,7 @@ __device__ __forceinline__ float dot_d_h(uint32_t t_lane, int c0)
 		tmem_ld32(t_lane + kColD + 32 * c, acc);
 		tmem_ld16(t_lane + kColH + 16 * c, hh);
 		tmem_ld_wait_for(acc);
-		tmem_ld_wait_for16(hh);
+		tmem_ld_wait_for(hh);
 #pragma unroll
 		for (int i = 0; i < 16; i++) {
 			const float2 h2 = BF16 ? make_float2(__uint_as_float(hh[i] << 16), __uint_as_float(hh[i] & 0xFFFF0000u))
@@ -360,7 +336,7 @@ __global__ void __launch_bounds__(32 * (2 + 4 * HV), 1) lerf_fwd_tc_kernel(const
 					fence_after();
 					const int l = mt.group_layer[grp];
 					const LayerInfo L = layer_info(l);
-					const uint32_t idesc = idesc16(128, L.N, false, 0, 0);
+					const uint32_t id = idesc(128, L.N, false, 0, 0);
 					const uint32_t lbo = L.N * 16;
 					uint32_t a_col = tmem + L.a_col;
 					bool first = true;
@@ -372,7 +348,7 @@ __global__ void __launch_bounds__(32 * (2 + 4 * HV), 1) lerf_fwd_tc_kernel(const
 						const uint32_t saddr = smem_u32(sm.ring[slot]);
 						const int ks = stage_k(l, s) / 16;
 						for (int j = 0; j < ks; j++) {
-							umma_ts(tmem + L.d_col, a_col, smem_desc(saddr + j * 2 * lbo, lbo, 128), idesc, first ? 0u : 1u);
+							umma_ts(tmem + L.d_col, a_col, smem_desc(saddr + j * 2 * lbo, lbo, 128), id, first ? 0u : 1u);
 							first = false;
 							a_col += 8;
 						}
@@ -462,7 +438,7 @@ __global__ void __launch_bounds__(32 * (2 + 4 * HV), 1) lerf_fwd_tc_kernel(const
 									pack_bf16(__uint_as_float(acc[8 * i + 4]), __uint_as_float(acc[8 * i + 5])), pack_bf16(__uint_as_float(acc[8 * i + 6]), __uint_as_float(acc[8 * i + 7])));
 					}
 				}
-				tmem_ld_wait_for4(c4);
+				tmem_ld_wait_for(c4);
 				sigma = __uint_as_float(c4[0]);
 				if (keep != nullptr && ok && keep[r] == 0) sigma = 0.f;               // src/LeRFRenderer.cpp:18-20
 				if (MODE != kRaw) {

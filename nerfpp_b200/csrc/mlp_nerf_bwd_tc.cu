@@ -26,8 +26,6 @@
 namespace nrf {
 namespace nerf_tc {
 
-using namespace tc;
-
 constexpr int kBwdThreads = 32 * 6;
 // TMEM columns of the chain kernel: D fp32 [128 x 256] and TWO A buffers of bf16 [128 x 256] (128 columns each): step st reads
 // A[st & 1] and its epilogue writes A[(st + 1) & 1] slab by slab while the MMAs of the later slabs still read the old operand.
@@ -71,21 +69,6 @@ struct __align__(128) ChainSmem {
 	uint32_t tmem_base;
 };
 
-__device__ __forceinline__ void publish_bwd(uint64_t* bar, int lane)
-{
-	tmem_st_wait();
-	fence_before();
-	__syncwarp();
-	if (lane == 0) mbar_arrive(bar);
-}
-
-__device__ __forceinline__ void store_chunks4(uint8_t* __restrict__ region_row, int first_chunk, const uint32_t (&a16)[16])
-{
-#pragma unroll
-	for (int i = 0; i < 4; i++)
-		*reinterpret_cast<uint4*>(region_row + (first_chunk + i) * 1024) = make_uint4(a16[4 * i], a16[4 * i + 1], a16[4 * i + 2], a16[4 * i + 3]);
-}
-
 #ifdef NRF_PROFILE_CHAIN
 // debug build only (NRF_NVCC_EXTRA=-DNRF_PROFILE_CHAIN): per-CTA cycle counters of the chain kernel, read back by nrf_debug_chain_profile
 __device__ unsigned long long g_chain_prof[kNumSMs][8];
@@ -127,11 +110,11 @@ __device__ __forceinline__ void epilogue_grad(uint32_t t_lane, uint64_t* slab_re
 		tmem_ld32(t_lane + kBD + 64 * sl + 32, acc1);
 		grad_pack<MASK>(acc0, bits[2 * sl], a16);
 		if (to_tmem) tmem_st16(t_lane + a_next + 32 * sl, a16);
-		store_chunks4(out_row, 8 * sl, a16);
+		store_chunks(out_row, 8 * sl, a16);
 		tmem_ld_wait_for(acc1);
 		grad_pack<MASK>(acc1, bits[2 * sl + 1], a16);
 		if (to_tmem) tmem_st16(t_lane + a_next + 32 * sl + 16, a16);
-		store_chunks4(out_row, 8 * sl + 4, a16);
+		store_chunks(out_row, 8 * sl + 4, a16);
 		if (threadIdx.x == 64) CH_ADD(4);
 	}
 }
@@ -144,14 +127,6 @@ __device__ __forceinline__ void load_bits(const uint8_t* __restrict__ bits_row, 
 		const uint4 hi = __ldg(reinterpret_cast<const uint4*>(bits_row) + 1);
 		b[4] = hi.x; b[5] = hi.y; b[6] = hi.z; b[7] = hi.w;
 	}
-}
-
-// KSTEPS K = 16 steps of one accumulator slab: A advances 8 TMEM columns, the MN-major B descriptor 256 bytes (16 output rows) per step
-template <int KSTEPS>
-__device__ __forceinline__ void issue_k(uint32_t d, uint32_t a0, uint64_t b0, uint32_t idesc)
-{
-#pragma unroll
-	for (int j = 0; j < KSTEPS; j++) umma_ts(d, a0 + 8 * j, b0 + static_cast<uint64_t>(16 * j), idesc, j ? 1u : 0u);
 }
 
 __global__ void __launch_bounds__(kBwdThreads, 1) mlp_nerf_bwd_chain_kernel(const uint8_t* __restrict__ blob, const uint8_t* __restrict__ saved,
@@ -215,7 +190,7 @@ __global__ void __launch_bounds__(kBwdThreads, 1) mlp_nerf_bwd_chain_kernel(cons
 					mbar_wait(&sm.full[slot], round & 1u);
 					fence_after();
 					if (leader) {
-						umma_ts(tmem + kBD, tmem + kBRgb, smem_desc(smem_u32(sm.ring[slot]), 128, 16 * 16), idesc_16(128, 128, true, 0, 1), 0u);
+						umma_ts(tmem + kBD, tmem + kBRgb, smem_desc(smem_u32(sm.ring[slot]), 128, 16 * 16), idesc(128, 128, true, 0, 1), 0u);
 						umma_commit(&sm.empty[slot]);
 						for (int s = 0; s < 4; s++) umma_commit(&sm.slab_ready[s]);
 					}
@@ -223,7 +198,7 @@ __global__ void __launch_bounds__(kBwdThreads, 1) mlp_nerf_bwd_chain_kernel(cons
 					g++;
 				} else {
 					const int n_out = layer_info(l).N;               // K of this product
-					const uint32_t idesc = idesc_16(128, 64, true, 0, 1);
+					const uint32_t id = idesc(128, 64, true, 0, 1);
 					for (int s = 0; s < 4; s++, g++) {
 						const uint32_t slot = g % kChainRing, round = g / kChainRing;
 						{ CH_T0(); mbar_wait(&sm.full[slot], round & 1u); if (leader) CH_ADD(1); }
@@ -234,8 +209,8 @@ __global__ void __launch_bounds__(kBwdThreads, 1) mlp_nerf_bwd_chain_kernel(cons
 						const uint64_t b0 = smem_desc(smem_u32(sm.ring[slot]), 128, n_out * 16);
 						const uint32_t d = tmem + kBD + 64 * s, a0 = tmem + a_buf(st);
 						if (leader) {
-							if (n_out == 256) issue_k<16>(d, a0, b0, idesc);
-							else issue_k<8>(d, a0, b0, idesc);
+							if (n_out == 256) issue_k<16>(d, a0, b0, id, 0u);
+							else issue_k<8>(d, a0, b0, id, 0u);
 							umma_commit(&sm.empty[slot]);
 							if (st != 2) umma_commit(&sm.slab_ready[s]);     // this 64-column slab of D is complete
 							CH_ADD(2);
@@ -248,7 +223,7 @@ __global__ void __launch_bounds__(kBwdThreads, 1) mlp_nerf_bwd_chain_kernel(cons
 						mbar_wait(&sm.full[slot], round & 1u);
 						fence_after();
 						if (leader) {
-							umma_ts(tmem + kBD, tmem + kBAlpha, smem_desc(smem_u32(sm.ring[slot]), 128, 16 * 16), idesc_16(128, 256, true, 0, 1), 1u);
+							umma_ts(tmem + kBD, tmem + kBAlpha, smem_desc(smem_u32(sm.ring[slot]), 128, 16 * 16), idesc(128, 256, true, 0, 1), 1u);
 							umma_commit(&sm.empty[slot]);
 							for (int s = 0; s < 4; s++) umma_commit(&sm.slab_ready[s]);
 						}
@@ -290,7 +265,7 @@ __global__ void __launch_bounds__(kBwdThreads, 1) mlp_nerf_bwd_chain_kernel(cons
 				*reinterpret_cast<uint4*>(o + 1024) = make_uint4(0u, 0u, 0u, 0u);
 			}
 			load_bits(rec_s + bits_offset(0, row), false, bits);
-			publish_bwd(&sm.a_ready, lane);
+			publish(&sm.a_ready, lane);
 
 #pragma unroll 1
 			for (int st = 0; st < kSteps; st++) {
@@ -307,7 +282,7 @@ __global__ void __launch_bounds__(kBwdThreads, 1) mlp_nerf_bwd_chain_kernel(cons
 					// the 32 mask bytes of the next step (h_8 after step 1, then h_7 .. h_1), requested before that step's MMAs are even issued
 					CH_T0();
 					if (st >= 1) load_bits(rec_s + bits_offset(st == 1 ? 8 : (st == 2 ? 8 : 10 - st) - 1, row), true, bits);
-					publish_bwd(&sm.a_ready, lane);
+					publish(&sm.a_ready, lane);
 				}
 			}
 		}
@@ -428,7 +403,7 @@ __global__ void __launch_bounds__(kBwdThreads, 1) mlp_nerf_bwd_dw_kernel(const _
 				fence_after();
 				// both operands bf16, MN-major.  (A and B of a tcgen05.mma kind::f16 must carry the SAME 16-bit format: an instruction descriptor that
 				// mixes bf16 gradient rows with fp16 activation rows raises an illegal-instruction fault on B200, gpurun_out/r2i.)
-				const uint32_t idesc = idesc_16(128, U.b_cols, true, 1, 1);
+				const uint32_t id = idesc(128, U.b_cols, true, 1, 1);
 				const int mblocks = U.a_cols / 128;
 				for (int64_t i = lo; i < hi; i++, g++) {
 					const uint32_t slot = g % kDwRing, round = g / kDwRing;
@@ -440,12 +415,12 @@ __global__ void __launch_bounds__(kBwdThreads, 1) mlp_nerf_bwd_dw_kernel(const _
 					if (mblocks == 2) {
 #pragma unroll
 						for (int j = 0; j < 4; j++) {
-							umma_ss(tmem, a0 + static_cast<uint64_t>(16 * j), b0 + static_cast<uint64_t>(16 * j), idesc, j ? 1u : acc);
-							umma_ss(tmem + 256, a0 + static_cast<uint64_t>(1024 + 16 * j), b0 + static_cast<uint64_t>(16 * j), idesc, j ? 1u : acc);
+							umma_ss(tmem, a0 + static_cast<uint64_t>(16 * j), b0 + static_cast<uint64_t>(16 * j), id, j ? 1u : acc);
+							umma_ss(tmem + 256, a0 + static_cast<uint64_t>(1024 + 16 * j), b0 + static_cast<uint64_t>(16 * j), id, j ? 1u : acc);
 						}
 					} else {
 #pragma unroll
-						for (int j = 0; j < 4; j++) umma_ss(tmem, a0 + static_cast<uint64_t>(16 * j), b0 + static_cast<uint64_t>(16 * j), idesc, j ? 1u : acc);
+						for (int j = 0; j < 4; j++) umma_ss(tmem, a0 + static_cast<uint64_t>(16 * j), b0 + static_cast<uint64_t>(16 * j), id, j ? 1u : acc);
 					}
 					umma_commit(&sm.empty[slot]);
 				}

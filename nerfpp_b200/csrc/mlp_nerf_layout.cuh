@@ -14,10 +14,11 @@
 // per row (512 contiguous bytes per warp instruction) and the consumer needs ONE bulk copy per operand and stage.
 #pragma once
 #include "tcgen05.cuh"
-#include "mlp_small_layout.cuh"
 
 namespace nrf {
 namespace nerf_tc {
+
+using namespace tc;
 
 constexpr int kW = 256, kInPts = 63, kInViews = 27, kInCh = kInPts + kInViews;
 
@@ -77,13 +78,7 @@ constexpr int kPackedBytes = kWeightBytes + kBiasFloats * 4;
 constexpr int kRing = 4;
 constexpr int kStageBytes = 256 * 64 * 2;       // largest stage: N = 256, K = 64
 
-// ---- training scratch: per-tile records -------------------------------------------------------------------------------
-__host__ __device__ constexpr int region_bytes(int cols) { return 128 * cols * 2; }
-// byte offset of the 16-byte chunk (row r, columns 8*chunk ..) inside a region of `cols` columns
-__host__ __device__ constexpr uint32_t chunk_offset(int cols, int r, int chunk)
-{
-	return static_cast<uint32_t>((r >> 6) * (cols * 128) + chunk * 1024 + (r & 63) * 16);
-}
+// ---- training scratch: per-tile records (region_bytes / chunk_offset: tcgen05.cuh) ------------------------------------
 // saved activations (operands of the weight-gradient products): pts(64) views(32) h1..h8 (256 each: h_l = input of pts_linears[l]; h8 feeds feature / alpha) feature(256) hv(128)
 constexpr int kSavePts = 0;
 constexpr int kSaveViews = kSavePts + region_bytes(64);
@@ -113,13 +108,6 @@ struct Grads {     // same order, accumulated into (+=)
 };
 
 int check_shape(const nrf_mlp_nerf_shape* s);
-
-// instruction descriptor, kind::f16, D fp32; A/B both fp16 (BF16 = false) or both bf16; majors: 0 = K, 1 = MN
-__host__ __device__ constexpr uint32_t idesc_16(int M, int N, bool bf16, int a_mn, int b_mn)
-{
-	return (1u << 4) | (bf16 ? (1u << 7) | (1u << 10) : 0u) | (uint32_t(a_mn) << 15) | (uint32_t(b_mn) << 16) | (uint32_t(N >> 3) << 17) |
-	       (uint32_t(M >> 4) << 24);
-}
 
 }  // namespace nerf_tc
 }  // namespace nrf

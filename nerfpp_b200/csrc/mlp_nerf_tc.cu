@@ -22,8 +22,6 @@
 namespace nrf {
 namespace nerf_tc {
 
-using namespace tc;
-
 constexpr int kThreads = 32 * 6;
 constexpr int kStagePitch = 98;      // 16-bit elements per staged row (96 used): 49 words, odd, so the per-row accesses are conflict-free
 
@@ -57,9 +55,7 @@ __global__ void __launch_bounds__(256) nerf_pack_kernel(Weights p, uint32_t* __r
 	while (l + 1 < kLayers && w * 4 >= layer_offset(l + 1)) l++;
 	int q = w - layer_offset(l) / 4, s = 0, k_off = 0;
 	while (q >= stage_bytes(l, s) / 4) { q -= stage_bytes(l, s) / 4; k_off += stage_k(l, s); s++; }
-	// UMMA K-major core-matrix layout: word q of a stage holds (n, k) and (n, k+1); byte = (k/8)*(N*16) + n*16 + (k%8)*2
-	const int N = layer_info(l).N;
-	const int kc = q / (4 * N), n = (q >> 2) % N, k = k_off + 8 * kc + 2 * (q & 3);
+	const auto [n, k] = stage_word(q, layer_info(l).N, k_off);
 	blob[w] = bf16 ? pack_bf16(wp(p, l, n, k), wp(p, l, n, k + 1)) : pack_f16(wp(p, l, n, k), wp(p, l, n, k + 1));
 }
 
@@ -108,16 +104,6 @@ __device__ __forceinline__ void bias_act_pack(const uint32_t (&acc)[32], const f
 	}
 }
 
-// D[:, 0 .. 32*CHUNKS) + bias -> (ReLU) -> fp16 -> the h columns, one thread per row.  The tcgen05.ld of chunk c+1 is in flight while
-// chunk c is converted and stored (two register buffers), so the TMEM read latency is paid once, not once per chunk.
-// 32 packed columns (16 words) of this thread's row -> 4 chunks of a scratch region (TRAIN only)
-__device__ __forceinline__ void save_chunks(uint8_t* __restrict__ region_row, int first_chunk, const uint32_t (&a16)[16])
-{
-#pragma unroll
-	for (int i = 0; i < 4; i++)
-		*reinterpret_cast<uint4*>(region_row + (first_chunk + i) * 1024) = make_uint4(a16[4 * i], a16[4 * i + 1], a16[4 * i + 2], a16[4 * i + 3]);
-}
-
 // ReLU mask word of 32 packed columns: bit i / 16+i = low / high half of pair i is non-zero (values are >= 0 after ReLU)
 __device__ __forceinline__ uint32_t relu_bits(const uint32_t (&a16)[16])
 {
@@ -127,6 +113,9 @@ __device__ __forceinline__ uint32_t relu_bits(const uint32_t (&a16)[16])
 	return bits;
 }
 
+// D[:, 0 .. 32*CHUNKS) + bias -> (ReLU) -> fp16 -> the h columns, one thread per row.  The tcgen05.ld of chunk c+1 is in flight while
+// chunk c is converted and stored (two register buffers), so the TMEM read latency is paid once, not once per chunk.  TRAIN: the packed
+// columns also go to the scratch record (save_row) and, RELU, their mask words to bits_row.
 template <int CHUNKS, bool RELU, bool TRAIN>
 __device__ __forceinline__ void epilogue_to_h(uint32_t t_lane, const float* __restrict__ bias, uint8_t* __restrict__ save_row, uint8_t* __restrict__ bits_row)
 {
@@ -139,14 +128,14 @@ __device__ __forceinline__ void epilogue_to_h(uint32_t t_lane, const float* __re
 		if (c + 1 < CHUNKS) tmem_ld32(t_lane + kColD + 32 * (c + 1), acc1);
 		bias_act_pack<RELU, TRAIN>(acc0, bias + 32 * c, a16);
 		tmem_st16(t_lane + kColH + 16 * c, a16);
-		if (TRAIN) save_chunks(save_row, 4 * c, a16);
+		if (TRAIN) store_chunks(save_row, 4 * c, a16);
 		if (TRAIN && RELU) bw[c] = relu_bits(a16);
 		if (c + 1 < CHUNKS) {
 			tmem_ld_wait_for(acc1);
 			if (c + 2 < CHUNKS) tmem_ld32(t_lane + kColD + 32 * (c + 2), acc0);
 			bias_act_pack<RELU, TRAIN>(acc1, bias + 32 * (c + 1), a16);
 			tmem_st16(t_lane + kColH + 16 * (c + 1), a16);
-			if (TRAIN) save_chunks(save_row, 4 * (c + 1), a16);
+			if (TRAIN) store_chunks(save_row, 4 * (c + 1), a16);
 			if (TRAIN && RELU) bw[c + 1] = relu_bits(a16);
 		}
 	}
@@ -154,14 +143,6 @@ __device__ __forceinline__ void epilogue_to_h(uint32_t t_lane, const float* __re
 #pragma unroll
 		for (int c = 0; c < CHUNKS; c += 4) *reinterpret_cast<uint4*>(bits_row + 4 * c) = make_uint4(bw[c], bw[c + 1], bw[c + 2], bw[c + 3]);
 	}
-}
-
-__device__ __forceinline__ void publish(uint64_t* bar, int lane)
-{
-	tmem_st_wait();
-	fence_before();
-	__syncwarp();
-	if (lane == 0) mbar_arrive(bar);
 }
 
 // groups of layers that share one A operand and one epilogue: {0} {1} {2} {3} {4} {5} {6} {7} {8,9} {10} {11}
@@ -272,7 +253,7 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(kThreads, 1) mlp_ne
 					fence_after();
 					for (int l = group_first(grp); l < group_first(grp) + group_count(grp); l++) {
 						const LayerInfo L = layer_info(l);
-						const uint32_t idesc = idesc_16(128, L.N, TRAIN, 0, 0);
+						const uint32_t id = idesc(128, L.N, TRAIN, 0, 0);
 						const uint32_t lbo = L.N * 16;
 						uint32_t a_col = tmem + L.a_col;
 						bool first = true;
@@ -283,7 +264,7 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(kThreads, 1) mlp_ne
 							const uint32_t saddr = smem_u32(sm.ring[slot]);
 							const int ks = stage_k(l, s) / 16;
 							for (int j = 0; j < ks; j++) {
-								umma_ts(tmem + L.d_col, a_col, smem_desc(saddr + j * 2 * lbo, lbo, 128), idesc, first ? 0u : 1u);
+								umma_ts(tmem + L.d_col, a_col, smem_desc(saddr + j * 2 * lbo, lbo, 128), id, first ? 0u : 1u);
 								first = false;
 								a_col += 8;
 							}
@@ -332,12 +313,12 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(kThreads, 1) mlp_ne
 #pragma unroll
 					for (int i = 0; i < 16; i++) a16[i] = srow32[16 * h + i];
 					tmem_st16(t_lane + kColPts + 16 * h, a16);
-					if (TRAIN) save_chunks(rec + kSavePts + chunk_offset(64, row, 0), 4 * h, a16);
+					if (TRAIN) store_chunks(rec + kSavePts + chunk_offset(64, row, 0), 4 * h, a16);
 				}
 #pragma unroll
 				for (int i = 0; i < 16; i++) a16[i] = srow32[32 + i];
 				tmem_st16(t_lane + kColViews, a16);
-				if (TRAIN) save_chunks(rec + kSaveViews + chunk_offset(32, row, 0), 0, a16);
+				if (TRAIN) store_chunks(rec + kSaveViews + chunk_offset(32, row, 0), 0, a16);
 			} else {
 				const float2* xr = reinterpret_cast<const float2*>(x + (ok ? r : 0) * kInCh);   // rows are 360 B: 8-byte aligned
 				uint32_t a16[16];
@@ -354,7 +335,7 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(kThreads, 1) mlp_ne
 						a16[i] = TRAIN ? pack_bf16(v.x, v.y) : pack_f16(v.x, v.y);
 					}
 					tmem_st16(t_lane + kColPts + 16 * h, a16);
-					if (TRAIN) save_chunks(rec + kSavePts + chunk_offset(64, row, 0), 4 * h, a16);
+					if (TRAIN) store_chunks(rec + kSavePts + chunk_offset(64, row, 0), 4 * h, a16);
 				}
 #pragma unroll
 				for (int i = 0; i < 16; i++) {
@@ -365,7 +346,7 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(kThreads, 1) mlp_ne
 					a16[i] = TRAIN ? pack_bf16(v0, v1) : pack_f16(v0, v1);
 				}
 				tmem_st16(t_lane + kColViews, a16);
-				if (TRAIN) save_chunks(rec + kSaveViews + chunk_offset(32, row, 0), 0, a16);
+				if (TRAIN) store_chunks(rec + kSaveViews + chunk_offset(32, row, 0), 0, a16);
 			}
 			publish(&sm.a_ready, lane);
 

@@ -46,9 +46,8 @@ __global__ void __launch_bounds__(256) mlp_pack_kernel(const float* __restrict__
 		else if (w < kU3) { layer = 2; base = kU2; N = 64; }
 		else if (w < kU4) { layer = 3; base = kU3; N = 64; }
 		else { layer = 4; base = kU4; N = 16; }
-		const int q = w - base;
-		const int kc = q / (4 * N), n = (q >> 2) % N, k = 8 * kc + 2 * (q & 3);
-		blob[w] = pack_f16(wp(p, V, layer, n, k), wp(p, V, layer, n, k + 1));
+		const auto [n, k] = tc::stage_word(w - base, N, 0);
+		blob[w] = tc::pack_f16(wp(p, V, layer, n, k), wp(p, V, layer, n, k + 1));
 		return;
 	}
 	int layer, base, NT;
@@ -83,7 +82,7 @@ __global__ void __launch_bounds__(256) mlp_pack_kernel(const float* __restrict__
 	}
 	// forward operands (activations AND weights) are fp16 on every layer: 10-bit mantissa, 8x fewer ReLU sign flips against
 	// the fp32 reference than bf16; the gradient chain stays bf16 (fp32 range, no loss scale)
-	blob[w] = !bwd ? pack_f16(lo, hi) : pack_bf16(lo, hi);
+	blob[w] = !bwd ? tc::pack_f16(lo, hi) : tc::pack_bf16(lo, hi);
 }
 
 // ---------------------------------------------------------------------------------------------- MMA helpers
@@ -127,7 +126,7 @@ __device__ __forceinline__ void repack(const float (&acc)[2 * KS][4], uint32_t (
 #pragma unroll
 		for (int e = 0; e < 4; e++) {
 			const float lo = acc[2 * ks + (e >> 1)][2 * (e & 1)], hi = acc[2 * ks + (e >> 1)][2 * (e & 1) + 1];
-			a[ks][e] = F16 ? (RELU ? pack_f16_relu(lo, hi) : pack_f16(lo, hi)) : (RELU ? pack_bf16_relu(lo, hi) : pack_bf16(lo, hi));
+			a[ks][e] = F16 ? (RELU ? tc::pack_f16_relu(lo, hi) : tc::pack_f16(lo, hi)) : (RELU ? tc::pack_bf16_relu(lo, hi) : tc::pack_bf16(lo, hi));
 		}
 	}
 }
@@ -136,7 +135,7 @@ __device__ __forceinline__ void repack(const float (&acc)[2 * KS][4], uint32_t (
 __device__ __forceinline__ uint32_t f16x2_to_bf16x2(uint32_t w)
 {
 	const float2 v = __half22float2(*reinterpret_cast<const __half2*>(&w));
-	return pack_bf16(v.x, v.y);
+	return tc::pack_bf16(v.x, v.y);
 }
 template <int KS>
 __device__ __forceinline__ void to_bf16(const uint32_t (&a)[KS][4], uint32_t (&b)[KS][4])
@@ -167,13 +166,13 @@ __device__ __forceinline__ void load_enc(const void* __restrict__ enc, int64_t r
 		for (int ks = 0; ks < 2; ks++) {
 			float2 v;
 			v = r_lo < n ? __ldg(reinterpret_cast<const float2*>(x + r_lo * 48 + ks * 16 + 2 * t)) : make_float2(0.f, 0.f);
-			a[ks][0] = pack_f16(v.x, v.y);
+			a[ks][0] = tc::pack_f16(v.x, v.y);
 			v = r_hi < n ? __ldg(reinterpret_cast<const float2*>(x + r_hi * 48 + ks * 16 + 2 * t)) : make_float2(0.f, 0.f);
-			a[ks][1] = pack_f16(v.x, v.y);
+			a[ks][1] = tc::pack_f16(v.x, v.y);
 			v = r_lo < n ? __ldg(reinterpret_cast<const float2*>(x + r_lo * 48 + ks * 16 + 8 + 2 * t)) : make_float2(0.f, 0.f);
-			a[ks][2] = pack_f16(v.x, v.y);
+			a[ks][2] = tc::pack_f16(v.x, v.y);
 			v = r_hi < n ? __ldg(reinterpret_cast<const float2*>(x + r_hi * 48 + ks * 16 + 8 + 2 * t)) : make_float2(0.f, 0.f);
-			a[ks][3] = pack_f16(v.x, v.y);
+			a[ks][3] = tc::pack_f16(v.x, v.y);
 		}
 	}
 }
@@ -239,9 +238,6 @@ constexpr int kRegionBytes = kCD4 + kBwdRows * 16 * 2;         // 184 320
 // weights + operand regions + the dW mbarrier and the TMEM address slot
 constexpr size_t kBwdSmem = static_cast<size_t>(kBlobWords) * 4 + kRegionBytes + 64;
 constexpr uint32_t kDwT0 = 0, kDwT1 = 64, kDwT2 = 144;        // TMEM columns of the three accumulators
-
-// instruction descriptor: kind::f16, bf16 x bf16 -> fp32, A and B MN-major, M = 128
-__host__ __device__ constexpr uint32_t idesc_mn(int N) { return (1u << 4) | (1u << 7) | (1u << 10) | (1u << 15) | (1u << 16) | (uint32_t(N >> 3) << 17) | (8u << 24); }
 
 // store an A-fragment-shaped register set (KS k-steps) for rows (g, g+8) of this warp's slab into a region, from 8-column chunk chunk0 on
 template <int KS, int CHUNK>
@@ -406,7 +402,7 @@ __global__ void __launch_bounds__(kBwdWarps * 32, 1) mlp_small_bwd_kernel(const 
 			layer_mma<4, 2, true>(a1, wf + kF1, lane, d1);
 			uint32_t a2[2][4];
 #pragma unroll
-			for (int e = 0; e < 4; e++) a2[0][e] = pack_f16(cur_v[e].x, cur_v[e].y);
+			for (int e = 0; e < 4; e++) a2[0][e] = tc::pack_f16(cur_v[e].x, cur_v[e].y);
 			if (t == 0) { d1[0][0] = 0.f; d1[0][2] = 0.f; }
 			repack<1, false, true>(d1, reinterpret_cast<uint32_t(&)[1][4]>(a2[1]));
 			to_bf16<2>(a2, xb2);
@@ -427,8 +423,8 @@ __global__ void __launch_bounds__(kBwdWarps * 32, 1) mlp_small_bwd_kernel(const 
 		// ---- backward chain
 		{
 			uint32_t d4[1][4];
-			d4[0][0] = t == 0 ? pack_bf16(g_lo.x, g_lo.y) : (t == 1 ? pack_bf16(g_lo.z, 0.f) : 0u);
-			d4[0][1] = t == 0 ? pack_bf16(g_hi.x, g_hi.y) : (t == 1 ? pack_bf16(g_hi.z, 0.f) : 0u);
+			d4[0][0] = t == 0 ? tc::pack_bf16(g_lo.x, g_lo.y) : (t == 1 ? tc::pack_bf16(g_lo.z, 0.f) : 0u);
+			d4[0][1] = t == 0 ? tc::pack_bf16(g_hi.x, g_hi.y) : (t == 1 ? tc::pack_bf16(g_hi.z, 0.f) : 0u);
 			d4[0][2] = 0u;
 			d4[0][3] = 0u;
 			store_frag_c<1, kChunk>(ctiles + kCD4, 0, row_g, t, d4);         // 8 real + 8 zero columns
@@ -447,10 +443,10 @@ __global__ void __launch_bounds__(kBwdWarps * 32, 1) mlp_small_bwd_kernel(const 
 			layer_mma<4, 4, false>(d3, wf + kB2, lane, da2);                 // dA2 = dD2 · W2p  (cols 0..15 views, 16..31 d1)
 			if (t == 0) { da2[2][0] += g_lo.w; da2[2][2] += g_hi.w; }        // + d(sigma)
 			uint32_t dd1[1][4];
-			dd1[0][0] = pack_bf16(da2[2][0], da2[2][1]);
-			dd1[0][1] = pack_bf16(da2[2][2], da2[2][3]);
-			dd1[0][2] = pack_bf16(da2[3][0], da2[3][1]);
-			dd1[0][3] = pack_bf16(da2[3][2], da2[3][3]);
+			dd1[0][0] = tc::pack_bf16(da2[2][0], da2[2][1]);
+			dd1[0][1] = tc::pack_bf16(da2[2][2], da2[2][3]);
+			dd1[0][2] = tc::pack_bf16(da2[3][0], da2[3][1]);
+			dd1[0][3] = tc::pack_bf16(da2[3][2], da2[3][3]);
 			store_frag_c<1, kChunk>(ctiles + kCD1, 0, row_g, t, dd1);
 			layer_mma<1, 8, false>(dd1, wf + kB1, lane, acc);                // dA1 = dD1 · W1
 			repack<4, false, false>(acc, d3);
@@ -463,8 +459,8 @@ __global__ void __launch_bounds__(kBwdWarps * 32, 1) mlp_small_bwd_kernel(const 
 					uint32_t* o = reinterpret_cast<uint32_t*>(grad_in);      // bf16 [N,32] = 16 words per row
 #pragma unroll
 					for (int nt = 0; nt < 4; nt++) {
-						if (r_lo < n) o[r_lo * 16 + nt * 4 + t] = pack_bf16(de[nt][0], de[nt][1]);
-						if (r_hi < n) o[r_hi * 16 + nt * 4 + t] = pack_bf16(de[nt][2], de[nt][3]);
+						if (r_lo < n) o[r_lo * 16 + nt * 4 + t] = tc::pack_bf16(de[nt][0], de[nt][1]);
+						if (r_hi < n) o[r_hi * 16 + nt * 4 + t] = tc::pack_bf16(de[nt][2], de[nt][3]);
 					}
 				} else {
 					float* o = reinterpret_cast<float*>(grad_in);            // fp32 [N,48]
@@ -495,9 +491,9 @@ __global__ void __launch_bounds__(kBwdWarps * 32, 1) mlp_small_bwd_kernel(const 
 #pragma unroll
 				for (int j = 0; j < kBwdWarps; j++) {                            // K = 16 rows per step: +256 B on both descriptors
 					const uint64_t o = static_cast<uint64_t>(16 * j);
-					tc::umma_ss(tmem + kDwT0, a1 + o, b1 + o, idesc_mn(64), j ? 1u : first);
-					tc::umma_ss(tmem + kDwT1, a2 + o, b2 + o, idesc_mn(80), j ? 1u : first);
-					tc::umma_ss(tmem + kDwT2, a3 + o, b3 + o, idesc_mn(16), j ? 1u : first);
+					tc::umma_ss(tmem + kDwT0, a1 + o, b1 + o, tc::idesc(128, 64, true, 1, 1), j ? 1u : first);
+					tc::umma_ss(tmem + kDwT1, a2 + o, b2 + o, tc::idesc(128, 80, true, 1, 1), j ? 1u : first);
+					tc::umma_ss(tmem + kDwT2, a3 + o, b3 + o, tc::idesc(128, 16, true, 1, 1), j ? 1u : first);
 				}
 				tc::umma_commit(dw_done);
 			}

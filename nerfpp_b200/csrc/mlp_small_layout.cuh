@@ -47,31 +47,6 @@ __device__ __forceinline__ float wp(const float* __restrict__ p, int V, int laye
 	return i >= 0 ? p[i] : 0.f;
 }
 
-__device__ __forceinline__ uint32_t pack_bf16(float lo, float hi)
-{
-	__nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
-	return *reinterpret_cast<uint32_t*>(&v);
-}
-__device__ __forceinline__ uint32_t pack_f16(float lo, float hi)
-{
-	__half2 v = __floats2half2_rn(lo, hi);
-	return *reinterpret_cast<uint32_t*>(&v);
-}
-__device__ __forceinline__ uint32_t pack_bf16_relu(float lo, float hi)
-{
-	uint32_t r;
-	asm("cvt.rn.relu.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
-	return r;
-}
-
-
-__device__ __forceinline__ uint32_t pack_f16_relu(float lo, float hi)
-{
-	uint32_t r;
-	asm("cvt.rn.relu.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
-	return r;
-}
-
 // UMMA operand region (fp16), offsets in 32-bit words; padded N: layer 1 -> 16, layer 4 -> 16 (rows 3..15 zero)
 constexpr int kUmmaBase = kBlobWords;
 constexpr int kU0 = kUmmaBase, kU1 = kU0 + 64 * 32 / 2, kU2 = kU1 + 16 * 64 / 2, kU3 = kU2 + 64 * 32 / 2, kU4 = kU3 + 64 * 64 / 2;

@@ -59,7 +59,7 @@ template <int L>
 __device__ __forceinline__ void issue_layer(uint64_t* a_ready, uint64_t* d_ready, uint32_t& pa, uint32_t col, uint32_t w_saddr)
 {
 	using LY = Layer<L>;
-	constexpr uint32_t idesc = idesc_f16(128, LY::N);
+	constexpr uint32_t id = idesc(128, LY::N, false, 0, 0);
 	constexpr uint32_t lbo = LY::N * 16;   // bytes between the two 8-wide K chunks of one instruction
 	mbar_wait(a_ready, pa);
 	pa ^= 1u;
@@ -67,7 +67,7 @@ __device__ __forceinline__ void issue_layer(uint64_t* a_ready, uint64_t* d_ready
 #pragma unroll
 	for (int j = 0; j < LY::KS; j++) {
 		const uint64_t bd = smem_desc(w_saddr + LY::off * 4 + j * 2 * lbo, lbo, 128);
-		umma_ts(col + LY::d_col, col + kColA + j * 8, bd, idesc, j > 0);
+		umma_ts(col + LY::d_col, col + kColA + j * 8, bd, id, j > 0);
 	}
 	umma_commit(d_ready);
 }
@@ -151,15 +151,6 @@ __device__ __forceinline__ void add_ray_bias(uint32_t (&acc)[32], const float* _
 	}
 }
 
-// publish the A operand this warp just wrote to TMEM: one mbarrier arrival per warp
-__device__ __forceinline__ void publish_a(uint64_t* a_ready, int lane)
-{
-	tmem_st_wait();
-	fence_before();
-	__syncwarp();
-	if (lane == 0) mbar_arrive(a_ready);
-}
-
 template <int IN_KIND, bool MAPPED>
 __global__ void __launch_bounds__(kThreads, 1) mlp_small_fwd_tc_kernel(const uint32_t* __restrict__ blob, const void* __restrict__ enc,
 	const float* __restrict__ ray_sh, int S, const uint8_t* __restrict__ keep, int64_t n, RowMap map, float* __restrict__ raw_out)
@@ -214,7 +205,7 @@ __global__ void __launch_bounds__(kThreads, 1) mlp_small_fwd_tc_kernel(const uin
 		const bool ok = w < n;
 		// ---- layer 0 operand
 		tmem_st16(t_lane + kColA, in.e);
-		publish_a(a_ready, lane);
+		publish(a_ready, lane);
 		if (issuer) issue_layer<0>(a_ready, d_ready, pa, col, w_saddr);
 
 		uint32_t acc0[32], acc1[32], a16[16];
@@ -228,7 +219,7 @@ __global__ void __launch_bounds__(kThreads, 1) mlp_small_fwd_tc_kernel(const uin
 		tmem_st16(t_lane + kColA, a16);
 		relu_pack(acc1, a16);
 		tmem_st16(t_lane + kColA + 16, a16);
-		publish_a(a_ready, lane);
+		publish(a_ready, lane);
 		if (issuer) issue_layer<1>(a_ready, d_ready, pa, col, w_saddr);
 		// this row's view channels (per-ray SH table: cache hits) arrive while layer 1 runs
 		load_view_row<IN_KIND>(in, enc, ray_sh, S, keep, w, r, ok);
@@ -244,7 +235,7 @@ __global__ void __launch_bounds__(kThreads, 1) mlp_small_fwd_tc_kernel(const uin
 #pragma unroll
 		for (int i = 0; i < 8; i++) { a16[i] = in.v[i]; a16[8 + i] = pack_f16(__uint_as_float(d1[2 * i]), __uint_as_float(d1[2 * i + 1])); }
 		tmem_st16(t_lane + kColA, a16);
-		publish_a(a_ready, lane);
+		publish(a_ready, lane);
 		const bool kept = in.kept;
 		if (issuer) issue_layer<2>(a_ready, d_ready, pa, col, w_saddr);
 
@@ -265,7 +256,7 @@ __global__ void __launch_bounds__(kThreads, 1) mlp_small_fwd_tc_kernel(const uin
 			tmem_st16(t_lane + kColA, a16);
 			relu_pack(acc1, a16);
 			tmem_st16(t_lane + kColA + 16, a16);
-			publish_a(a_ready, lane);
+			publish(a_ready, lane);
 			if (issuer) {
 				if (l == 2) issue_layer<3>(a_ready, d_ready, pa, col, w_saddr);
 				else issue_layer<4>(a_ready, d_ready, pa, col, w_saddr);

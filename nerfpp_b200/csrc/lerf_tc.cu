@@ -278,8 +278,12 @@ __device__ __forceinline__ void epilogue_sync()
 	asm volatile("bar.sync 1, %0;" ::"n"(128 * HV) : "memory");
 }
 
-template <int MODE, int HV>
-__global__ void __launch_bounds__(32 * (2 + 4 * HV), 1) lerf_fwd_tc_kernel(const uint8_t* __restrict__ blob, const uint4* __restrict__ enc,
+// epilogue warps per TMEM lane quarter: two for RAW (its 403 MB of 4-byte stores are instruction-bound: 331 -> 251 us), one otherwise
+// (the TMEM read bandwidth, not the per-thread work, bounds those epilogues: 98.4 us with four warps, 102.0 us with eight)
+__host__ __device__ constexpr int epi_warps_per_quarter(int mode) { return mode == kRaw ? 2 : 1; }
+
+template <int MODE>
+__global__ void __launch_bounds__(32 * (2 + 4 * epi_warps_per_quarter(MODE)), 1) lerf_fwd_tc_kernel(const uint8_t* __restrict__ blob, const uint4* __restrict__ enc,
 	const uint8_t* __restrict__ keep, int64_t n, float* __restrict__ raw4, uint8_t* __restrict__ hidden, float* __restrict__ q_out, float* __restrict__ raw_le)
 {
 	extern __shared__ __align__(128) uint8_t smem_raw[];
@@ -288,6 +292,7 @@ __global__ void __launch_bounds__(32 * (2 + 4 * HV), 1) lerf_fwd_tc_kernel(const
 	const int64_t n_tiles = (n + 127) / 128;
 	const int64_t my_tiles = blockIdx.x < n_tiles ? (n_tiles - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
 	const ModeTable& mt = c_modes[MODE];
+	constexpr int HV = epi_warps_per_quarter(MODE);
 	constexpr int CH = 8 / HV;               // 32-column accumulator chunks per epilogue warp
 	constexpr int PRE = 16 / HV;             // 16-byte pieces of the input row per epilogue thread
 	constexpr uint32_t colEnc = kColEnc, colGeo = kColGeo;
@@ -533,18 +538,10 @@ static int launch(const nrf_lerf_shape* shape, const void* packed, const void* e
 	const int64_t tiles = (n + 127) / 128;
 	const int smem = static_cast<int>(sizeof(Smem)) + 256;
 	const int blocks = static_cast<int>(std::min<int64_t>(tiles, kNumSMs));
-	// epilogue warps per TMEM lane quarter: two for RAW (its 403 MB of 4-byte stores are instruction-bound: 331 -> 251 us), one otherwise
-	// (the TMEM read bandwidth, not the per-thread work, bounds those epilogues: 98.4 us with four warps, 102.0 us with eight); NRF_LERF_EPI_WARPS=4|8 overrides
-	static const int hv = MODE == kTrain ? 1 : [] { const char* e = getenv("NRF_LERF_EPI_WARPS"); return e && e[0] == '4' ? 1 : (e && e[0] == '8' ? 2 : (MODE == kRaw ? 2 : 1)); }();
-	if (hv == 2) {
-		NRF_CUDA(cudaFuncSetAttribute(lerf_fwd_tc_kernel<MODE, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-		lerf_fwd_tc_kernel<MODE, 2><<<blocks, 32 * 10, smem, as_stream(stream)>>>(reinterpret_cast<const uint8_t*>(packed), reinterpret_cast<const uint4*>(enc), keep, n,
-			raw4, reinterpret_cast<uint8_t*>(hidden), q, raw_le);
-	} else {
-		NRF_CUDA(cudaFuncSetAttribute(lerf_fwd_tc_kernel<MODE, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-		lerf_fwd_tc_kernel<MODE, 1><<<blocks, 32 * 6, smem, as_stream(stream)>>>(reinterpret_cast<const uint8_t*>(packed), reinterpret_cast<const uint4*>(enc), keep, n,
-			raw4, reinterpret_cast<uint8_t*>(hidden), q, raw_le);
-	}
+	constexpr int threads = 32 * (2 + 4 * epi_warps_per_quarter(MODE));
+	NRF_CUDA(cudaFuncSetAttribute(lerf_fwd_tc_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+	lerf_fwd_tc_kernel<MODE><<<blocks, threads, smem, as_stream(stream)>>>(reinterpret_cast<const uint8_t*>(packed), reinterpret_cast<const uint4*>(enc), keep, n,
+		raw4, reinterpret_cast<uint8_t*>(hidden), q, raw_le);
 	NRF_CHECK_LAUNCH("lerf_fwd_tc_kernel");
 	return NRF_OK;
 }

@@ -450,11 +450,7 @@ __global__ void __launch_bounds__(kBwdThreads, 1) mlp_nerf_bwd_dw_kernel(const _
 			for (int a = 0; a < 8; a++)
 #pragma unroll
 				for (int e = 0; e < 8; e++) bs[a][e] = 0.f;
-#ifdef NRF_DW_NOSUM
-			const bool sum_a = false, sum_b = false;
-#else
 			const bool sum_a = U.bias_mode == 1, sum_b = U.bias_mode == 2 && q == 0;
-#endif
 			const int per_warp = U.a_cols / 32;          // column chunks of the A slab per warp: 8 (256 columns) or 4
 			for (int64_t i = lo; i < hi; i++, g++) {
 				const uint32_t slot = g % kDwRing, round = g / kDwRing;

@@ -152,9 +152,6 @@ __host__ __device__ constexpr int group_count(int g) { return g == 8 ? 2 : 1; }
 
 // TRAIN: bf16 operands (the exponent range survives Xavier(0.1) initialisation, src/LibTorchTraining/Trainable.h:43, where fp16
 // activations of the deep layers flush to zero) and every layer's input is stored to the scratch records of mlp_nerf_layout.cuh
-// CL = 2: the CTAs of a 2-CTA cluster walk their tiles in lockstep and share ONE weight stream: each loads half of every stage and
-// multicasts it into both shared memories, so a stage costs one L2 read per cluster instead of one per SM.  (All 148 SMs pulling
-// the whole 1.2 MB blob per tile is 5.7 TB/s of L2 -> SM traffic — the measured pace of the CL = 1 kernel, not its tensor pipe.)
 // RAW: x is the sample positions [N,3] and the positional embedding (EmbedderImpl::forward, src/NeRF.cpp:22-39: [x, sin(f0 x), cos(f0 x), ..],
 // same fp32 product and libdevice sinf / cosf as nrf_posenc_fwd, hence bit-identical operands) is evaluated by the thread that owns the row,
 // directions are read per RAY (row / samples_per_ray; the reference expands them per sample, src/NeRFRenderer.h:179-181): the [N,63] / [N,27]
@@ -190,22 +187,20 @@ __device__ __forceinline__ void posenc_stage(const float (&p)[3], const float* _
 	}
 }
 
-template <bool TRAIN, int CL, bool RAW>
-__global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(kThreads, 1) mlp_nerf_fwd_tc_kernel(const uint8_t* __restrict__ blob,
+template <bool TRAIN, bool RAW>
+__global__ void __launch_bounds__(kThreads, 1) mlp_nerf_fwd_tc_kernel(const uint8_t* __restrict__ blob,
 	const float* __restrict__ x, int64_t n, float* __restrict__ out, uint8_t* __restrict__ saved, const RawInput raw)
 {
 	extern __shared__ __align__(128) uint8_t smem_raw[];
 	Smem& sm = *reinterpret_cast<Smem*>(smem_raw);
 	const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 	const int64_t n_tiles = (n + 127) / 128;
-	// every CTA runs the same number of rounds (the cluster shares the weight stream); a round past the last tile is a tile of no rows
+	// every CTA runs the same number of rounds; a round past the last tile is a tile of no rows
 	const int64_t my_tiles = (n_tiles + gridDim.x - 1) / gridDim.x;
-	const uint32_t cta_rank = CL > 1 ? cluster_ctarank() : 0u;
-	constexpr uint16_t kAll = static_cast<uint16_t>((1u << CL) - 1u);
 
 	if (warp == 1) {
 		if (lane == 0) {
-			for (int s = 0; s < kRing; s++) { mbar_init(&sm.full[s], 1); mbar_init(&sm.empty[s], CL); }
+			for (int s = 0; s < kRing; s++) { mbar_init(&sm.full[s], 1); mbar_init(&sm.empty[s], 1); }
 			mbar_init(&sm.a_ready, 4);
 			mbar_init(&sm.d_ready, 1);
 			asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -216,7 +211,6 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(kThreads, 1) mlp_ne
 	for (int i = threadIdx.x; i < kBiasFloats; i += kThreads) sm.bias[i] = reinterpret_cast<const float*>(blob + kWeightBytes)[i];
 	fence_before();
 	__syncthreads();
-	if (CL > 1) cluster_sync();          // the peers' barriers exist before anything is multicast to them
 	fence_after();
 	const uint32_t tmem = sm.tmem_base;
 
@@ -232,12 +226,7 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(kThreads, 1) mlp_ne
 					const uint32_t bytes = c_fwd_table.bytes[i];
 					const int off = c_fwd_table.off[i];
 					mbar_expect_tx(&sm.full[slot], bytes);
-					if (CL > 1) {
-						const uint32_t part = bytes / CL;       // this CTA's share, delivered to every CTA of the cluster
-						tma_bulk_g2s_mc(sm.ring[slot] + cta_rank * part, blob + off + cta_rank * part, part, &sm.full[slot], kAll);
-					} else {
-						tma_bulk_g2s(sm.ring[slot], blob + off, bytes, &sm.full[slot]);
-					}
+					tma_bulk_g2s(sm.ring[slot], blob + off, bytes, &sm.full[slot]);
 				}
 			}
 		}
@@ -268,8 +257,7 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(kThreads, 1) mlp_ne
 								first = false;
 								a_col += 8;
 							}
-							if (CL > 1) umma_commit_mc(&sm.empty[slot], kAll);   // free in a peer's ring only when every CTA has read it
-							else umma_commit(&sm.empty[slot]);                  // the stage is free again once these MMAs have read it
+							umma_commit(&sm.empty[slot]);   // the stage is free again once these MMAs have read it
 						}
 					}
 					umma_commit(&sm.d_ready);
@@ -387,7 +375,6 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(kThreads, 1) mlp_ne
 
 	fence_before();
 	__syncthreads();
-	if (CL > 1) cluster_sync();          // no CTA leaves while a peer can still multicast into its shared memory
 	if (warp == 1) {
 		fence_after();
 		tmem_free_all(tmem);
@@ -422,22 +409,14 @@ static int fwd_common(const nrf_mlp_nerf_shape* shape, const void* packed, const
 		(reinterpret_cast<uintptr_t>(saved) & 127) == 0, "packed / saved must be 128-byte, x 8-byte, out 16-byte aligned");
 	const int64_t tiles = (n + 127) / 128;
 	const int smem = static_cast<int>(sizeof(Smem)) + 128;
-	// NRF_NERF_CLUSTER=2 selects 2-CTA clusters that share one multicast weight stream.  Measured equal to the default (0.332 vs 0.330 ms
-	// at 196 608 rows): halving the L2 -> SM weight traffic changes nothing, i.e. the weight stream does not pace this kernel.  What does:
-	// one tile in flight, so a layer is its MMAs (16 x 128 cycles) THEN its epilogue, and the epilogue reads 128 KB of fp32 accumulators
-	// out of TMEM at 64 B/clk (2 048 cycles) — splitting it over 8 warps instead of 4 gained 5 % (inference) / lost 7 % (training).
-	static const int cluster = [] { const char* e = getenv("NRF_NERF_CLUSTER"); return e && e[0] == '2' ? 2 : 1; }();
-	if (cluster == 2) {
-		const int blocks = static_cast<int>(std::min<int64_t>((tiles + 1) / 2 * 2, kNumSMs));
-		NRF_CUDA(cudaFuncSetAttribute(mlp_nerf_fwd_tc_kernel<TRAIN, 2, RAW>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-		mlp_nerf_fwd_tc_kernel<TRAIN, 2, RAW><<<blocks, kThreads, smem, as_stream(stream)>>>(reinterpret_cast<const uint8_t*>(packed), x, n, out,
-			reinterpret_cast<uint8_t*>(saved), raw);
-	} else {
-		const int blocks = static_cast<int>(std::min<int64_t>(tiles, kNumSMs));
-		NRF_CUDA(cudaFuncSetAttribute(mlp_nerf_fwd_tc_kernel<TRAIN, 1, RAW>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-		mlp_nerf_fwd_tc_kernel<TRAIN, 1, RAW><<<blocks, kThreads, smem, as_stream(stream)>>>(reinterpret_cast<const uint8_t*>(packed), x, n, out,
-			reinterpret_cast<uint8_t*>(saved), raw);
-	}
+	// Every CTA streams the whole weight blob for each of its tiles.  That L2 -> SM weight traffic does not pace this kernel: 2-CTA clusters
+	// that shared one multicast weight stream halved it and measured equal (0.332 vs 0.330 ms at 196 608 rows).  What does: one tile in
+	// flight, so a layer is its MMAs (16 x 128 cycles) THEN its epilogue, and the epilogue reads 128 KB of fp32 accumulators out of TMEM
+	// at 64 B/clk (2 048 cycles) — splitting it over 8 warps instead of 4 gained 5 % (inference) / lost 7 % (training).
+	const int blocks = static_cast<int>(std::min<int64_t>(tiles, kNumSMs));
+	NRF_CUDA(cudaFuncSetAttribute(mlp_nerf_fwd_tc_kernel<TRAIN, RAW>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+	mlp_nerf_fwd_tc_kernel<TRAIN, RAW><<<blocks, kThreads, smem, as_stream(stream)>>>(reinterpret_cast<const uint8_t*>(packed), x, n, out,
+		reinterpret_cast<uint8_t*>(saved), raw);
 	NRF_CHECK_LAUNCH("mlp_nerf_fwd_tc_kernel");
 	return NRF_OK;
 }
@@ -487,7 +466,7 @@ int nrf_mlp_nerf_pack_train(const nrf_mlp_nerf_shape* shape, const nrf_mlp_nerf_
 int64_t nrf_mlp_nerf_saved_bytes(const nrf_mlp_nerf_shape* shape, int64_t n)
 {
 	if (nerf_tc::check_shape(shape) || n < 0) return -1;
-	return ((n + 127) / 128 + 1) * static_cast<int64_t>(kSaveTile);      // + one spare record (idle rounds of a cluster write there)
+	return ((n + 127) / 128 + 1) * static_cast<int64_t>(kSaveTile);      // + one spare record (a CTA's rounds past the last tile write there)
 }
 
 int nrf_mlp_nerf_fwd(const nrf_mlp_nerf_shape* shape, const void* packed, const float* x, int64_t n, float* out, nrf_stream stream)

@@ -77,7 +77,8 @@ __global__ void adam_schedule_kernel(AdamSchedState* st, double lr0, double deca
 // L2 residency hints.  The step streams 303 MB through the 126 MB L2 here; without hints the two arrays the NEXT step reads at random —
 // the fp16 shadow (17.8 MB: hash encode gathers) and the zeroed gradient (35.6 MB: hash backward REDs) — are evicted by the fp32
 // master / moment streams and the next coarse-pass encode starts cold.  Masters and moments are marked evict_first, shadow and gradient
-// zeros evict_last.
+// zeros evict_last.  A/B against plain loads and stores on the same B200, 100 graph-replayed steps each: adam_step 51.3 -> 46.4 us,
+// step 0.8683 -> 0.8613 ms (profiles/r1_adam_l2hint_ab.json).
 __device__ __forceinline__ uint64_t l2_policy_evict_first()
 {
 	uint64_t p;
@@ -105,7 +106,6 @@ __device__ __forceinline__ void st_hint2(void* p, uint32_t a, uint32_t b, uint64
 	asm volatile("st.global.L2::cache_hint.v2.b32 [%0], {%1, %2}, %3;" ::"l"(p), "r"(a), "r"(b), "l"(pol) : "memory");
 }
 
-template <bool HINT>
 __global__ void __launch_bounds__(256) adam_kernel(float* __restrict__ param, float* __restrict__ grad, float* __restrict__ m,
 	float* __restrict__ v, int64_t n, AdamArgs a, int zero_grad, __half* __restrict__ shadow, const AdamSchedState* __restrict__ sched)
 {
@@ -115,13 +115,10 @@ __global__ void __launch_bounds__(256) adam_kernel(float* __restrict__ param, fl
 		a.inv_sqrt_bc2 = sched->inv_sqrt_bc2;
 	}
 	const int64_t stride = static_cast<int64_t>(gridDim.x) * blockDim.x * 4;
-	uint64_t pol_first = 0, pol_last = 0;
-	if (HINT) { pol_first = l2_policy_evict_first(); pol_last = l2_policy_evict_last(); }
+	const uint64_t pol_first = l2_policy_evict_first(), pol_last = l2_policy_evict_last();
 	for (int64_t i = (static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x) * 4; i < n; i += stride) {
 		if (i + 3 < n) {
-			float4 p4, m4, v4;
-			if (HINT) { p4 = ld_hint(param + i, pol_first); m4 = ld_hint(m + i, pol_first); v4 = ld_hint(v + i, pol_first); }
-			else { p4 = *reinterpret_cast<float4*>(param + i); m4 = *reinterpret_cast<float4*>(m + i); v4 = *reinterpret_cast<float4*>(v + i); }
+			float4 p4 = ld_hint(param + i, pol_first), m4 = ld_hint(m + i, pol_first), v4 = ld_hint(v + i, pol_first);
 			float4 g4 = *reinterpret_cast<float4*>(grad + i);
 			p4.x = adam_one(p4.x, g4.x * a.grad_scale, m4.x, v4.x, a);
 			p4.y = adam_one(p4.y, g4.y * a.grad_scale, m4.y, v4.y, a);
@@ -129,19 +126,11 @@ __global__ void __launch_bounds__(256) adam_kernel(float* __restrict__ param, fl
 			p4.w = adam_one(p4.w, g4.w * a.grad_scale, m4.w, v4.w, a);
 			const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
 			__half2 lo = __floats2half2_rn(p4.x, p4.y), hi = __floats2half2_rn(p4.z, p4.w);
-			if (HINT) {
-				st_hint(param + i, p4, pol_first);
-				st_hint(m + i, m4, pol_first);
-				st_hint(v + i, v4, pol_first);
-				if (zero_grad) st_hint(grad + i, zero, pol_last);
-				if (shadow) st_hint2(shadow + i, *reinterpret_cast<uint32_t*>(&lo), *reinterpret_cast<uint32_t*>(&hi), pol_last);
-			} else {
-				*reinterpret_cast<float4*>(param + i) = p4;
-				*reinterpret_cast<float4*>(m + i) = m4;
-				*reinterpret_cast<float4*>(v + i) = v4;
-				if (zero_grad) *reinterpret_cast<float4*>(grad + i) = zero;
-				if (shadow) *reinterpret_cast<uint2*>(shadow + i) = make_uint2(*reinterpret_cast<uint32_t*>(&lo), *reinterpret_cast<uint32_t*>(&hi));
-			}
+			st_hint(param + i, p4, pol_first);
+			st_hint(m + i, m4, pol_first);
+			st_hint(v + i, v4, pol_first);
+			if (zero_grad) st_hint(grad + i, zero, pol_last);
+			if (shadow) st_hint2(shadow + i, *reinterpret_cast<uint32_t*>(&lo), *reinterpret_cast<uint32_t*>(&hi), pol_last);
 		} else {
 			for (int64_t j = i; j < n; j++) {
 				float mm = m[j], vv = v[j];
@@ -152,14 +141,6 @@ __global__ void __launch_bounds__(256) adam_kernel(float* __restrict__ param, fl
 			}
 		}
 	}
-}
-
-// L2 eviction-priority variant, on by default; NRF_ADAM_L2HINT=0 selects the plain kernel (A/B on the same B200, 100 graph-replayed
-// steps each: adam_step 51.3 -> 46.4 us, step 0.8683 -> 0.8613 ms, gpurun_out/lerf1 -> profiles/r1_adam_l2hint_ab.json)
-static bool adam_l2_hint()
-{
-	static const bool on = [] { const char* e = getenv("NRF_ADAM_L2HINT"); return !(e && e[0] == '0'); }();
-	return on;
 }
 
 }  // namespace nrf
@@ -197,8 +178,7 @@ int nrf_adam_step(float* param, float* grad, float* exp_avg, float* exp_avg_sq, 
 	a.beta1 = beta1; a.beta2 = beta2; a.eps = eps; a.grad_scale = grad_scale;
 	const int64_t quads = (n + 3) / 4;
 	const int blocks = static_cast<int>(std::min<int64_t>((quads + 255) / 256, kNumSMs * 8));
-	if (adam_l2_hint()) adam_kernel<true><<<blocks, 256, 0, as_stream(stream)>>>(param, grad, exp_avg, exp_avg_sq, n, a, zero_grad, reinterpret_cast<__half*>(shadow_f16), nullptr);
-	else adam_kernel<false><<<blocks, 256, 0, as_stream(stream)>>>(param, grad, exp_avg, exp_avg_sq, n, a, zero_grad, reinterpret_cast<__half*>(shadow_f16), nullptr);
+	adam_kernel<<<blocks, 256, 0, as_stream(stream)>>>(param, grad, exp_avg, exp_avg_sq, n, a, zero_grad, reinterpret_cast<__half*>(shadow_f16), nullptr);
 	NRF_CHECK_LAUNCH("adam_kernel");
 	return NRF_OK;
 }
@@ -227,9 +207,7 @@ int nrf_adam_step_scheduled(float* param, float* grad, float* exp_avg, float* ex
 	a.beta1 = beta1; a.beta2 = beta2; a.eps = eps; a.grad_scale = grad_scale;
 	const int64_t quads = (n + 3) / 4;
 	const int blocks = static_cast<int>(std::min<int64_t>((quads + 255) / 256, kNumSMs * 8));
-	if (adam_l2_hint()) launch_kernel(adam_kernel<true>, blocks, 256, 0, as_stream(stream), param, grad, exp_avg, exp_avg_sq, n, a, zero_grad,
-		reinterpret_cast<__half*>(shadow_f16), reinterpret_cast<const AdamSchedState*>(sched_state));
-	else launch_kernel(adam_kernel<false>, blocks, 256, 0, as_stream(stream), param, grad, exp_avg, exp_avg_sq, n, a, zero_grad,
+	launch_kernel(adam_kernel, blocks, 256, 0, as_stream(stream), param, grad, exp_avg, exp_avg_sq, n, a, zero_grad,
 		reinterpret_cast<__half*>(shadow_f16), reinterpret_cast<const AdamSchedState*>(sched_state));
 	NRF_CHECK_LAUNCH("adam_kernel");
 	return NRF_OK;

@@ -40,23 +40,6 @@ __device__ __forceinline__ void tma_bulk_g2s(void* dst, const void* src, uint32_
 	asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
 	             ::"r"(smem_u32(dst)), "l"(src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
 }
-// The same copy delivered to the SAME shared-memory offset of every CTA of the cluster named in cta_mask (one L2 read), each
-// destination CTA's mbarrier (same offset) receiving the complete_tx
-__device__ __forceinline__ void tma_bulk_g2s_mc(void* dst, const void* src, uint32_t bytes, uint64_t* bar, uint16_t cta_mask)
-{
-	asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1], %2, [%3], %4;"
-	             ::"r"(smem_u32(dst)), "l"(src), "r"(bytes), "r"(smem_u32(bar)), "h"(cta_mask) : "memory");
-}
-__device__ __forceinline__ uint32_t cluster_ctarank()
-{
-	uint32_t r;
-	asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-	return r;
-}
-__device__ __forceinline__ void cluster_sync()
-{
-	asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
 // asynchronous L2 prefetch of a contiguous global range (bytes: multiple of 16)
 __device__ __forceinline__ void tma_prefetch_l2(const void* src, uint32_t bytes)
 {
@@ -96,13 +79,6 @@ __device__ __forceinline__ void umma_ss(uint32_t d_tmem, uint64_t a_desc, uint64
 __device__ __forceinline__ void umma_commit(uint64_t* bar)
 {
 	asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-
-// the same arrival on the mbarrier at this offset in every CTA of cta_mask
-__device__ __forceinline__ void umma_commit_mc(uint64_t* bar, uint16_t cta_mask)
-{
-	asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-	             ::"r"(smem_u32(bar)), "h"(cta_mask) : "memory");
 }
 // KSTEPS K = 16 steps of one accumulator block with the A operand in TMEM and an MN-major B operand: A advances 8 TMEM columns, the B
 // descriptor 256 bytes (16 rows of K) per step; the first step accumulates onto D iff acc_first

@@ -1,8 +1,5 @@
 """The A/B variants that ship in libnerfpp_b200.so behind environment switches (read once per process) stay correct: each is run in a fresh
 process through the parity tests of the default path.
-  NRF_NERF_CLUSTER=2    classic-NeRF forward with 2-CTA clusters sharing one multicast weight stream (csrc/mlp_nerf_tc.cu)
-  NRF_LERF_EPI_WARPS=8  eight epilogue warps in the LeRF SIGMA / HIDDEN programs (csrc/lerf_tc.cu)
-  NRF_ADAM_L2HINT=0     Adam without the L2 eviction-priority hints (csrc/optim.cu)
   NRF_RENDER_REUSE=0    nrf_render_rays_fwd evaluating every merged row of the fine pass instead of the importance samples only (csrc/render.cu):
                         the test compares it with the composed path, which reuses — bit for bit
   NRF_HASH_SPLIT=0      hash forward with one thread per point instead of four lanes per point (csrc/hash_encode.cu)
@@ -18,9 +15,6 @@ pytestmark = pytest.mark.gpu
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 VARIANTS = [
-    ({"NRF_NERF_CLUSTER": "2"}, ["test_gpu_mlp_nerf.py"], "forward_matches_oracle or repeatable"),
-    ({"NRF_LERF_EPI_WARPS": "8"}, ["test_gpu_lerf.py"], "fixture or oracle"),
-    ({"NRF_ADAM_L2HINT": "0"}, ["test_gpu_render.py"], "adam"),
     ({"NRF_RENDER_REUSE": "0"}, ["test_gpu_pipeline.py"], "fused_render_entry"),
     ({"NRF_HASH_SPLIT": "0"}, ["test_gpu_hash.py"], "fixture or reuse or rays"),
     ({"NRF_PDL": "1"}, ["test_gpu_pipeline.py"], "graph or gradients or trains or reuse or render"),

@@ -5,7 +5,6 @@
 #include <cuda_bf16.h>
 #include <stdint.h>
 #include <stdio.h>
-#include <utility>
 #include "../../include/nerfpp_b200.h"
 
 namespace nrf {
@@ -44,36 +43,6 @@ inline cudaStream_t as_stream(nrf_stream s) { return reinterpret_cast<cudaStream
 	} while (0)
 
 constexpr int kNumSMs = 148;  // B200
-
-// Programmatic dependent launch along the step's kernel chain (opt-in: NRF_PDL=1; default plain stream order).  A kernel
-// launched through launch_kernel may become resident while its predecessor in the stream drains — its CTAs fill SMs the predecessor's tail
-// leaves idle and the launch latency disappears behind it — and MUST start with pdl_prologue(): griddepcontrol.wait blocks until the
-// predecessor has completed and its writes are visible (so nothing of it is ever read early), then launch_dependents lets the successor do the
-// same behind this kernel.  Both instructions are no-ops in a kernel launched without the attribute.  Stream capture records the edges as
-// programmatic dependencies of the graph.
-bool pdl_enabled();
-
-__device__ __forceinline__ void pdl_prologue()
-{
-	asm volatile("griddepcontrol.wait;" ::: "memory");
-	asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-}
-
-template <typename... KArgs, typename... Args>
-inline void launch_kernel(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, Args&&... args)
-{
-	cudaLaunchConfig_t cfg = {};
-	cfg.gridDim = grid;
-	cfg.blockDim = block;
-	cfg.dynamicSmemBytes = smem;
-	cfg.stream = s;
-	cudaLaunchAttribute attr[1];
-	attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-	attr[0].val.programmaticStreamSerializationAllowed = 1;
-	cfg.attrs = attr;
-	cfg.numAttrs = pdl_enabled() ? 1 : 0;
-	cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);     // errors surface in NRF_CHECK_LAUNCH (cudaGetLastError)
-}
 
 __device__ __forceinline__ float warp_sum(float v)
 {

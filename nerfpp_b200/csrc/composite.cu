@@ -85,7 +85,6 @@ __global__ void __launch_bounds__(kRaysPerCta * 32) composite_fwd_kernel(const f
 	int64_t R, int S, float* __restrict__ rgb, float* __restrict__ depth, float* __restrict__ disp, float* __restrict__ acc,
 	float* __restrict__ weights)
 {
-	pdl_prologue();
 	const int lane = threadIdx.x & 31;
 	const int64_t ray = static_cast<int64_t>(blockIdx.x) * kRaysPerCta + (threadIdx.x >> 5);
 	if (ray >= R) return;
@@ -137,7 +136,6 @@ __global__ void __launch_bounds__(kRaysPerCta * 32) composite_fwd_nb_kernel(cons
 	int64_t R, int S, float* __restrict__ rgb, float* __restrict__ depth, float* __restrict__ disp, float* __restrict__ acc,
 	float* __restrict__ weights)
 {
-	pdl_prologue();
 	const int lane = threadIdx.x & 31;
 	const int64_t ray = static_cast<int64_t>(blockIdx.x) * kRaysPerCta + (threadIdx.x >> 5);
 	if (ray >= R) return;
@@ -206,7 +204,6 @@ __global__ void __launch_bounds__(kRaysPerCta * 32) composite_bwd_kernel(const f
 	int64_t R, int S, const float* __restrict__ g_rgb, const float* __restrict__ g_depth, const float* __restrict__ g_disp,
 	const float* __restrict__ g_acc, const float* __restrict__ g_weights, float* __restrict__ d_raw, HuberArgs hub)
 {
-	pdl_prologue();
 	const int lane = threadIdx.x & 31;
 	const int64_t ray = static_cast<int64_t>(blockIdx.x) * kRaysPerCta + (threadIdx.x >> 5);
 	if (ray >= R) return;
@@ -445,7 +442,7 @@ int nrf_composite_fwd(const float* raw, int32_t raw_stride, const float* z, cons
 	const int nb = (n_samples + 31) / 32;
 #define NRF_CF(NBV)                                                                                                     \
 	case NBV:                                                                                                           \
-		launch_kernel(composite_fwd_nb_kernel<NBV>, blocks, kRaysPerCta * 32, 0, s, raw, raw_stride, z, rays_d, noise, raw_noise_std, \
+		composite_fwd_nb_kernel<NBV><<<blocks, kRaysPerCta * 32, 0, s>>>(raw, raw_stride, z, rays_d, noise, raw_noise_std, \
 			white_bkgr, n_rays, n_samples, rgb, depth, disp, acc, weights);                                              \
 		break
 	switch (nb) {
@@ -474,7 +471,7 @@ int nrf_composite_bwd(const float* raw, int32_t raw_stride, const float* z, cons
 	const HuberArgs none{};
 #define NRF_CB(NBV)                                                                                                  \
 	case NBV:                                                                                                        \
-		launch_kernel(composite_bwd_kernel<NBV, false>, blocks, kRaysPerCta * 32, 0, s, raw, raw_stride, z, rays_d, noise, raw_noise_std, \
+		composite_bwd_kernel<NBV, false><<<blocks, kRaysPerCta * 32, 0, s>>>(raw, raw_stride, z, rays_d, noise, raw_noise_std, \
 			white_bkgr, n_rays, n_samples, g_rgb, g_depth, g_disp, g_acc, g_weights, d_raw, none);                    \
 		break
 	switch (nb) {
@@ -505,7 +502,7 @@ int nrf_composite_huber_bwd(const float* raw, int32_t raw_stride, const float* z
 	hub.loss_out = loss_out; hub.rgb_out = rgb_out;
 #define NRF_CH(NBV)                                                                                                  \
 	case NBV:                                                                                                        \
-		launch_kernel(composite_bwd_kernel<NBV, true>, blocks, kRaysPerCta * 32, 0, s, raw, raw_stride, z, rays_d, noise, raw_noise_std, \
+		composite_bwd_kernel<NBV, true><<<blocks, kRaysPerCta * 32, 0, s>>>(raw, raw_stride, z, rays_d, noise, raw_noise_std, \
 			white_bkgr, n_rays, n_samples, static_cast<const float*>(nullptr), static_cast<const float*>(nullptr), static_cast<const float*>(nullptr), \
 			static_cast<const float*>(nullptr), static_cast<const float*>(nullptr), d_raw, hub);                      \
 		break

@@ -18,7 +18,6 @@
 //   * the backward accumulates in fp32 with vector RED (red.global.add.v2.f32), no x128 loss scale.
 #include "common.cuh"
 #include "jitter.cuh"
-#include <stdlib.h>
 #include <string.h>
 
 namespace nrf {
@@ -262,7 +261,6 @@ __device__ __forceinline__ void hash_fwd_body(const HashArgs& a, const __half* _
 	constexpr int CH = 8 / F;
 	using V = typename FeatVec<F>::type;
 	__shared__ HashMeta m;
-	pdl_prologue();
 	stage_meta(m, a);
 	const int L = a.n_levels;
 	const int row_bytes = L * F * (OUT_F32 ? 4 : 2);
@@ -419,7 +417,6 @@ __device__ __forceinline__ void hash_bwd_body(HashArgs a, PS ps, int64_t n_point
 	constexpr int CH = 8 / F;   // levels per 8-value gradient chunk (16 B of bf16 / 32 B of fp32)
 	constexpr uint32_t FULL = 0xffffffffu;
 	__shared__ HashMeta m;
-	pdl_prologue();
 	stage_meta(m, a);
 
 	const int lane = threadIdx.x & 31;
@@ -627,18 +624,6 @@ static int fill_args(const nrf_hash_grid* g, HashArgs& a)
 // ceiling as the fine pass (1 sector / clk / SM), not a launch-shape effect.
 struct LaunchPlan { unsigned grid; int64_t stride; int iters; };
 
-// experiment hook (scripts/exp/hash_occupancy.py): NRF_HASH_OCC=k pads every CTA with dynamic shared memory so that only k CTAs of 128 threads are
-// resident per SM — how much of the machine the gather / scatter kernels need before the L1-miss path saturates (can a tensor-core kernel co-run?)
-static int occ_pad_bytes()
-{
-	static const int pad = [] {
-		const char* e = getenv("NRF_HASH_OCC");
-		const int k = e ? atoi(e) : 0;
-		return k > 0 ? (227 * 1024) / k - 2048 : 0;
-	}();
-	return pad;
-}
-
 static LaunchPlan launch_plan(int64_t items, int block)
 {
 	const int64_t ctas = (items + block - 1) / block;
@@ -699,31 +684,24 @@ static int launch_hash_fwd(const nrf_hash_grid* grid, const void* table_f16, con
 	const int F = grid->n_features;
 	const __half* t = reinterpret_cast<const __half*>(table_f16);
 	cudaStream_t s = as_stream(stream);
-	// lanes per point: one per 16-byte chunk of the row when the chunks of a row are a power of two (4 at L16 F2, 16 at L16 F8)
-	static const int split_env = [] { const char* e = getenv("NRF_HASH_SPLIT"); return e ? atoi(e) : -1; }();
+	// lanes per point: one per 16-byte chunk of the row at 16 levels (4 at F2, 8 at F4, 16 at F8); every other shape, for example L12 F2 or
+	// L8 F8, runs one thread per point
 	const int chunks = (grid->n_levels * F + 7) / 8;
-	const bool can_split = (grid->n_levels * F) % 8 == 0 && (chunks & (chunks - 1)) == 0 && chunks <= 32 && chunks > 1;
-	const bool split = can_split && split_env != 0;
+	const bool split = (grid->n_levels * F) % 8 == 0 && (chunks & (chunks - 1)) == 0 && chunks <= 32 && chunks > 1;
 #define NRF_LAUNCH_FWD2(FF, O32, SP)                                                                                              \
 	do {                                                                                                                          \
 		const int64_t items = (ps.group > 1 ? (static_cast<int64_t>(ps.R) + ps.group - 1) / ps.group * ps.group * ps.S_work : n_points) * (SP); \
 		const LaunchPlan lp = launch_plan(items, 128);                                                                           \
-		if (occ_pad_bytes() > 48 * 1024) cudaFuncSetAttribute(fwd_kernel<FF, O32, SP>(ps), cudaFuncAttributeMaxDynamicSharedMemorySize, occ_pad_bytes()); \
-		launch_kernel(fwd_kernel<FF, O32, SP>(ps), lp.grid, 128, occ_pad_bytes(), s, a, t, ps, ru, items, lp.stride, lp.iters, clamp_points, keep, enc_out); \
+		fwd_kernel<FF, O32, SP>(ps)<<<lp.grid, 128, 0, s>>>(a, t, ps, ru, items, lp.stride, lp.iters, clamp_points, keep, enc_out);       \
 	} while (0)
 #define NRF_LAUNCH_FWD(FF, SP)                                                     \
 	do {                                                                           \
-		if (split) {                                                               \
-			if (layout == NRF_ENC_F32) NRF_LAUNCH_FWD2(FF, true, SP);              \
-			else NRF_LAUNCH_FWD2(FF, false, SP);                                   \
-		} else {                                                                   \
-			if (layout == NRF_ENC_F32) NRF_LAUNCH_FWD2(FF, true, 1);               \
-			else NRF_LAUNCH_FWD2(FF, false, 1);                                    \
-		}                                                                          \
+		if (layout == NRF_ENC_F32) NRF_LAUNCH_FWD2(FF, true, SP);                  \
+		else NRF_LAUNCH_FWD2(FF, false, SP);                                       \
 	} while (0)
-	if (F == 2) { if (chunks == 4) NRF_LAUNCH_FWD(2, 4); else NRF_LAUNCH_FWD(2, 1); }
-	else if (F == 4) { if (chunks == 8) NRF_LAUNCH_FWD(4, 8); else NRF_LAUNCH_FWD(4, 1); }
-	else if (F == 8) { if (chunks == 16) NRF_LAUNCH_FWD(8, 16); else NRF_LAUNCH_FWD(8, 1); }
+	if (F == 2) { if (split && chunks == 4) NRF_LAUNCH_FWD(2, 4); else NRF_LAUNCH_FWD(2, 1); }
+	else if (F == 4) { if (split && chunks == 8) NRF_LAUNCH_FWD(4, 8); else NRF_LAUNCH_FWD(4, 1); }
+	else if (F == 8) { if (split && chunks == 16) NRF_LAUNCH_FWD(8, 16); else NRF_LAUNCH_FWD(8, 1); }
 	else { set_error("nrf_hash_encode_fwd: n_features must be 2, 4 or 8"); return NRF_ERR_UNSUPPORTED; }
 #undef NRF_LAUNCH_FWD
 #undef NRF_LAUNCH_FWD2
@@ -748,9 +726,8 @@ static int launch_hash_bwd(const nrf_hash_grid* grid, const PS& ps, int64_t n_po
 #define NRF_LAUNCH_BWD2(FF, BF)                                                                                                   \
 	do {                                                                                                                          \
 		const LaunchPlan lp = launch_plan(n_points, 128);                                                                        \
-		if (occ_pad_bytes() > 48 * 1024) cudaFuncSetAttribute(bwd_kernel<FF, BF>(ps), cudaFuncAttributeMaxDynamicSharedMemorySize, occ_pad_bytes()); \
-		launch_kernel(bwd_kernel<FF, BF>(ps), lp.grid, 128, occ_pad_bytes(), s, a, ps, n_points, lp.stride, lp.iters, clamp_points, grad_enc, grad_table, \
-			level_begin, level_end);                                                                                                  \
+		bwd_kernel<FF, BF>(ps)<<<lp.grid, 128, 0, s>>>(a, ps, n_points, lp.stride, lp.iters, clamp_points, grad_enc, grad_table, level_begin, \
+			level_end);                                                                                                               \
 	} while (0)
 #define NRF_LAUNCH_BWD(FF)                                             \
 	do {                                                               \

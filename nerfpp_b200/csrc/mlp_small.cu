@@ -30,7 +30,6 @@ namespace nrf {
 
 __global__ void __launch_bounds__(256) mlp_pack_kernel(const float* __restrict__ p, int V, uint32_t* __restrict__ blob)
 {
-	pdl_prologue();
 	const int w = blockIdx.x * blockDim.x + threadIdx.x;
 	if (w >= kPackedWords) return;
 	if (w >= kViewBase) {
@@ -321,7 +320,6 @@ __global__ void __launch_bounds__(kBwdWarps * 32, 1) mlp_small_bwd_kernel(const 
 	void* __restrict__ grad_in, float* __restrict__ grad_params, int V, float* __restrict__ grad_bias)
 {
 	extern __shared__ __align__(16) uint8_t smem_raw[];
-	pdl_prologue();
 	uint32_t* wf = reinterpret_cast<uint32_t*>(smem_raw);
 	uint8_t* ctiles = smem_raw + static_cast<size_t>(kBlobWords) * 4;                       // the operand regions
 	uint64_t* dw_done = reinterpret_cast<uint64_t*>(ctiles + kRegionBytes);                 // the tile's MMAs have read the regions
@@ -542,7 +540,6 @@ __global__ void __launch_bounds__(kViewBiasThreads) view_bias_fwd_kernel(const u
 	float* __restrict__ bias, float* __restrict__ grad_bias_zero)
 {
 	extern __shared__ float vb_smem[];
-	pdl_prologue();
 	float* w = vb_smem;                              // [64][V + 1]
 	float* sh = vb_smem + 64 * (V + 1);              // [4][V]
 	for (int i = threadIdx.x; i < 64 * V; i += blockDim.x) {
@@ -576,7 +573,6 @@ __global__ void __launch_bounds__(256) view_bias_bwd_kernel(const float* __restr
 	float* __restrict__ grad_params)
 {
 	extern __shared__ float vb_smem[];
-	pdl_prologue();
 	float* g = vb_smem;                              // [kBiasBwdRays][64]
 	float* sh = vb_smem + kBiasBwdRays * 64;         // [kBiasBwdRays][V]
 	const int64_t ray0 = static_cast<int64_t>(blockIdx.x) * kBiasBwdRays;
@@ -639,7 +635,7 @@ int nrf_mlp_small_pack(const nrf_mlp_small_shape* shape, const float* params_fla
 	if (int rc = check_shape(shape)) return rc;
 	NRF_REQUIRE(params_flat && packed, "null pointer");
 	NRF_REQUIRE((reinterpret_cast<uintptr_t>(packed) & 15) == 0, "packed blob must be 16-byte aligned");
-	launch_kernel(mlp_pack_kernel, (kPackedWords + 255) / 256, 256, 0, as_stream(stream), params_flat, shape->input_ch_views, reinterpret_cast<uint32_t*>(packed));
+	mlp_pack_kernel<<<(kPackedWords + 255) / 256, 256, 0, as_stream(stream)>>>(params_flat, shape->input_ch_views, reinterpret_cast<uint32_t*>(packed));
 	NRF_CHECK_LAUNCH("mlp_pack_kernel");
 	return NRF_OK;
 }
@@ -654,7 +650,7 @@ int nrf_mlp_small_view_bias_fwd(const nrf_mlp_small_shape* shape, const void* pa
 	const int V = shape->input_ch_views;
 	const size_t smem = static_cast<size_t>(64 * (V + 1) + 4 * V) * sizeof(float);
 	const unsigned blocks = static_cast<unsigned>((n_rays + kRaysPerBlock - 1) / kRaysPerBlock);
-	launch_kernel(view_bias_fwd_kernel, blocks, kViewBiasThreads, smem, as_stream(stream), reinterpret_cast<const uint32_t*>(packed), V, ray_sh, n_rays, bias_out,
+	view_bias_fwd_kernel<<<blocks, kViewBiasThreads, smem, as_stream(stream)>>>(reinterpret_cast<const uint32_t*>(packed), V, ray_sh, n_rays, bias_out,
 		grad_bias_zero);
 	NRF_CHECK_LAUNCH("view_bias_fwd_kernel");
 	return NRF_OK;
@@ -670,7 +666,7 @@ int nrf_mlp_small_view_bias_bwd(const nrf_mlp_small_shape* shape, const float* r
 	const int V = shape->input_ch_views;
 	const size_t smem = static_cast<size_t>(kBiasBwdRays) * (64 + V) * sizeof(float);
 	const unsigned blocks = static_cast<unsigned>((n_rays + kBiasBwdRays - 1) / kBiasBwdRays);
-	launch_kernel(view_bias_bwd_kernel, blocks, 256, smem, as_stream(stream), ray_sh, V, grad_bias, n_rays, grad_params_flat);
+	view_bias_bwd_kernel<<<blocks, 256, smem, as_stream(stream)>>>(ray_sh, V, grad_bias, n_rays, grad_params_flat);
 	NRF_CHECK_LAUNCH("view_bias_bwd_kernel");
 	return NRF_OK;
 }
@@ -737,7 +733,7 @@ int nrf_mlp_small_bwd_raybias(const nrf_mlp_small_shape* shape, const void* pack
 	if (in_kind == NRF_MLP_IN_ENC16_RAYDIRS) kernel = mlp_small_bwd_kernel<NRF_MLP_IN_ENC16_RAYDIRS>;
 	else if (in_kind == NRF_MLP_IN_ENC16_RAYBIAS) kernel = mlp_small_bwd_kernel<NRF_MLP_IN_ENC16_RAYBIAS>;
 	NRF_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(kBwdSmem)));
-	launch_kernel(kernel, blocks, kBwdWarps * 32, kBwdSmem, as_stream(stream), blob, enc, ray_sh, samples_per_ray, keep, n, grad_raw, grad_in,
+	kernel<<<blocks, kBwdWarps * 32, kBwdSmem, as_stream(stream)>>>(blob, enc, ray_sh, samples_per_ray, keep, n, grad_raw, grad_in,
 		grad_params_flat, V, grad_bias);
 	NRF_CHECK_LAUNCH("mlp_small_bwd_kernel");
 	return NRF_OK;

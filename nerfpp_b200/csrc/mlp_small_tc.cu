@@ -156,7 +156,6 @@ __global__ void __launch_bounds__(kThreads, 1) mlp_small_fwd_tc_kernel(const uin
 	const float* __restrict__ ray_sh, int S, const uint8_t* __restrict__ keep, int64_t n, RowMap map, float* __restrict__ raw_out)
 {
 	__shared__ Smem sm;
-	pdl_prologue();
 	const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 	const int64_t n_tiles = (n + 127) / 128;
 
@@ -296,11 +295,11 @@ cudaError_t launch_mlp_small_fwd_tc(const uint32_t* blob, int in_kind, const voi
 	const int blocks = static_cast<int>(std::min<int64_t>((tiles + tc::kSlots - 1) / tc::kSlots, kNumSMs));
 	const tc::RowMap none{nullptr, 1, 1};
 	if (in_kind == NRF_MLP_IN_ENC16_RAYDIRS)
-		launch_kernel(tc::mlp_small_fwd_tc_kernel<NRF_MLP_IN_ENC16_RAYDIRS, false>, blocks, tc::kThreads, 0, stream, blob, enc, ray_sh, S, keep, n, none, raw_out);
+		tc::mlp_small_fwd_tc_kernel<NRF_MLP_IN_ENC16_RAYDIRS, false><<<blocks, tc::kThreads, 0, stream>>>(blob, enc, ray_sh, S, keep, n, none, raw_out);
 	else if (in_kind == NRF_MLP_IN_ENC16_RAYBIAS)
-		launch_kernel(tc::mlp_small_fwd_tc_kernel<NRF_MLP_IN_ENC16_RAYBIAS, false>, blocks, tc::kThreads, 0, stream, blob, enc, ray_sh, S, keep, n, none, raw_out);
+		tc::mlp_small_fwd_tc_kernel<NRF_MLP_IN_ENC16_RAYBIAS, false><<<blocks, tc::kThreads, 0, stream>>>(blob, enc, ray_sh, S, keep, n, none, raw_out);
 	else
-		launch_kernel(tc::mlp_small_fwd_tc_kernel<NRF_MLP_IN_F32_CAT, false>, blocks, tc::kThreads, 0, stream, blob, enc, ray_sh, S, keep, n, none, raw_out);
+		tc::mlp_small_fwd_tc_kernel<NRF_MLP_IN_F32_CAT, false><<<blocks, tc::kThreads, 0, stream>>>(blob, enc, ray_sh, S, keep, n, none, raw_out);
 	return cudaGetLastError();
 }
 
@@ -312,9 +311,9 @@ cudaError_t launch_mlp_small_fwd_tc_importance(const uint32_t* blob, int in_kind
 	const int blocks = static_cast<int>(std::min<int64_t>((tiles + tc::kSlots - 1) / tc::kSlots, kNumSMs));
 	const tc::RowMap map{perm, n_importance, n_merged};
 	if (in_kind == NRF_MLP_IN_ENC16_RAYBIAS)
-		launch_kernel(tc::mlp_small_fwd_tc_kernel<NRF_MLP_IN_ENC16_RAYBIAS, true>, blocks, tc::kThreads, 0, stream, blob, enc, ray_sh, n_importance, keep, n, map, raw_out);
+		tc::mlp_small_fwd_tc_kernel<NRF_MLP_IN_ENC16_RAYBIAS, true><<<blocks, tc::kThreads, 0, stream>>>(blob, enc, ray_sh, n_importance, keep, n, map, raw_out);
 	else
-		launch_kernel(tc::mlp_small_fwd_tc_kernel<NRF_MLP_IN_ENC16_RAYDIRS, true>, blocks, tc::kThreads, 0, stream, blob, enc, ray_sh, n_importance, keep, n, map, raw_out);
+		tc::mlp_small_fwd_tc_kernel<NRF_MLP_IN_ENC16_RAYDIRS, true><<<blocks, tc::kThreads, 0, stream>>>(blob, enc, ray_sh, n_importance, keep, n, map, raw_out);
 	return cudaGetLastError();
 }
 

@@ -59,7 +59,6 @@ struct AdamSchedState {
 
 __global__ void adam_schedule_kernel(AdamSchedState* st, double lr0, double decay_rate, double decay_steps, double beta1, double beta2)
 {
-	pdl_prologue();
 	if (threadIdx.x != 0 || blockIdx.x != 0) return;
 	const int step = st->step + 1;
 	// src/NeRFExecutor.h:986-996: step() runs with the rate set at the END of the previous iteration, lr0 * rate^(global_step / decay_steps)
@@ -109,7 +108,6 @@ __device__ __forceinline__ void st_hint2(void* p, uint32_t a, uint32_t b, uint64
 __global__ void __launch_bounds__(256) adam_kernel(float* __restrict__ param, float* __restrict__ grad, float* __restrict__ m,
 	float* __restrict__ v, int64_t n, AdamArgs a, int zero_grad, __half* __restrict__ shadow, const AdamSchedState* __restrict__ sched)
 {
-	pdl_prologue();
 	if (sched) {
 		a.lr_over_bc1 = sched->lr_over_bc1;
 		a.inv_sqrt_bc2 = sched->inv_sqrt_bc2;
@@ -187,7 +185,7 @@ int nrf_adam_schedule_advance(void* sched_state, float lr0, float decay_rate, fl
 {
 	NRF_REQUIRE(sched_state != nullptr, "null schedule state");
 	NRF_REQUIRE((reinterpret_cast<uintptr_t>(sched_state) & 15) == 0, "schedule state must be 16-byte aligned");
-	launch_kernel(adam_schedule_kernel, 1, 32, 0, as_stream(stream), reinterpret_cast<AdamSchedState*>(sched_state), static_cast<double>(lr0),
+	adam_schedule_kernel<<<1, 32, 0, as_stream(stream)>>>(reinterpret_cast<AdamSchedState*>(sched_state), static_cast<double>(lr0),
 		static_cast<double>(decay_rate), static_cast<double>(decay_steps), static_cast<double>(beta1), static_cast<double>(beta2));
 	NRF_CHECK_LAUNCH("adam_schedule_kernel");
 	return NRF_OK;
@@ -207,7 +205,7 @@ int nrf_adam_step_scheduled(float* param, float* grad, float* exp_avg, float* ex
 	a.beta1 = beta1; a.beta2 = beta2; a.eps = eps; a.grad_scale = grad_scale;
 	const int64_t quads = (n + 3) / 4;
 	const int blocks = static_cast<int>(std::min<int64_t>((quads + 255) / 256, kNumSMs * 8));
-	launch_kernel(adam_kernel, blocks, 256, 0, as_stream(stream), param, grad, exp_avg, exp_avg_sq, n, a, zero_grad,
+	adam_kernel<<<blocks, 256, 0, as_stream(stream)>>>(param, grad, exp_avg, exp_avg_sq, n, a, zero_grad,
 		reinterpret_cast<__half*>(shadow_f16), reinterpret_cast<const AdamSchedState*>(sched_state));
 	NRF_CHECK_LAUNCH("adam_kernel");
 	return NRF_OK;

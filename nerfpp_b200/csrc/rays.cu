@@ -146,7 +146,6 @@ __global__ void __launch_bounds__(256) ray_setup_kernel(const float* __restrict_
 	float near_plane, const float* __restrict__ t_vals, int S, int lin_disp, float* __restrict__ ray_batch, float* __restrict__ z,
 	float* __restrict__ ray_sh, float* __restrict__ zero_scalar)
 {
-	pdl_prologue();
 	const int64_t e = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
 	if (e == 0 && zero_scalar) *zero_scalar = 0.f;
 	if (e >= R * S) return;
@@ -319,8 +318,8 @@ static int launch_ray_setup(bool pixels, const float* rays_o, const float* rays_
 	const unsigned blocks = static_cast<unsigned>((n + 255) / 256);
 	cudaStream_t s = as_stream(stream);
 #define NRF_RS(D) case D:                                                                                                                                     \
-		if (pixels) launch_kernel(ray_setup_kernel<D, true>, blocks, 256, 0, s, rays_o, rays_d, ps, n_rays, b, near_plane, t_vals, n_samples, lin_disp, ray_batch, z, ray_sh, zero_scalar); \
-		else launch_kernel(ray_setup_kernel<D, false>, blocks, 256, 0, s, rays_o, rays_d, ps, n_rays, b, near_plane, t_vals, n_samples, lin_disp, ray_batch, z, ray_sh, zero_scalar);   \
+		if (pixels) ray_setup_kernel<D, true><<<blocks, 256, 0, s>>>(rays_o, rays_d, ps, n_rays, b, near_plane, t_vals, n_samples, lin_disp, ray_batch, z, ray_sh, zero_scalar); \
+		else ray_setup_kernel<D, false><<<blocks, 256, 0, s>>>(rays_o, rays_d, ps, n_rays, b, near_plane, t_vals, n_samples, lin_disp, ray_batch, z, ray_sh, zero_scalar);   \
 		break
 	switch (ray_sh ? sh_degree : 1) {
 		NRF_RS(1); NRF_RS(2); NRF_RS(3); NRF_RS(4); NRF_RS(5); NRF_RS(6); NRF_RS(7); NRF_RS(8);

@@ -10,6 +10,10 @@
 
 namespace nrf {
 
+// The rays of a chunk are adjacent pixels of a frame (GetRays order): the encode kernel walks the same sample of kRayGroup neighbouring rays
+// together (nrf_hash_encode_rays_fwd_grouped).
+constexpr int kRayGroup = 32;
+
 static inline int64_t align256(int64_t v) { return (v + 255) & ~int64_t(255); }
 
 struct RenderWs {
@@ -98,12 +102,7 @@ static int render_impl(const nrf_render_config* cfg, const nrf_hash_grid* grid, 
 	float* raw_coarse = reinterpret_cast<float*>(base + w.raw_coarse);
 	int16_t* perm = reinterpret_cast<int16_t*>(base + w.perm);
 	// One network for both passes (src/NeRFRenderer.h:422,447): the merged fine pass re-uses the coarse pass's raw rows for the coarse
-	// samples and gathers / evaluates the importance samples only — the same bits as evaluating all S + N rows (tests/test_gpu_render.py).
-	// NRF_RENDER_REUSE=0 evaluates every merged row (the A/B baseline).
-	static const bool reuse = [] { const char* e = getenv("NRF_RENDER_REUSE"); return !(e && e[0] == '0'); }();
-	// The rays of a chunk are adjacent pixels of a frame (GetRays order): the encode kernel walks the same sample of kRayGroup neighbouring rays
-	// together (nrf_hash_encode_rays_fwd_grouped).  NRF_RENDER_RAY_GROUP=1 restores the per-ray order (the A/B baseline).
-	static const int group = [] { const char* e = getenv("NRF_RENDER_RAY_GROUP"); const int g = e ? atoi(e) : 32; return g >= 1 && g <= 1024 ? g : 32; }();
+	// samples and gathers / evaluates the importance samples only — the same bits as evaluating all S + N rows (tests/test_gpu_pipeline.py).
 
 	int rc;
 	// Render prologue + coarse depths + per-ray SH table: one launch (bit-identical to nrf_rays_prepare + nrf_sh_encode_fwd + nrf_z_sample)
@@ -130,23 +129,16 @@ static int render_impl(const nrf_render_config* cfg, const nrf_hash_grid* grid, 
 		views = vb;
 	}
 	// coarse pass
-	if ((rc = nrf_hash_encode_rays_fwd_grouped(grid, table_f16, ray_batch, 11, z, n_rays, S, 1, keep, enc, NRF_ENC_F16, nullptr, nullptr, nullptr, 0, group, stream)))
+	if ((rc = nrf_hash_encode_rays_fwd_grouped(grid, table_f16, ray_batch, 11, z, n_rays, S, 1, keep, enc, NRF_ENC_F16, nullptr, nullptr, nullptr, 0, kRayGroup, stream)))
 		return rc;
-	if ((rc = nrf_mlp_small_fwd(shape, packed, kind, enc, views, S, keep, n_rays * S, reuse ? raw_coarse : raw, stream))) return rc;
-	if ((rc = nrf_composite_fwd(reuse ? raw_coarse : raw, 4, z, rays_d, nullptr, 0.f, cfg->white_bkgr, n_rays, S, nullptr, nullptr, nullptr, nullptr, w_coarse,
+	if ((rc = nrf_mlp_small_fwd(shape, packed, kind, enc, views, S, keep, n_rays * S, raw_coarse, stream))) return rc;
+	if ((rc = nrf_composite_fwd(raw_coarse, 4, z, rays_d, nullptr, 0.f, cfg->white_bkgr, n_rays, S, nullptr, nullptr, nullptr, nullptr, w_coarse,
 	                            stream))) return rc;
 	// importance sampling + merge, fine pass
-	if (reuse) {
-		if ((rc = nrf_sample_pdf_merge_rows(z, w_coarse, u, 0, n_rays, S, N, nullptr, z_fine, perm, raw_coarse, raw, stream))) return rc;
-		if ((rc = nrf_hash_encode_rays_fwd_grouped(grid, table_f16, ray_batch, 11, z_fine, n_rays, T, 1, keep, enc, NRF_ENC_F16, perm, nullptr, nullptr, S, group,
-		                                           stream))) return rc;
-		if ((rc = nrf_mlp_small_fwd_importance(shape, packed, kind, enc, views, keep, perm, n_rays, N, T, raw, stream))) return rc;
-	} else {
-		if ((rc = nrf_sample_pdf_merge(z, w_coarse, u, 0, n_rays, S, N, nullptr, z_fine, stream))) return rc;
-		if ((rc = nrf_hash_encode_rays_fwd_grouped(grid, table_f16, ray_batch, 11, z_fine, n_rays, T, 1, keep, enc, NRF_ENC_F16, nullptr, nullptr, nullptr, 0, group,
-		                                           stream))) return rc;
-		if ((rc = nrf_mlp_small_fwd(shape, packed, kind, enc, views, T, keep, n_rays * T, raw, stream))) return rc;
-	}
+	if ((rc = nrf_sample_pdf_merge_rows(z, w_coarse, u, 0, n_rays, S, N, nullptr, z_fine, perm, raw_coarse, raw, stream))) return rc;
+	if ((rc = nrf_hash_encode_rays_fwd_grouped(grid, table_f16, ray_batch, 11, z_fine, n_rays, T, 1, keep, enc, NRF_ENC_F16, perm, nullptr, nullptr, S, kRayGroup,
+	                                           stream))) return rc;
+	if ((rc = nrf_mlp_small_fwd_importance(shape, packed, kind, enc, views, keep, perm, n_rays, N, T, raw, stream))) return rc;
 	if ((rc = nrf_composite_fwd(raw, 4, z_fine, rays_d, nullptr, 0.f, cfg->white_bkgr, n_rays, T, rgb, depth, disp, acc, weights, stream))) return rc;
 	return NRF_OK;
 }

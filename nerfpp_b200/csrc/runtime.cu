@@ -2,7 +2,6 @@
 #include "common.cuh"
 #include <atomic>
 #include <cstdarg>
-#include <cstdlib>
 
 namespace nrf {
 
@@ -18,12 +17,6 @@ void set_error(const char* fmt, ...)
 }
 
 void count_launch(int n) { g_launches.fetch_add(n, std::memory_order_relaxed); }
-
-bool pdl_enabled()
-{
-	static const bool v = [] { const char* e = getenv("NRF_PDL"); return e && e[0] == '1'; }();   // opt-in: measured gain 3 us of 812 (DESIGN.md §4)
-	return v;
-}
 
 }  // namespace nrf
 

@@ -141,7 +141,6 @@ __global__ void __launch_bounds__(kSamplerWarps * 32) sample_pdf_merge_kernel(co
 	float4* __restrict__ rows_merged, int per_warp_floats, int sort_pow2)
 {
 	extern __shared__ float smem[];
-	pdl_prologue();
 	const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 	const int64_t ray = static_cast<int64_t>(blockIdx.x) * kSamplerWarps + warp;
 	if (ray >= R) return;
@@ -227,7 +226,6 @@ __global__ void __launch_bounds__(kSamplerBlock) sample_pdf_merge_block_kernel(c
 	const float4* __restrict__ rows_coarse, float4* __restrict__ rows_merged)
 {
 	extern __shared__ float smem[];
-	pdl_prologue();
 	const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, tid = threadIdx.x;
 	const int64_t ray = blockIdx.x;
 	const int B = S - 1;
@@ -359,19 +357,18 @@ int nrf_sample_pdf_merge_rows(const float* z_coarse, const float* weights, const
 	const int per_warp = 2 * (n_samples - 1) + n_importance + n_samples + (u_per_ray ? pow2 : 0);
 	const size_t smem = static_cast<size_t>(kSamplerWarps) * per_warp * sizeof(float);
 	NRF_REQUIRE(smem <= 48 * 1024, "shared memory budget exceeded");
-	// few rays (a training batch): one CTA per ray, latency of 3 searches instead of 14; many rays (a render chunk): one warp per ray, fewer
-	// instructions per ray.  NRF_SAMPLER_BLOCK=0 / 1 forces the warp / CTA kernel (tests, A/B).
-	static const int force = [] { const char* e = getenv("NRF_SAMPLER_BLOCK"); return e ? atoi(e) : -1; }();
-	const bool per_block = !u_per_ray && (force == 1 || (force != 0 && n_rays <= kBlockPerRayMaxRays));
+	// few rays (a training batch): one CTA per ray, latency of 3 searches instead of 14; many rays (a render chunk) or per-ray u: one warp
+	// per ray, fewer instructions per ray
+	const bool per_block = !u_per_ray && n_rays <= kBlockPerRayMaxRays;
 	if (per_block) {
 		const size_t smem_b = static_cast<size_t>(2 * (n_samples - 1) + n_importance + n_samples) * sizeof(float);
-		launch_kernel(sample_pdf_merge_block_kernel, static_cast<unsigned>(n_rays), kSamplerBlock, smem_b, as_stream(stream), z_coarse, weights, u, n_rays,
+		sample_pdf_merge_block_kernel<<<static_cast<unsigned>(n_rays), kSamplerBlock, smem_b, as_stream(stream)>>>(z_coarse, weights, u, n_rays,
 			n_samples, n_importance, z_samples, z_merged, perm_out, reinterpret_cast<const float4*>(rows_coarse), reinterpret_cast<float4*>(rows_merged));
 		NRF_CHECK_LAUNCH("sample_pdf_merge_block_kernel");
 		return NRF_OK;
 	}
 	const unsigned blocks = static_cast<unsigned>((n_rays + kSamplerWarps - 1) / kSamplerWarps);
-	launch_kernel(sample_pdf_merge_kernel, blocks, kSamplerWarps * 32, smem, as_stream(stream), z_coarse, weights, u, u_per_ray, n_rays,
+	sample_pdf_merge_kernel<<<blocks, kSamplerWarps * 32, smem, as_stream(stream)>>>(z_coarse, weights, u, u_per_ray, n_rays,
 		n_samples, n_importance, z_samples, z_merged, perm_out, reinterpret_cast<const float4*>(rows_coarse), reinterpret_cast<float4*>(rows_merged),
 		per_warp, pow2);
 	NRF_CHECK_LAUNCH("sample_pdf_merge_kernel");

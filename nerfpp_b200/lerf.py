@@ -19,7 +19,6 @@ CLIP target, backward, Adam over {lang_embedder, lang_model}): `LeRFField.train_
 from __future__ import annotations
 
 import math
-import os
 
 import torch
 
@@ -79,7 +78,7 @@ class LeRFField(FlatAdamModel):
         self.u = torch.linspace(0.0, 1.0, n_importance, dtype=f32).to(device)                     # src/Sampler.h:20
         self.packed = None
         self._render_graph = None
-        self.render_ray_group = int(os.environ.get("NRF_RENDER_RAY_GROUP", "32"))   # render_image: GetRays order = adjacent pixels
+        self.render_ray_group = 32           # render_image: GetRays order = adjacent pixels
         self.reuse_coarse_rows = True        # the fine pass copies the coarse samples' encoding rows instead of gathering them again (bit-identical)
         self._bwd_ws = None
         self.refresh()

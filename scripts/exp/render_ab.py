@@ -1,5 +1,5 @@
-"""C4 render frame (1920x1080, 64 + 64 samples, 131072-ray chunks) under the environment switches of the render path; prints ms/frame.
-Usage: [NRF_RENDER_REUSE=0] [NRF_HASH_SPLIT=0] python scripts/exp/render_ab.py"""
+"""C4 render frame (1920x1080, 64 + 64 samples, 131072-ray chunks); prints ms/frame.
+Usage: python scripts/exp/render_ab.py"""
 import json
 import math
 import os

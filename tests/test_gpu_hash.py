@@ -17,6 +17,10 @@ def _grid(L=16, F=2, T=19, base=16, finest=512, seed=1):
     return pipeline.make_grid(BBOX, L, F, T, base, finest, "cuda", seed)
 
 
+# L16 F2: the forward runs four lanes per point; L12 F2 (three 16-byte chunks per row, not a power of two): one thread per point
+SHAPES = [(16, 2), (12, 2)]
+
+
 def _np(grid):
     grid.c_struct()  # materialises the device-computed level scales
     return dict(box_min=BBOX[:3], box_max=BBOX[3:], scales=grid.level_scale.cpu().numpy(),
@@ -105,10 +109,10 @@ def test_every_point_level_corner_address_is_bit_exact(F, T):
     assert got.max() + F <= grid.used_scalars()
 
 
-@pytest.mark.parametrize("table_kind", ["init", "unit"])
-def test_forward_matches_oracle(table_kind):
+@pytest.mark.parametrize("table_kind,L", [("init", 16), ("unit", 16), ("init", 12), ("unit", 12)], ids=["init", "unit", "init-L12F2", "unit-L12F2"])
+def test_forward_matches_oracle(table_kind, L):
     from nerfpp_b200 import ops
-    grid = _grid()
+    grid = _grid(L=L)
     meta = _np(grid)
     g = torch.Generator().manual_seed(5)
     n_sc = grid.table_scalars()
@@ -273,9 +277,14 @@ def _ray_batch(n_rays, seed=0):
 
 def test_fused_point_generation_is_bit_identical():
     """nrf_hash_encode_rays_fwd/_bwd (points built in-kernel from ray_batch and z) == nrf_sample_points followed by the
-    point-array entries, bit for bit (forward) / to accumulation order (backward), incl. rays that miss the box."""
+    point-array entries, bit for bit (forward) / to accumulation order (backward), incl. rays that miss the box; at each of SHAPES."""
+    for L, F in SHAPES:
+        _fused_point_generation(L, F)
+
+
+def _fused_point_generation(L, F):
     from nerfpp_b200 import ops
-    grid = _grid()
+    grid = _grid(L=L, F=F)
     g = torch.Generator(device="cuda").manual_seed(4)
     t16 = ops.table_to_half(torch.rand(grid.table_scalars(), generator=g, device="cuda") * 2 - 1)
     rb = _ray_batch(300, seed=2)
@@ -286,7 +295,7 @@ def test_fused_point_generation_is_bit_identical():
     assert torch.equal(e0, e1) and torch.equal(k0, k1)
     e2, _ = ops.hash_encode_rays_fwd(grid, t16, rb, z, clamp=True, out_f16=False)
     assert torch.equal(e2, ops.hash_encode_fwd(grid, t16, pts.view(-1, 3), clamp=True)[0])
-    G = torch.randn(300 * 77, 32, generator=g, device="cuda").bfloat16()
+    G = torch.randn(300 * 77, L * F, generator=g, device="cuda").bfloat16()
     g0 = torch.zeros(grid.table_scalars(), device="cuda")
     g1 = torch.zeros_like(g0)
     ops.hash_encode_bwd(grid, pts.view(-1, 3), G, g0)
@@ -298,9 +307,14 @@ def test_fused_point_generation_is_bit_identical():
 def test_coarse_row_reuse_is_bit_identical():
     """The fine pass copies the encoding rows of the coarse samples it contains (same z => same point): the result must
     equal a full re-encode bit for bit, perm must name only bit-identical z, and EVERY coarse sample must be found — also on the
-    ray that misses the box, whose coarse depths the merge re-orders.  The raw-row scatter follows the same positions."""
+    ray that misses the box, whose coarse depths the merge re-orders.  The raw-row scatter follows the same positions.  At each of SHAPES."""
+    for L, F in SHAPES:
+        _coarse_row_reuse(L, F)
+
+
+def _coarse_row_reuse(L, F):
     from nerfpp_b200 import ops
-    grid = _grid()
+    grid = _grid(L=L, F=F)
     g = torch.Generator(device="cuda").manual_seed(6)
     t16 = ops.table_to_half(torch.rand(grid.table_scalars(), generator=g, device="cuda") * 2 - 1)
     R, S, N = 257, 64, 128
@@ -341,12 +355,13 @@ def test_coarse_row_reuse_is_bit_identical():
     assert torch.equal(full, fast) and torch.equal(keep_full, keep_fast)
 
 
-@pytest.mark.parametrize("feat", [2, 8])
-def test_ray_grouped_order_changes_no_bit(feat):
+@pytest.mark.parametrize("L,feat", [(16, 2), (16, 8), (12, 2)], ids=["2", "8", "L12F2"])
+def test_ray_grouped_order_changes_no_bit(L, feat):
     """nrf_hash_encode_rays_fwd_grouped walks the same sample of ray_group neighbouring rays together: rows and keep flags are those of the
-    per-ray order, for a ragged ray count (not a multiple of the group), with and without row reuse, at F = 2 (4 lanes / point) and F = 8 (16)."""
+    per-ray order, for a ragged ray count (not a multiple of the group), with and without row reuse, at L16 F = 2 (4 lanes / point) and F = 8
+    (16), and at L12 F2 (one thread per point)."""
     from nerfpp_b200 import ops
-    grid = _grid(F=feat, T=16)
+    grid = _grid(L=L, F=feat, T=16)
     g = torch.Generator(device="cuda").manual_seed(16)
     t16 = ops.table_to_half(torch.rand(grid.table_scalars(), generator=g, device="cuda") * 2 - 1)
     R, S, N = 301, 64, 64

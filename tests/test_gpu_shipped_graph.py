@@ -2,8 +2,6 @@
 from FillRenderParams, src/NeRFExecutor.h:411-412) on the fast path: jittered sample points generated inside the hash kernels
 (nrf_hash_encode_rays_jitter_fwd / _bwd) and HashNeRFTrainGraph driven through train_steps_shipped."""
 import ctypes
-import os
-import subprocess
 import sys
 
 import numpy as np
@@ -11,12 +9,13 @@ import pytest
 import torch
 
 BBOX = [-1.5, -1.5, -1.5, 1.5, 1.5, 1.5]
-HERE = os.path.dirname(os.path.abspath(__file__))
+# grid shapes (L, F): the hash forward runs four lanes per point at L16 F2, one thread per point at L12 F2 (three 16-byte chunks per row)
+SHAPES = [(16, 2), (12, 2)]
 
 
-def _grid():
+def _grid(L, F):
     from nerfpp_b200 import pipeline
-    return pipeline.make_grid(BBOX, 16, 2, 19, 16, 512, "cuda", 1)
+    return pipeline.make_grid(BBOX, L, F, 19, 16, 512, "cuda", 1)
 
 
 def _case(n_rays=300, n_samples=77, seed=2):
@@ -48,18 +47,20 @@ def _composed(rb, z, cone, rand_r, rand_t, clamp, noise, alpha):
     return pts.view(-1, 3)
 
 
-# (stochastic preconditioning, cone: None / "scalar" / "ray", clamp)
+# (stochastic preconditioning, cone: None / "scalar" / "ray", clamp) at each grid shape; the L16 F2 cases keep their ids
 CASES = [(False, "scalar", True), (False, "scalar", False), (False, "ray", True), (False, "ray", False),
          (True, "scalar", True), (True, "scalar", False), (True, "ray", True), (True, "ray", False), (True, None, False)]
+SHAPED_CASES = [c + s for s in SHAPES for c in CASES]
+SHAPED_IDS = [f"sp{int(a)}-{b}-clamp{int(c)}" + ("" if (L, F) == SHAPES[0] else f"-L{L}F{F}") for a, b, c, L, F in SHAPED_CASES]
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("sp,cone_kind,clamp", CASES, ids=[f"sp{int(a)}-{b}-clamp{int(c)}" for a, b, c in CASES])
-def test_jitter_encode_equals_the_composed_path(sp, cone_kind, clamp):
+@pytest.mark.parametrize("sp,cone_kind,clamp,L,F", SHAPED_CASES, ids=SHAPED_IDS)
+def test_jitter_encode_equals_the_composed_path(sp, cone_kind, clamp, L, F):
     """Same variates: the in-kernel points give the encoding and keep mask of the materialised ones bit for bit (forward), and the scatter of
     nrf_hash_encode_bwd on them to accumulation order (backward) — incl. rays that miss the box, which the clamp pulls onto its surface."""
     from nerfpp_b200 import ops
-    grid = _grid()
+    grid = _grid(L, F)
     g = torch.Generator(device="cuda").manual_seed(4)
     t16 = ops.table_to_half(torch.rand(grid.table_scalars(), generator=g, device="cuda") * 2 - 1)
     rb, z, rand_r, rand_t, noise, cone_ray = _case()
@@ -79,7 +80,7 @@ def test_jitter_encode_equals_the_composed_path(sp, cone_kind, clamp):
         assert bool(k1.bool().all())                                   # clamped into the box: every sample passes the keep test
     elif cone is not None:
         assert not bool(k1.bool().all())                               # the rays that miss the box stay outside
-    G = torch.randn(pts.shape[0], 32, generator=g, device="cuda").bfloat16()
+    G = torch.randn(pts.shape[0], L * F, generator=g, device="cuda").bfloat16()
     g0 = torch.zeros(grid.table_scalars(), device="cuda")
     g1 = torch.zeros_like(g0)
     ops.hash_encode_bwd(grid, pts, G, g0)
@@ -90,24 +91,17 @@ def test_jitter_encode_equals_the_composed_path(sp, cone_kind, clamp):
 
 @pytest.mark.gpu
 def test_zero_amplitudes_are_the_parity_kernel():
-    """Cone angle 0, no preconditioning, no clamp: the jitter entry encodes exactly what nrf_hash_encode_rays_fwd does."""
+    """Cone angle 0, no preconditioning, no clamp: the jitter entry encodes exactly what nrf_hash_encode_rays_fwd does, at each grid shape."""
     from nerfpp_b200 import ops
-    grid = _grid()
-    g = torch.Generator(device="cuda").manual_seed(6)
-    t16 = ops.table_to_half(torch.rand(grid.table_scalars(), generator=g, device="cuda") * 2 - 1)
-    rb, z, rand_r, rand_t, _, _ = _case(seed=5)
-    jit = ops.PointJitter(torch.zeros(1, device="cuda"), rand_r, rand_t, False)
-    e0, k0 = ops.hash_encode_rays_fwd(grid, t16, rb, z, clamp=True, out_f16=True)
-    e1, k1 = ops.hash_encode_rays_fwd(grid, t16, rb, z, clamp=True, out_f16=True, jitter=jit)
-    assert torch.equal(e0, e1) and torch.equal(k0, k1)
-
-
-@pytest.mark.gpu
-def test_jitter_encode_with_one_thread_per_point():
-    """The comparisons above with the hash forward at one thread per point (NRF_HASH_SPLIT=0) instead of four lanes per point."""
-    cmd = [sys.executable, "-m", "pytest", "-q", "-x", "--no-header", "-k", "composed_path or parity_kernel", os.path.abspath(__file__)]
-    out = subprocess.run(cmd, capture_output=True, text=True, timeout=600, env={**os.environ, "NRF_HASH_SPLIT": "0"})
-    assert out.returncode == 0 and " passed" in out.stdout, out.stdout[-3000:] + out.stderr[-2000:]
+    for L, F in SHAPES:
+        grid = _grid(L, F)
+        g = torch.Generator(device="cuda").manual_seed(6)
+        t16 = ops.table_to_half(torch.rand(grid.table_scalars(), generator=g, device="cuda") * 2 - 1)
+        rb, z, rand_r, rand_t, _, _ = _case(seed=5)
+        jit = ops.PointJitter(torch.zeros(1, device="cuda"), rand_r, rand_t, False)
+        e0, k0 = ops.hash_encode_rays_fwd(grid, t16, rb, z, clamp=True, out_f16=True)
+        e1, k1 = ops.hash_encode_rays_fwd(grid, t16, rb, z, clamp=True, out_f16=True, jitter=jit)
+        assert torch.equal(e0, e1) and torch.equal(k0, k1), (L, F)
 
 
 def test_jitter_entries_validate_their_arguments_without_gpu():

@@ -126,12 +126,6 @@ int nrf_hash_encode_rays_fwd_grouped(const nrf_hash_grid* grid, const void* tabl
 int nrf_hash_encode_rays_bwd(const nrf_hash_grid* grid, const float* ray_batch, int32_t ray_stride, const float* z,
                              int64_t n_rays, int32_t n_samples, int clamp_points, const void* grad_enc, nrf_grad_layout layout,
                              float* grad_table, nrf_stream stream);
-/* The same scatter for levels [level_begin, level_end) only (level_end < 0: n_levels).  Two calls over [0, k) and [k, L) add up to the full
- * gradient; grad_table below level k's offset is complete after the first call, so a data-parallel exchange of that prefix can run while the
- * second call scatters (nerfpp_b200/parallel.py). */
-int nrf_hash_encode_rays_bwd_levels(const nrf_hash_grid* grid, const float* ray_batch, int32_t ray_stride, const float* z,
-                                    int64_t n_rays, int32_t n_samples, int clamp_points, const void* grad_enc, nrf_grad_layout layout,
-                                    float* grad_table, int32_t level_begin, int32_t level_end, nrf_stream stream);
 
 /* The ray entries above with the per-sample perturbations of the reference's shipped training configuration (src/main.cpp:187
  * thin_ray = false; src/NeRFExecutor.h:411-412 RawNoiseStd / StochasticPreconditioningAlpha) applied inside the kernels, in the order of
@@ -529,13 +523,6 @@ int64_t nrf_peer_flags_bytes(int32_t world);
 int nrf_adam_step_sharded(const nrf_peer_group* pg, float* param, float* exp_avg, float* exp_avg_sq, int64_t n_sharded,
                           int64_t n_total, const void* sched_state, float beta1, float beta2, float eps, float grad_scale,
                           nrf_stream stream);
-/* The same step on part of the flat vector: sharded scalars [range_begin, range_end) (multiples of 4, partitioned over the ranks within the
- * range) and replicated scalars [tail_begin, tail_end); n_ctas CTAs (0: one per SM).  nrf_adam_step_sharded = one call over
- * [0, n_sharded / 4 * 4) + [n_sharded / 4 * 4, n_total).  A second call that may overlap a first one in time needs its own flag block
- * (a second nrf_peer_group over the same gradient / shadow buffers). */
-int nrf_adam_step_sharded_range(const nrf_peer_group* pg, float* param, float* exp_avg, float* exp_avg_sq, int64_t range_begin,
-                                int64_t range_end, int64_t tail_begin, int64_t tail_end, const void* sched_state, float beta1,
-                                float beta2, float eps, float grad_scale, int32_t n_ctas, nrf_stream stream);
 
 /* ------------------------------------------------------------------------------------------------------------
  * LeRF language head (SURVEY §8f-1, BASELINE C5) — LeRFImpl::forward (src/LeRF.cpp:28-111), the keep mask of

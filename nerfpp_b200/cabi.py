@@ -101,7 +101,6 @@ SIGNATURES = {
     "nrf_hash_encode_rays_fwd_grouped": (c_int32, [POINTER(HashGrid), _P, _P, c_int32, _P, c_int64, c_int32, c_int32, _P, _P, c_int32, _P, _P, _P, c_int32,
                                                    c_int32, _P]),
     "nrf_hash_encode_rays_bwd": (c_int32, [POINTER(HashGrid), _P, c_int32, _P, c_int64, c_int32, c_int32, _P, c_int32, _P, _P]),
-    "nrf_hash_encode_rays_bwd_levels": (c_int32, [POINTER(HashGrid), _P, c_int32, _P, c_int64, c_int32, c_int32, _P, c_int32, _P, c_int32, c_int32, _P]),
     "nrf_hash_encode_rays_jitter_fwd": (c_int32, [POINTER(HashGrid), _P, _P, c_int32, _P, c_int64, c_int32, c_int32, _P, _P, c_int32,
                                                   POINTER(PointJitter), _P]),
     "nrf_hash_encode_rays_jitter_bwd": (c_int32, [POINTER(HashGrid), _P, c_int32, _P, c_int64, c_int32, c_int32, _P, c_int32, _P,
@@ -172,8 +171,6 @@ SIGNATURES = {
     "nrf_lerf_bwd_rows": (c_int32, [POINTER(LerfShape), _P, POINTER(LerfWeights), _P, _P, _P, c_int64, c_int32, _P, POINTER(LerfWeights), _P, _P]),
     "nrf_peer_flags_bytes": (c_int64, [c_int32]),
     "nrf_adam_step_sharded": (c_int32, [POINTER(PeerGroup), _P, _P, _P, c_int64, c_int64, _P, c_float, c_float, c_float, c_float, _P]),
-    "nrf_adam_step_sharded_range": (c_int32, [POINTER(PeerGroup), _P, _P, _P, c_int64, c_int64, c_int64, c_int64, _P, c_float, c_float, c_float, c_float,
-                                              c_int32, _P]),
     "nrf_adam_schedule_advance": (c_int32, [_P, c_float, c_float, c_float, c_float, c_float, _P]),
     "nrf_adam_step_scheduled": (c_int32, [_P, _P, _P, _P, c_int64, _P, c_float, c_float, c_float, c_float, c_int32, _P, _P]),
 }

@@ -412,7 +412,7 @@ __device__ __forceinline__ void red_add_v4(float* addr, float a, float b, float 
 // Thread t handles points t, t + stride, ... (`iters` of them, warp-uniform; the launch passes iters = 1).
 template <int F, bool GRAD_BF16, class PS>
 __device__ __forceinline__ void hash_bwd_body(HashArgs a, PS ps, int64_t n_points, int64_t stride, int iters,
-	int clamp_points, const void* __restrict__ grad_enc, float* __restrict__ grad_table, int level_begin, int level_end)
+	int clamp_points, const void* __restrict__ grad_enc, float* __restrict__ grad_table)
 {
 	constexpr int CH = 8 / F;   // levels per 8-value gradient chunk (16 B of bf16 / 32 B of fp32)
 	constexpr uint32_t FULL = 0xffffffffu;
@@ -435,8 +435,7 @@ __device__ __forceinline__ void hash_bwd_body(HashArgs a, PS ps, int64_t n_point
 	const int D = L * F;
 	const int64_t row = i * static_cast<int64_t>(D);
 	const bool vec_ok = (D % 8) == 0;   // rows are 16-byte (bf16) / 32-byte (fp32) aligned
-	// levels [level_begin, level_end): [0, L) unless the caller splits the scatter by level range (any split; a chunk straddling it is read by both calls)
-	for (int l0 = level_begin / CH * CH; l0 < level_end; l0 += CH) {
+	for (int l0 = 0; l0 < L; l0 += CH) {
 		float g8[8];
 #pragma unroll
 		for (int k = 0; k < 8; k++) g8[k] = 0.f;
@@ -469,9 +468,9 @@ __device__ __forceinline__ void hash_bwd_body(HashArgs a, PS ps, int64_t n_point
 				}
 			}
 		}
-		for (int j = 0; j < CH; j++) {
+		const int jn = min(CH, L - l0);   // levels of this chunk (warp-uniform)
+		for (int j = 0; j < jn; j++) {
 			const int l = l0 + j;
-			if (l >= L || l >= level_end) break;   // warp-uniform
 			float g[F];
 			bool any = false;
 #pragma unroll
@@ -481,7 +480,6 @@ __device__ __forceinline__ void hash_bwd_body(HashArgs a, PS ps, int64_t n_point
 			}
 #pragma unroll
 			for (int k = 0; k + F < 8; k++) g8[k] = g8[k + F];   // next level's values move to the front (static indices only)
-			if (l < level_begin) continue;      // warp-uniform: the chunk straddles the lower bound of a level-split call
 			const bool active = valid && any;   // src/CuHashEmbedder.cu:195 skips all-zero gradients
 			Cell c;
 			locate(m, l, qx, qy, qz, c);
@@ -538,16 +536,16 @@ __device__ __forceinline__ void hash_bwd_body(HashArgs a, PS ps, int64_t n_point
 
 template <int F, bool GRAD_BF16>
 __global__ void __launch_bounds__(128) hash_bwd_kernel(HashArgs a, PointSrc ps, int64_t n_points, int64_t stride, int iters,
-	int clamp_points, const void* __restrict__ grad_enc, float* __restrict__ grad_table, int level_begin, int level_end)
+	int clamp_points, const void* __restrict__ grad_enc, float* __restrict__ grad_table)
 {
-	hash_bwd_body<F, GRAD_BF16>(a, ps, n_points, stride, iters, clamp_points, grad_enc, grad_table, level_begin, level_end);
+	hash_bwd_body<F, GRAD_BF16>(a, ps, n_points, stride, iters, clamp_points, grad_enc, grad_table);
 }
 
 template <int F, bool GRAD_BF16>
 __global__ void __launch_bounds__(128) hash_bwd_jitter_kernel(HashArgs a, JitterSrc ps, int64_t n_points, int64_t stride, int iters,
-	int clamp_points, const void* __restrict__ grad_enc, float* __restrict__ grad_table, int level_begin, int level_end)
+	int clamp_points, const void* __restrict__ grad_enc, float* __restrict__ grad_table)
 {
-	hash_bwd_body<F, GRAD_BF16>(a, ps, n_points, stride, iters, clamp_points, grad_enc, grad_table, level_begin, level_end);
+	hash_bwd_body<F, GRAD_BF16>(a, ps, n_points, stride, iters, clamp_points, grad_enc, grad_table);
 }
 
 // kernel of a point source, for the launch code shared by both
@@ -711,23 +709,19 @@ static int launch_hash_fwd(const nrf_hash_grid* grid, const void* table_f16, con
 
 template <class PS>
 static int launch_hash_bwd(const nrf_hash_grid* grid, const PS& ps, int64_t n_points, int clamp_points, const void* grad_enc,
-	nrf_grad_layout layout, float* grad_table, nrf_stream stream, int level_begin = 0, int level_end = -1)
+	nrf_grad_layout layout, float* grad_table, nrf_stream stream)
 {
 	HashArgs a;
 	if (int rc = fill_args(grid, a)) return rc;
 	NRF_REQUIRE(grad_table != nullptr && grad_enc != nullptr, "null grad_table / grad");
 	NRF_REQUIRE(layout == NRF_GRAD_F32 || layout == NRF_GRAD_BF16, "bad layout");
 	const int F = grid->n_features;
-	if (level_end < 0) level_end = grid->n_levels;
 	NRF_REQUIRE(F == 2 || F == 4 || F == 8, "n_features must be 2, 4 or 8");
-	NRF_REQUIRE(level_begin >= 0 && level_begin <= level_end && level_end <= grid->n_levels, "bad level range");
-	if (level_begin == level_end) return NRF_OK;
 	cudaStream_t s = as_stream(stream);
 #define NRF_LAUNCH_BWD2(FF, BF)                                                                                                   \
 	do {                                                                                                                          \
 		const LaunchPlan lp = launch_plan(n_points, 128);                                                                        \
-		bwd_kernel<FF, BF>(ps)<<<lp.grid, 128, 0, s>>>(a, ps, n_points, lp.stride, lp.iters, clamp_points, grad_enc, grad_table, level_begin, \
-			level_end);                                                                                                               \
+		bwd_kernel<FF, BF>(ps)<<<lp.grid, 128, 0, s>>>(a, ps, n_points, lp.stride, lp.iters, clamp_points, grad_enc, grad_table); \
 	} while (0)
 #define NRF_LAUNCH_BWD(FF)                                             \
 	do {                                                               \
@@ -802,20 +796,13 @@ int nrf_hash_encode_rays_fwd_grouped(const nrf_hash_grid* grid, const void* tabl
 int nrf_hash_encode_rays_bwd(const nrf_hash_grid* grid, const float* ray_batch, int32_t ray_stride, const float* z, int64_t n_rays,
 	int32_t n_samples, int clamp_points, const void* grad_enc, nrf_grad_layout layout, float* grad_table, nrf_stream stream)
 {
-	return nrf_hash_encode_rays_bwd_levels(grid, ray_batch, ray_stride, z, n_rays, n_samples, clamp_points, grad_enc, layout, grad_table, 0, -1, stream);
-}
-
-int nrf_hash_encode_rays_bwd_levels(const nrf_hash_grid* grid, const float* ray_batch, int32_t ray_stride, const float* z, int64_t n_rays,
-	int32_t n_samples, int clamp_points, const void* grad_enc, nrf_grad_layout layout, float* grad_table, int32_t level_begin, int32_t level_end,
-	nrf_stream stream)
-{
 	NRF_REQUIRE(n_rays >= 0 && n_samples >= 1 && ray_stride >= 6, "bad sizes");
 	if (n_rays == 0) { HashArgs a; return fill_args(grid, a); }
 	NRF_REQUIRE(ray_batch && z, "null ray_batch / z");
 	const int64_t n_points = n_rays * n_samples;
 	NRF_REQUIRE(n_points < (int64_t(1) << 31), "n_rays * n_samples must be < 2^31 per call");
 	const PointSrc ps{nullptr, ray_batch, z, ray_stride, n_samples};
-	return launch_hash_bwd(grid, ps, n_points, clamp_points, grad_enc, layout, grad_table, stream, level_begin, level_end);
+	return launch_hash_bwd(grid, ps, n_points, clamp_points, grad_enc, layout, grad_table, stream);
 }
 
 

@@ -130,9 +130,8 @@ __device__ __forceinline__ float adam_update(float p, float g, float& m, float& 
 // together (NVLink round trips are ~2 us: the kernel lives on memory-level parallelism).
 // MC: the gradient sum of a quad is ONE multimem.ld_reduce on the multicast mapping and the fp16 result ONE multimem.st, instead of WORLD peer
 // loads and WORLD peer stores: per GPU and step 1/W x 35.6 MB arrives reduced (4.5 MB at W = 8) instead of (W-1)/W x 35.6 MB.
-// One call may cover only part of the flat vector: the sharded scalars [range_lo, range_hi) (multiples of 4; partitioned over the ranks) and the
-// replicated scalars [tail_lo, tail_hi).  The default step is one call over everything; the overlapped step (parallel.py) exchanges the part of
-// the gradient that is already complete on a side stream, with a narrow grid and its own flag block, while the backward still scatters the rest.
+// The kernel takes its two regions as ranges: the sharded scalars [range_lo, range_hi) (multiples of 4; partitioned over the ranks) and the
+// replicated scalars [tail_lo, tail_hi).  nrf_adam_step_sharded launches it over the whole flat vector: [0, n_sharded / 4 * 4) and the rest.
 template <int WORLD, int U, bool MC>
 __global__ void __launch_bounds__(512, 1) adam_sharded_kernel(PeerArgs a, float* __restrict__ param, float* __restrict__ m, float* __restrict__ v,
 	float* grad_local, int64_t range_lo, int64_t range_hi, int64_t tail_lo, int64_t tail_hi, const AdamSchedState* __restrict__ sched, float beta1,
@@ -250,19 +249,9 @@ int nrf_adam_step_sharded(const nrf_peer_group* pg, float* param, float* exp_avg
 	const void* sched_state, float beta1, float beta2, float eps, float grad_scale, nrf_stream stream)
 {
 	NRF_REQUIRE(n_sharded >= 0 && n_total >= n_sharded, "bad sizes");
-	const int64_t q4 = n_sharded / 4 * 4;
-	return nrf_adam_step_sharded_range(pg, param, exp_avg, exp_avg_sq, 0, q4, q4, n_total, sched_state, beta1, beta2, eps, grad_scale, 0, stream);
-}
-
-int nrf_adam_step_sharded_range(const nrf_peer_group* pg, float* param, float* exp_avg, float* exp_avg_sq, int64_t range_begin, int64_t range_end,
-	int64_t tail_begin, int64_t tail_end, const void* sched_state, float beta1, float beta2, float eps, float grad_scale, int32_t n_ctas,
-	nrf_stream stream)
-{
 	NRF_REQUIRE(pg != nullptr && pg->world >= 1 && pg->world <= NRF_MAX_PEERS && pg->rank >= 0 && pg->rank < pg->world, "bad peer group");
-	NRF_REQUIRE(range_begin >= 0 && range_end >= range_begin && range_begin % 4 == 0 && range_end % 4 == 0, "sharded range must be made of whole quads");
-	NRF_REQUIRE(tail_begin >= 0 && tail_end >= tail_begin, "bad tail range");
-	NRF_REQUIRE(n_ctas >= 0, "bad n_ctas");
-	if (range_end == range_begin && tail_end == tail_begin) return NRF_OK;
+	if (n_total == 0) return NRF_OK;
+	const int64_t q4 = n_sharded / 4 * 4;   // sharded: whole quads of the table; replicated: [q4, n_total)
 	NRF_REQUIRE(param && exp_avg && exp_avg_sq && sched_state, "null pointer");
 	PeerArgs a;
 	a.world = pg->world; a.rank = pg->rank;
@@ -275,16 +264,15 @@ int nrf_adam_step_sharded_range(const nrf_peer_group* pg, float* param, float* e
 	}
 	NRF_REQUIRE(((reinterpret_cast<uintptr_t>(param) | reinterpret_cast<uintptr_t>(exp_avg) | reinterpret_cast<uintptr_t>(exp_avg_sq)) & 15) == 0,
 		"buffers must be 16-byte aligned");
-	// one CTA per SM (or n_ctas of them), all co-resident: the in-kernel barriers need every CTA of the grid running
+	// one CTA per SM, all co-resident: the in-kernel barriers need every CTA of the grid running
 	int sms = kNumSMs;
 	int dev = 0;
 	if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-	NRF_REQUIRE(n_ctas <= sms, "n_ctas exceeds the number of SMs");
 	// cooperative launch: the driver guarantees that all CTAs are co-resident (or refuses the launch) — the in-kernel barriers spin
 	float* grad_local = const_cast<float*>(a.grads[a.rank]);
 	const AdamSchedState* sched = reinterpret_cast<const AdamSchedState*>(sched_state);
 	cudaLaunchConfig_t cfg = {};
-	cfg.gridDim = dim3(n_ctas > 0 ? n_ctas : sms);
+	cfg.gridDim = dim3(sms);
 	cfg.blockDim = dim3(512);
 	cfg.dynamicSmemBytes = 0;
 	cfg.stream = as_stream(stream);
@@ -299,10 +287,10 @@ int nrf_adam_step_sharded_range(const nrf_peer_group* pg, float* param, float* e
 	const bool mc = pg->grads_mc != nullptr && pg->shadow_f16_mc != nullptr && pg->world > 1;
 	NRF_REQUIRE(!mc || (((reinterpret_cast<uintptr_t>(pg->grads_mc) & 15) | (reinterpret_cast<uintptr_t>(pg->shadow_f16_mc) & 7)) == 0), "multicast mappings must be 16-byte aligned");
 #define NRF_LAUNCH_SHARDED(W, U)                                                                                                                 \
-	launch_err = mc ? cudaLaunchKernelEx(&cfg, adam_sharded_kernel<W, 4, true>, a, param, exp_avg, exp_avg_sq, grad_local, range_begin, range_end,     \
-	                      tail_begin, tail_end, sched, beta1, beta2, eps, grad_scale)                                                            \
-	                : cudaLaunchKernelEx(&cfg, adam_sharded_kernel<W, U, false>, a, param, exp_avg, exp_avg_sq, grad_local, range_begin, range_end,    \
-	                      tail_begin, tail_end, sched, beta1, beta2, eps, grad_scale)
+	launch_err = mc ? cudaLaunchKernelEx(&cfg, adam_sharded_kernel<W, 4, true>, a, param, exp_avg, exp_avg_sq, grad_local, 0, q4, q4, n_total,  \
+	                      sched, beta1, beta2, eps, grad_scale)                                                                                  \
+	                : cudaLaunchKernelEx(&cfg, adam_sharded_kernel<W, U, false>, a, param, exp_avg, exp_avg_sq, grad_local, 0, q4, q4, n_total, \
+	                      sched, beta1, beta2, eps, grad_scale)
 	switch (pg->world) {
 		case 1: NRF_LAUNCH_SHARDED(1, 4); break;
 		case 2: NRF_LAUNCH_SHARDED(2, 4); break;

@@ -187,22 +187,18 @@ def hash_encode_rays_fwd(grid: HashGridSpec, table_f16: torch.Tensor, ray_batch:
 
 
 def hash_encode_rays_bwd(grid: HashGridSpec, ray_batch: torch.Tensor, z: torch.Tensor, grad_enc: torch.Tensor, grad_table: torch.Tensor,
-                         clamp: bool = True, levels: tuple[int, int] | None = None, jitter: PointJitter | None = None) -> torch.Tensor:
-    """levels = (begin, end): scatter those levels only (two calls over [0, k) and [k, L) add up to the full gradient).
-    jitter: the forward's perturbed points, re-derived from the same variates (nrf_hash_encode_rays_jitter_bwd; all levels)."""
+                         clamp: bool = True, jitter: PointJitter | None = None) -> torch.Tensor:
+    """jitter: the forward's perturbed points, re-derived from the same variates (nrf_hash_encode_rays_jitter_bwd)."""
     r, s = z.shape
     layout = {f32: cabi.GRAD_F32, bf16: cabi.GRAD_BF16}[grad_enc.dtype]
     g = grid.c_struct()
     if jitter is not None:
-        if levels is not None:
-            raise cabi.NrfError("the jittered scatter covers all levels")
         j = jitter.c_struct()
         _run("hash_encode_bwd", lambda: lib().nrf_hash_encode_rays_jitter_bwd(C.byref(g), ptr(ray_batch, f32), ray_batch.shape[1], ptr(z, f32), r, s,
                                         int(clamp), ptr(grad_enc), layout, ptr(grad_table, f32), C.byref(j), stream()))
         return grad_table
-    lb, le = levels if levels is not None else (0, -1)
-    _run("hash_encode_bwd", lambda: lib().nrf_hash_encode_rays_bwd_levels(C.byref(g), ptr(ray_batch, f32), ray_batch.shape[1], ptr(z, f32), r, s, int(clamp),
-                                    ptr(grad_enc), layout, ptr(grad_table, f32), lb, le, stream()))
+    _run("hash_encode_bwd", lambda: lib().nrf_hash_encode_rays_bwd(C.byref(g), ptr(ray_batch, f32), ray_batch.shape[1], ptr(z, f32), r, s, int(clamp),
+                                    ptr(grad_enc), layout, ptr(grad_table, f32), stream()))
     return grad_table
 
 
@@ -526,13 +522,6 @@ def render_rays_fwd(grid: HashGridSpec, table_f16, packed, rays_o, rays_d, t_val
                                         ptr(rays_d, f32), r, ptr(t_vals, f32), ptr(u, f32), ptr(workspace), workspace.numel(), ptr(rgb), ptr(depth),
                                         ptr(disp), ptr(acc), ptr(weights), ptr(z), stream()))
     return {"rgb": rgb, "depth": depth, "disp": disp, "acc": acc, "weights": weights, "z": z}, workspace
-
-
-def adam_step_sharded_range(peer_group, param, exp_avg, exp_avg_sq, sharded: tuple[int, int], tail: tuple[int, int], sched_state, beta1=0.9,
-                            beta2=0.99, eps=1e-15, grad_scale=1.0, n_ctas: int = 0) -> None:
-    """nrf_adam_step_sharded_range: the fused data-parallel step on the sharded scalars [sharded) and the replicated scalars [tail)."""
-    _run("adam_step", lambda: lib().nrf_adam_step_sharded_range(C.byref(peer_group), ptr(param, f32), ptr(exp_avg, f32), ptr(exp_avg_sq, f32), sharded[0],
-                              sharded[1], tail[0], tail[1], ptr(sched_state), beta1, beta2, eps, grad_scale, n_ctas, stream()))
 
 
 def adam_step_sharded(peer_group, param, exp_avg, exp_avg_sq, n_sharded: int, sched_state, beta1=0.9, beta2=0.99, eps=1e-15, grad_scale=1.0) -> None:

@@ -132,32 +132,7 @@ class PeerShardedOptimizer:
                 pg.grads_mc = mc[0] + (self.grads.data_ptr() - list(handles[0].buffer_ptrs)[rank])
                 pg.shadow_f16_mc = mc[1] + (self.shadow.data_ptr() - list(handles[1].buffer_ptrs)[rank])
                 self.multicast = True
-        # Overlapped exchange (NRF_DP_OVERLAP=1; models that can split their backward by table level: HashNeRF.dp_overlap_split): the gradient
-        # below level k's offset is complete once the scatter of levels [0, k) has run, so its reduce-scatter + Adam + shadow all-gather goes to
-        # a side stream — a narrow cooperative grid with its OWN flag block — while the main stream scatters levels [k, L); the rest follows as
-        # usual.  Ownership is per range (each range is partitioned over the ranks on its own), fixed for the life of this object.
-        q4 = model.n_table // 4 * 4
-        self.ranges = [(0, q4)]
-        self.overlap, self.pg_side, self._side_pending = False, None, False
-        split = model.dp_overlap_split() if hasattr(model, "dp_overlap_split") else None
-        if os.environ.get("NRF_DP_OVERLAP", "0") == "1" and world > 1 and split is not None:
-            self.split_level, off = split
-            self.split = min(max(off // 4 * 4, 0), q4)
-            self.flags_side = symm.empty(n_flags, dtype=torch.int32, device=dev)
-            self.flags_side.zero_()
-            h = symm.rendezvous(self.flags_side, group.group_name)
-            ptrs = list(h.buffer_ptrs)
-            off_b = self.flags_side.data_ptr() - ptrs[rank]
-            side = cabi.PeerGroup()
-            side.world, side.rank = world, rank
-            for pr in range(world):
-                side.grads[pr], side.shadow_f16[pr], side.flags[pr] = pg.grads[pr], pg.shadow_f16[pr], ptrs[pr] + off_b
-            side.grads_mc, side.shadow_f16_mc = pg.grads_mc, pg.shadow_f16_mc
-            self.pg_side, self._side_handle = side, h
-            self.ranges = [(0, self.split), (self.split, q4)]
-            self.side_stream = torch.cuda.Stream(device=dev, priority=-1)   # its CTAs go first when the scatter frees a slot
-            self.side_ctas = int(os.environ.get("NRF_DP_OVERLAP_CTAS", "32"))
-            self.overlap = True
+        self.n_table = model.n_table
         model.grads, model.shadow = self.grads, self.shadow
         model.peer = self
         if hasattr(model, "bind_peer_buffers"):
@@ -203,11 +178,9 @@ class PeerShardedOptimizer:
         ref = model.shadow.clone()
         dist.broadcast(ref, src=0)
         same = torch.equal(ref, model.shadow)
-        owner_ok, master_diff = True, torch.zeros((), device=dev)
-        for lo, hi in self.owned_ranges():
-            owner_ok = owner_ok and torch.equal(model.params[lo:hi].half(), model.shadow[lo:hi])
-            if hi > lo:
-                master_diff = torch.maximum(master_diff, (model.params[lo:hi] - pa[lo:hi]).abs().max())
+        lo, hi = self.owned_range()
+        owner_ok = torch.equal(model.params[lo:hi].half(), model.shadow[lo:hi])
+        master_diff = (model.params[lo:hi] - pa[lo:hi]).abs().max() if hi > lo else torch.zeros((), device=dev)
         cleared = float(model.grads.abs().max()) == 0.0
         stats = torch.tensor([float(diff), float(master_diff), float(not same), float(not owner_ok), float(not cleared), float(self.timeout()), float(n_diff)],
                              dtype=torch.float64, device=dev)
@@ -226,32 +199,27 @@ class PeerShardedOptimizer:
                "shadows_bit_identical_across_ranks": stats[2].item() == 0.0, "owner_master_matches_shadow": stats[3].item() == 0.0,
                "gradient_cleared": stats[4].item() == 0.0, "flags_timeout": int(stats[5].item()), "entries_differing_by_more_than_5pct_of_lr": int(stats[6].item()),
                "entries": int(model.params.numel()), "lr": model.lr0,
-               "multicast": bool(self.multicast), "overlap": bool(self.overlap),
+               "multicast": bool(self.multicast),
                "what": "one step on a random per-rank gradient: fused peer-memory kernel vs NCCL all-reduce + dense Adam"}
         out["ok"] = bool(out["shadows_bit_identical_across_ranks"] and out["owner_master_matches_shadow"] and out["gradient_cleared"]
                          and out["flags_timeout"] == 0 and out["entries_differing_by_more_than_5pct_of_lr"] <= 8)
         return out
 
     def timeout(self) -> int:
-        """The sticky barrier-timeout marker of this rank's flag block(s) (synchronises the device)."""
-        t = int(self.flags[2 * self.world + 2])
-        if self.overlap:
-            t = max(t, int(self.flags_side[2 * self.world + 2]))
-        return t
+        """The sticky barrier-timeout marker of this rank's flag block (synchronises the device)."""
+        return int(self.flags[2 * self.world + 2])
 
     def check(self) -> None:
         """Raises if a peer barrier of the fused optimiser ever gave up waiting.  Reads a pinned-host mirror of the marker that
         `mirror_flag` refreshes asynchronously after every step: no device synchronisation, at most a few steps late."""
-        if self._flag_host is not None and (int(self._flag_host[0]) != 0 or int(self._flag_host[1]) != 0):
+        if self._flag_host is not None and int(self._flag_host[0]) != 0:
             raise RuntimeError(f"nerfpp_b200: rank {self.rank}: a peer barrier of the fused data-parallel optimiser timed out — a rank missed a "
                                "step; parameters were left untouched from that step on (nrf_adam_step_sharded)")
 
     def mirror_flag(self) -> None:
         if self._flag_host is None:
-            self._flag_host = torch.zeros(2, dtype=torch.int32).pin_memory()
-        self._flag_host[0:1].copy_(self.flags[2 * self.world + 2: 2 * self.world + 3], non_blocking=True)
-        if self.overlap:
-            self._flag_host[1:2].copy_(self.flags_side[2 * self.world + 2: 2 * self.world + 3], non_blocking=True)
+            self._flag_host = torch.zeros(1, dtype=torch.int32).pin_memory()
+        self._flag_host.copy_(self.flags[2 * self.world + 2: 2 * self.world + 3], non_blocking=True)
 
     def allgather_master(self, model) -> None:
         """Re-assemble the fp32 master and the Adam moments on every rank: under the fused optimiser a rank only updates the shard it
@@ -260,38 +228,13 @@ class PeerShardedOptimizer:
         Collective (one broadcast per rank and buffer: 3 x 35 MB in total, off the hot path)."""
         torch.cuda.synchronize(model.device)
         for r in range(self.world):
-            for lo, hi in self.owned_ranges(r):
-                for buf in (model.params, model.exp_avg, model.exp_avg_sq):
-                    dist.broadcast(buf[lo:hi], src=r)
+            lo, hi = self.owned_range(r)
+            for buf in (model.params, model.exp_avg, model.exp_avg_sq):
+                dist.broadcast(buf[lo:hi], src=r)
         model.masters_synced = True
 
-    def owned_ranges(self, rank: int | None = None) -> list[tuple[int, int]]:
-        """[begin, end) scalars of the table that `rank` (default: this rank) owns: one slice per exchanged range, the kernel's own split
-        (quads, the first ranks take one extra)."""
-        rank = self.rank if rank is None else rank
-        out = []
-        for lo, hi in self.ranges:
-            b, e = shard_bounds((hi - lo) // 4, rank, self.world)
-            out.append((lo + 4 * b, lo + 4 * e))
-        return out
-
-    def shard_bounds(self, n_sharded: int) -> tuple[int, int]:
-        """[begin, end) scalars of the table this rank owns when the table is exchanged as ONE range (no overlap)."""
-        assert not self.overlap, "with the overlapped exchange ownership is per range: owned_ranges()"
-        b, e = shard_bounds(n_sharded // 4, self.rank, self.world)
+    def owned_range(self, rank: int | None = None) -> tuple[int, int]:
+        """[begin, end) scalars of the table that `rank` (default: this rank) owns: the kernel's own split (quads, the first ranks take one
+        extra); the scalars past the last whole quad belong to the replicated tail."""
+        b, e = shard_bounds(self.n_table // 4, self.rank if rank is None else rank, self.world)
         return 4 * b, 4 * e
-
-    # -- overlapped exchange
-    def backward_overlapped(self, model, scatter) -> None:
-        """scatter(levels) runs the model's table-gradient scatter for a level range on the current stream.  Levels [0, k) first; then their
-        slice of the gradient is exchanged and applied on the side stream while levels [k, L) scatter here.  _optimizer_step_sharded joins."""
-        from . import ops
-        cur = torch.cuda.current_stream(model.device)
-        scatter((0, self.split_level))
-        ops.adam_schedule_advance(model.sched, model.lr0, 0.1, float(model.lrate_decay * 1000))
-        self.side_stream.wait_stream(cur)
-        with torch.cuda.stream(self.side_stream):
-            ops.adam_step_sharded_range(self.pg_side, model.params, model.exp_avg, model.exp_avg_sq, self.ranges[0], (0, 0), model.sched, 0.9, 0.99, 1e-15,
-                                        1.0 / self.world, n_ctas=self.side_ctas)
-        scatter((self.split_level, -1))
-        self._side_pending = True

@@ -16,7 +16,6 @@ Configuration is the parity one: ThinRay, Perturb 0, no raw noise, no stochastic
 from __future__ import annotations
 
 import math
-import os
 
 import numpy as np
 import torch
@@ -132,22 +131,8 @@ class FlatAdamModel:
     def _optimizer_step_sharded(self):
         """Data-parallel step without NCCL: one kernel per rank over NVLink peer memory (parallel.PeerShardedOptimizer)."""
         self.masters_synced = False
-        peer = self.peer
-        q4, n = self.n_table // 4 * 4, self.params.numel()
-        args = (self.params, self.exp_avg, self.exp_avg_sq)
-        if not peer.overlap:
-            ops.adam_schedule_advance(self.sched, self.lr0, 0.1, float(self.lrate_decay * 1000))
-            ops.adam_step_sharded_range(peer.pg, *args, (0, q4), (q4, n), self.sched, 0.9, 0.99, 1e-15, 1.0 / peer.world)
-        else:
-            # two ranges, each partitioned over the ranks on its own (ownership never changes).  The first one was already exchanged behind the
-            # backward (PeerShardedOptimizer.backward_overlapped) or, when the step is taken on a finished gradient (dp_check), goes first here.
-            if peer._side_pending:
-                torch.cuda.current_stream(self.device).wait_stream(peer.side_stream)
-                peer._side_pending = False
-            else:
-                ops.adam_schedule_advance(self.sched, self.lr0, 0.1, float(self.lrate_decay * 1000))
-                ops.adam_step_sharded_range(peer.pg_side, *args, peer.ranges[0], (0, 0), self.sched, 0.9, 0.99, 1e-15, 1.0 / peer.world)
-            ops.adam_step_sharded_range(peer.pg, *args, peer.ranges[1], (q4, n), self.sched, 0.9, 0.99, 1e-15, 1.0 / peer.world)
+        ops.adam_schedule_advance(self.sched, self.lr0, 0.1, float(self.lrate_decay * 1000))
+        ops.adam_step_sharded(self.peer.pg, self.params, self.exp_avg, self.exp_avg_sq, self.n_table, self.sched, 0.9, 0.99, 1e-15, 1.0 / self.peer.world)
         self.repack()
 
     def flags_timeout(self) -> int:
@@ -190,9 +175,8 @@ class FlatAdamModel:
         from . import cabi
         l0 = cabi.launch_count()
         self._g_fb = torch.cuda.CUDAGraph()
-        overlap = world > 1 and self.peer is not None and getattr(self.peer, "overlap", False)
         with torch.cuda.graph(self._g_fb):
-            self._g_out = self.forward_backward(*self._g_in, dp_overlap=True) if overlap else self.forward_backward(*self._g_in)
+            self._g_out = self.forward_backward(*self._g_in)
             if world == 1:
                 self._optimizer_step_scheduled(1.0)
             elif self.peer is not None:
@@ -450,18 +434,9 @@ class HashNeRF(FlatAdamModel):
         return g_enc
 
     # -- one optimisation step (src/NeRFExecutor.h:868-890, 923, 986-996)
-    def dp_overlap_split(self):
-        """(level k, scalar offset of level k in the flat table): the table gradient below that offset is complete once levels [0, k) have been
-        scattered — what parallel.PeerShardedOptimizer exchanges behind the scatter of levels [k, L) (NRF_DP_OVERLAP=1)."""
-        k = int(os.environ.get("NRF_DP_OVERLAP_LEVEL", "14"))
-        k = min(max(k, 1), self.grid.n_levels - 1)
-        return k, int(self.grid.feat_local_idx[k])
-
-    def forward_backward(self, *inputs, grad_scale=1.0, dp_overlap=False):
+    def forward_backward(self, *inputs, grad_scale=1.0):
         """Render + huber + backward into self.grads (accumulating).  self.loss holds the mean huber loss.  inputs: (rays_o, rays_d, target), or
-        (pix_hw,) — int32 [R,2] pixel coordinates of the view given to set_camera: rays and targets are then formed on the device.
-        dp_overlap (a training step under the fused data-parallel optimiser with NRF_DP_OVERLAP=1): the table gradient is scattered in two level
-        ranges and the exchange of the first starts behind the second (the optimiser step that follows joins it)."""
+        (pix_hw,) — int32 [R,2] pixel coordinates of the view given to set_camera: rays and targets are then formed on the device."""
         if len(inputs) == 1:
             image, cam = self._cam
             rays_o, rays_d, target, rb, z, sh = ops.ray_setup_pixels(inputs[0], None, None, image, self.bbox, 0.0, self.t_vals, self.sh_degree,
@@ -474,11 +449,7 @@ class HashNeRF(FlatAdamModel):
         # RawToOutputs of the fine pass + huber + their backward: one launch
         d_raw, out["rgb"] = ops.composite_huber_bwd(raw, out["z"], rays_d, target, self.loss, grad_scale=grad_scale)
         g_enc = self._mlp_backward(enc, views, ray_sh, raw.shape[1], keep, d_raw)
-        if dp_overlap and self.peer is not None and self.peer.overlap:
-            self.peer.backward_overlapped(self, lambda levels: ops.hash_encode_rays_bwd(self.grid, ray_batch, out["z"], g_enc, self.grads[:self.n_table],
-                                                                                        clamp=True, levels=levels))
-        else:
-            ops.hash_encode_rays_bwd(self.grid, ray_batch, out["z"], g_enc, self.grads[:self.n_table], clamp=True)
+        ops.hash_encode_rays_bwd(self.grid, ray_batch, out["z"], g_enc, self.grads[:self.n_table], clamp=True)
         return out
 
 

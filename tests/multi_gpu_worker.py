@@ -64,19 +64,8 @@ def main():
     assert chk["ok"], chk
     assert c.step == 0 and torch.equal(before, c.params) and float(c.grads.abs().max()) == 0.0
     c.capture_train_step(R, world)
-    # D: the overlapped exchange (NRF_DP_OVERLAP=1): levels [0, k) of the table gradient are exchanged on a side stream behind the scatter of
-    # levels [k, L), inside the captured graph; ownership is per range
-    d_ = HashNeRF(BBOX, log2_hashmap_size=15, seed=3, device=dev, lrate_decay=1)
-    parallel.broadcast_parameters(d_.params, world); d_.refresh()
-    os.environ["NRF_DP_OVERLAP"] = "1"
-    peer_d = parallel.PeerShardedOptimizer(d_, rank, world)
-    os.environ.pop("NRF_DP_OVERLAP")
-    assert peer_d.overlap and len(peer_d.ranges) == 2 and 0 < peer_d.split < d_.n_table
-    chk_d = peer_d.dp_check(d_)                      # the step on a finished gradient: both ranges one after the other
-    assert chk_d["ok"] and chk_d["overlap"], chk_d
-    d_.capture_train_step(R, world)
 
-    la, lb, lc, ld = [], [], [], []
+    la, lb, lc = [], [], []
     for i in range(6):
         batch = batches[i % 3]
         a.forward_backward(*batch)
@@ -86,9 +75,8 @@ def main():
         b_.optimizer_step_sharded()
         lb.append(float(b_.loss))
         lc.append(float(c.train_step_graph(*batch)))
-        ld.append(float(d_.train_step_graph(*batch)))
     torch.cuda.synchronize()
-    for name, m, losses in (("eager", b_, lb), ("graph", c, lc), ("overlap", d_, ld)):
+    for name, m, losses in (("eager", b_, lb), ("graph", c, lc)):
         assert int(m.flags_timeout()) == 0, f"{name}: peer barrier timed out"
         m.peer.check()
         # every rank holds the SAME fp16 shadow, bit for bit
@@ -96,8 +84,8 @@ def main():
         dist.broadcast(ref, src=0)
         assert torch.equal(ref, m.shadow), f"{name}: shadows differ between ranks"
         # the owner's fp32 master agrees with the shadow it published; the MLP tail is replicated
-        for lo, hi in m.peer.owned_ranges():
-            assert torch.equal(m.params[lo:hi].half(), m.shadow[lo:hi]), f"{name}: owner shard / shadow mismatch"
+        lo, hi = m.peer.owned_range()
+        assert torch.equal(m.params[lo:hi].half(), m.shadow[lo:hi]), f"{name}: owner shard / shadow mismatch"
         assert torch.equal(m.params[m.n_table:].half(), m.shadow[m.n_table:])
         tail = m.params[m.n_table:].clone()
         dist.broadcast(tail, src=0)
@@ -144,7 +132,7 @@ def main():
     if rank == 0:
         whole = c.render_image(H, W, K, c2w)["rgb"]
         assert torch.equal(full, whole)
-        print("MULTI_GPU_WORKER_OK", world, la[-1], lb[-1], lc[-1], "dp_grad_rel", rel, rel_mlp, "multicast(b)", b_.peer.multicast, "overlap(d)", ld[-1], peer_d.split_level, "dp_check", chk)
+        print("MULTI_GPU_WORKER_OK", world, la[-1], lb[-1], lc[-1], "dp_grad_rel", rel, rel_mlp, "multicast(b)", b_.peer.multicast, "dp_check", chk)
     dist.barrier()
     dist.destroy_process_group()
 

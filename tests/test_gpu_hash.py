@@ -386,31 +386,6 @@ def test_ray_grouped_order_changes_no_bit(L, feat):
         assert torch.equal(torch.gather(kc.view(R, S + N), 1, new), torch.gather(keep_f.view(R, S + N), 1, new)), group
 
 
-@pytest.mark.parametrize("split", [4, 12, 14])
-def test_level_split_backward_adds_up(split):
-    """nrf_hash_encode_rays_bwd_levels over [0, k) and [k, L) == the one-call scatter (up to the order of the atomic sums), also for a split that
-    cuts an 8-value gradient chunk (k = 14); and the table gradient below level k's offset is complete after the first call — what the overlapped
-    data-parallel exchange relies on (nerfpp_b200/parallel.py)."""
-    from nerfpp_b200 import ops
-    grid = _grid(T=16)
-    g = torch.Generator(device="cuda").manual_seed(21)
-    R, S = 129, 96
-    rb = _ray_batch(R, seed=3)
-    rb2 = ops.rays_prepare(rb[:, 0:3].contiguous(), rb[:, 3:6].contiguous(), BBOX, 0.0, True)
-    z = ops.z_sample(rb2, torch.linspace(0, 1, S).cuda())
-    G = torch.randn(R * S, 32, generator=g, device="cuda").to(torch.bfloat16)
-    whole = torch.zeros(grid.table_scalars(), device="cuda")
-    ops.hash_encode_rays_bwd(grid, rb2, z, G, whole)
-    part = torch.zeros_like(whole)
-    ops.hash_encode_rays_bwd(grid, rb2, z, G, part, levels=(0, split))
-    off = int(grid.feat_local_idx[split])
-    tol = 2e-6 * float(whole.abs().max())
-    assert float((part[:off] - whole[:off]).abs().max()) <= tol          # the prefix is complete
-    ops.hash_encode_rays_bwd(grid, rb2, z, G, part, levels=(split, 16))
-    assert float((part - whole).abs().max()) <= tol
-    assert torch.equal(part != 0, whole != 0)
-
-
 def test_against_reference_cuda_kernels(ref_cuda):
     """Live: the reference's CuHashEmbedder forward/backward kernels on the same table, primes and points."""
     if ref_cuda is None:

@@ -45,27 +45,23 @@ def test_shard_bounds_partition():
         assert max(sizes) - min(sizes) <= 1
 
 
-def test_owned_ranges_of_the_fused_optimiser_partition_every_exchanged_range():
-    """PeerShardedOptimizer.owned_ranges mirrors the kernel's split (csrc/optim_sharded.cu: quads, the first ranks take one extra) for one range
-    (the default step) and for two (the overlapped exchange): per range the owners' slices tile it exactly, in whole quads."""
+def test_owned_range_of_the_fused_optimiser_partitions_the_table():
+    """PeerShardedOptimizer.owned_range mirrors the kernel's split (csrc/optim_sharded.cu: quads, the first ranks take one extra): the owners'
+    slices tile the table's whole quads exactly."""
     n_table = 8912896 + 3                                   # not a multiple of 4: the leftover scalars belong to the replicated tail
     q4 = n_table // 4 * 4
     for world in (1, 2, 3, 4, 8):
-        for ranges in ([(0, q4)], [(0, 4220000), (4220000, q4)], [(0, 12), (12, q4)]):
-            per_rank = []
-            for rank in range(world):
-                opt = object.__new__(parallel.PeerShardedOptimizer)
-                opt.rank, opt.world, opt.ranges = rank, world, ranges
-                per_rank.append(opt.owned_ranges())
-                assert per_rank[-1] == opt.owned_ranges(rank)
-            for k, (lo, hi) in enumerate(ranges):
-                spans = [per_rank[r][k] for r in range(world)]
-                assert spans[0][0] == lo and spans[-1][1] == hi
-                assert all(a[1] == b[0] for a, b in zip(spans, spans[1:]))
-                assert all(b % 4 == 0 and e % 4 == 0 for b, e in spans)
-                quads = (hi - lo) // 4
-                base, extra = divmod(quads, world)
-                assert [(e - b) // 4 for b, e in spans] == [base + (1 if r < extra else 0) for r in range(world)]   # the kernel's formula
+        spans = []
+        for rank in range(world):
+            opt = object.__new__(parallel.PeerShardedOptimizer)
+            opt.rank, opt.world, opt.n_table = rank, world, n_table
+            spans.append(opt.owned_range())
+            assert spans[-1] == opt.owned_range(rank)
+        assert spans[0][0] == 0 and spans[-1][1] == q4
+        assert all(a[1] == b[0] for a, b in zip(spans, spans[1:]))
+        assert all(b % 4 == 0 and e % 4 == 0 for b, e in spans)
+        base, extra = divmod(q4 // 4, world)
+        assert [(e - b) // 4 for b, e in spans] == [base + (1 if r < extra else 0) for r in range(world)]   # the kernel's formula
 
 
 def test_lr_schedule_matches_reference_order():
